@@ -454,6 +454,41 @@ def measure_tool(args):
     return out
 
 
+DUMP_TASKS = 1 << 19
+DUMP_MAX_BYTES = 60 << 20   # (the .npy headers and the 64 MB limit stay clear of it)
+
+
+def dump_outputs(out_dir, res, seed):
+    """Writes what the resident plan's last step returned as out_dir/<name>.npy, so that two builds can be compared
+    output for output on the same inputs.  For a fixed, seeded sample of up to DUMP_TASKS tasks (all of them in a
+    smaller batch): the best total per task and the task's winning rows, with each row's column list in row order (the
+    library may lay its column pool out differently from build to build).  The sample is the longest prefix of a seeded
+    permutation of the tasks that fits in DUMP_MAX_BYTES.  Values are integers, written as float32 when every one of
+    them is below 2**24 (exact there), else as float64."""
+    n = len(res.best)
+    rows, cols = res.rows, res.cols
+    width = rows["n1"].astype(np.int64) + rows["n2"]
+    fields = ("task", "read_split", "score1", "score2", "n1", "n2")
+    big = max([n] + [int(np.abs(a).max(initial=0)) for a in [res.best, cols] + [rows[f] for f in fields]])
+    dtype = np.float32 if big < 1 << 24 else np.float64
+    per_task = 2 + len(fields) * np.bincount(rows["task"], minlength=n) + np.bincount(rows["task"], weights=width, minlength=n)
+    order = np.random.default_rng(seed).permutation(n)[:DUMP_TASKS]
+    k = int(np.searchsorted(np.cumsum(per_task[order] * np.dtype(dtype).itemsize), DUMP_MAX_BYTES, side="right"))
+    tasks = np.sort(order[:k])
+    picked = np.zeros(n, dtype=bool)
+    picked[tasks] = True
+    sel = picked[rows["task"]]
+    rows, width = rows[sel], width[sel]
+    first = np.cumsum(width) - width
+    out = {"tasks": tasks, "best": res.best[tasks],
+           "row_cols": cols[np.repeat(rows["col_begin"], width) + np.arange(int(width.sum())) - np.repeat(first, width)]}
+    for f in fields:
+        out["row_" + f] = rows[f]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=dtype))
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -527,6 +562,8 @@ def run_ours(args):
     sweep_ms.append(st["ms_sweep"])
     probe_ms.append(st["ms_probe"])
     res = plan.fetch(copy=False)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, res, args.seed)
     st = plan.stats()
     n_hit = int((res.best > 0).sum())
     n_rows = len(res.rows)
@@ -692,7 +729,11 @@ def main():
     ap.add_argument("--no-sharded", action="store_true")
     ap.add_argument("--shard-clusters", type=int, default=8000)                # sharded_merge leg: clusters of the ONE batch all ranks share
     ap.add_argument("--tool-clusters", type=int, default=2000)                 # tool leg: clusters (x 100 read pairs) of the generated split
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step (a seeded sample of rank 0's tasks) to DIR/<name>.npy, 64 MB at most")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.out = _claim_stdout()
     if args.impl == "reference":
         return run_reference_arm(args)

@@ -164,6 +164,18 @@ def split_align_count(read, ref1, ref2, min_score, match=2, mismatch=-1, gap=-2,
     return int(n), (int(out[0, 4]) if n else 0)
 
 
+def split_alignment(read, ref1, ref2, min_score, which, match=2, mismatch=-1, gap=-2, end_gaps=False, min_split_score=8):
+    """Number of alignments GetAlignments would emit and alignment number `which` in emission order (None when
+    there are not that many), without materialising the others (port only)."""
+    read, ref1, ref2 = bytes(read), bytes(ref1), bytes(ref2)
+    out = np.zeros((which + 1, 7), dtype=np.int32)
+    a, b, c = _u8(read), _u8(ref1), _u8(ref2)
+    n = _lib("port").dpo_split_align(_p(a, _c_u8p), len(read), _p(b, _c_u8p), len(ref1), _p(c, _c_u8p), len(ref2),
+                                     match, mismatch, gap, int(end_gaps), min_split_score, min_score,
+                                     _p(out, _c_i32p), which + 1, None, None)
+    return int(n), (out[which].copy() if which < n else None)
+
+
 def split_rowmax(read, ref1, ref2, match=2, mismatch=-1, gap=-2, end_gaps=False, min_split_score=8):
     """FindMaxRowEntry of every row of both matrices (port only): two (L+1,) int32 arrays."""
     read, ref1, ref2 = bytes(read), bytes(ref1), bytes(ref2)

@@ -1,4 +1,5 @@
 import os
+import subprocess
 import sys
 
 import pytest
@@ -25,3 +26,16 @@ def oracle_mod():
 def gpu_ctx():
     import defuse_b200
     return defuse_b200.default_context(0)
+
+
+@pytest.fixture(scope="session")
+def device_double(tmp_path_factory):
+    """tests/device_double built into a temporary directory: the eight C-ABI entry points the tools call, answered by
+    the parity oracle, for running the tools with LD_PRELOAD where there is no GPU."""
+    out = tmp_path_factory.mktemp("device_double")
+    obj, lib = str(out / "dp_oracle.o"), str(out / "libdevice_double.so")
+    subprocess.run(["gcc", "-O2", "-fPIC", "-c", os.path.join(ROOT, "oracle", "dp_oracle.c"), "-o", obj], check=True)
+    subprocess.run(["g++", "-O2", "-std=c++17", "-fPIC", "-shared", "-I" + os.path.join(ROOT, "include"), "-o", lib,
+                    os.path.join(ROOT, "tests", "device_double", "device_double.cpp"), obj, "-lpthread", "-Wl,--no-undefined"],
+                   check=True)
+    return lib

@@ -53,14 +53,13 @@ def test_no_gpu_means_failure_not_fallback():
 
 def test_dosplitalign_input_errors_like_the_reference(tmp_path):
     """Errors that come before any alignment (so no GPU is needed): same exit code, stdout and stderr as the compiled
-    reference tool for unreadable inputs and malformed region tables."""
+    reference tool for unreadable inputs and malformed region tables (its outputs stored as digests, with the dataset's
+    directory written as <dir>; where oracle/_ref is built the tool runs as well)."""
     import sys
     sys.path.insert(0, ROOT)
+    import oracle
+    import util
     from synth import files
-    from oracle import ref_tool
-    ref = ref_tool("ref_dosplitalign")
-    if not ref:
-        pytest.skip("oracle/_ref tools not built")
     d = str(tmp_path / "s")
     args = files.make_split_dataset(d, seed=3, n_clusters=6, pairs_per_cluster=10)
 
@@ -75,23 +74,23 @@ def test_dosplitalign_input_errors_like_the_reference(tmp_path):
     cases = [swap("-e", d + "/nope"), swap("-r", d + "/nope"), swap("-r", d + "/bad2.regions"), swap("-r", d + "/bad3.regions"),
              swap("-1", d + "/reads.1.txt"), swap("-2", d + "/nope.fastq"), swap("-i", d + "/nope.sam")]
     strip = lambda b: b.replace(b"[fai_load] build FASTA index.\n", b"")   # printed when the .fai does not exist yet
-    for a in cases:
+    for k, a in enumerate(cases):
         ours = subprocess.run([_tool("dosplitalign")] + a, capture_output=True)
-        theirs = subprocess.run([ref] + a, capture_output=True)
-        assert ours.returncode == theirs.returncode == 1, a
-        assert ours.stdout == theirs.stdout and strip(ours.stderr) == strip(theirs.stderr), a
+        theirs = util.reference_tool_digest(oracle, "dosplitalign_tool_errors/%d" % k, "ref_dosplitalign",
+                                            lambda ref: _exit_1([ref] + a, d, strip))
+        assert ours.returncode == 1, a
+        assert util.digest(ours.stdout.replace(d.encode(), b"<dir>"), strip(ours.stderr).replace(d.encode(), b"<dir>")) == theirs, a
 
 
 def test_matealign_input_errors_like_the_reference(tmp_path):
     """matealign's SAM checks and unreadable inputs: they come before any alignment (no GPU needed) and must give the
-    compiled reference tool's exit code, stdout and stderr -- with the SAM parsed by chunks on several threads."""
+    compiled reference tool's exit code, stdout and stderr -- with the SAM parsed by chunks on several threads (the
+    reference's outputs stored as digests, as above)."""
     import sys
     sys.path.insert(0, ROOT)
+    import oracle
+    import util
     from synth import files
-    from oracle import ref_tool
-    ref = ref_tool("ref_matealign")
-    if not ref:
-        pytest.skip("oracle/_ref tools not built")
     d = str(tmp_path / "m")
     args, sam = files.make_matealign_dataset(d, seed=4, n_pairs=50)
     lines = sam.split(b"\n")
@@ -106,10 +105,19 @@ def test_matealign_input_errors_like_the_reference(tmp_path):
     cases = [(swap("-r", d + "/nope.fa"), sam), (swap("-1", d + "/reads.1.txt"), sam), (swap("-2", d + "/nope.fastq"), sam),
              (args, b"\n".join(lines[:10] + [b""] + lines[10:])), (args, b"\n".join(lines[:7] + [b"a\tb\tc"] + lines[7:])),
              (args, b"\n".join(lines[:5] + [b"7/3\t0" + hit] + lines[5:])), (args, b"\n".join(lines[:5] + [b"73\t0" + hit] + lines[5:]))]
-    for a, text in cases:
-        theirs = subprocess.run([ref] + a, input=text, capture_output=True)
+    for k, (a, text) in enumerate(cases):
+        theirs = util.reference_tool_digest(oracle, "matealign_tool_errors/%d" % k, "ref_matealign",
+                                            lambda ref: _exit_1([ref] + a, d, input=text))
         for chunk in ("1", "65536"):
             ours = subprocess.run([_tool("matealign")] + a, input=text, capture_output=True,
                                   env=dict(os.environ, DFB_TOOL_CHUNK_MIN=chunk, DFB_TOOL_THREADS="8"))
-            assert ours.returncode == theirs.returncode == 1, a
-            assert ours.stdout == theirs.stdout and ours.stderr == theirs.stderr, (a, ours.stderr, theirs.stderr)
+            assert ours.returncode == 1, a
+            assert util.digest(ours.stdout.replace(d.encode(), b"<dir>"), ours.stderr.replace(d.encode(), b"<dir>")) == theirs, \
+                (a, ours.stderr)
+
+
+def _exit_1(cmd, d, strip=lambda b: b, input=None):
+    """stdout and stderr of a run that must exit 1, with the dataset directory `d` written as <dir>."""
+    p = subprocess.run(cmd, input=input, capture_output=True)
+    assert p.returncode == 1, cmd
+    return p.stdout.replace(d.encode(), b"<dir>"), strip(p.stderr).replace(d.encode(), b"<dir>")

@@ -1,5 +1,8 @@
 """evalsplitalign (host-only, runs without a GPU) and splitseq (GPU: alignment + backtrace) against the committed
-golden outputs of the compiled reference tools and, where oracle/_ref exists, against those tools on fresh files."""
+golden outputs of the compiled reference tools, and on fresh files against the stored digests of those tools' outputs
+(tests/golden/reference_digests.json; where oracle/_ref exists, the reference tools run as well).  The tools are unchanged
+since they last ran beside the compiled reference tools on these inputs and gave the same bytes; the digests are of those
+outputs."""
 import json
 import os
 import subprocess
@@ -11,6 +14,8 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
 BIN = os.path.join(ROOT, "defuse_b200", "bin")
 sys.path.insert(0, ROOT)
+
+import util  # noqa: E402
 
 
 def _tool(name):
@@ -42,6 +47,15 @@ def _eval(tool, ev, d, tag):
     return {k: open(v).read() for k, v in names.items()}
 
 
+def _eval_bytes(outs):
+    return tuple(outs[k].encode() for k in ("seq", "break", "predalign"))
+
+
+def _output_file(cmd, path, env=None):
+    _run(cmd, env=env)
+    return (open(path, "rb").read(),)
+
+
 def test_evalsplitalign_golden(tmp_path):
     g, d, common, ev = _golden_dataset(tmp_path)
     got = _eval(_tool("evalsplitalign"), ev, d, "ours")
@@ -51,19 +65,25 @@ def test_evalsplitalign_golden(tmp_path):
 
 @pytest.mark.parametrize("kw", [dict(seed=51, n_clusters=80, pairs_per_cluster=50),
                                 dict(seed=52, n_clusters=40, pairs_per_cluster=40, read_len_jitter=20, lower_frac=0.02, n_rate=0.01)])
-def test_evalsplitalign_vs_reference_tool(oracle_mod, tmp_path, kw):
+def test_evalsplitalign_vs_reference_tool(oracle_mod, tmp_path, kw, device_double):
+    """The reference dosplitalign's records, sorted, through our evalsplitalign and the reference's.  Without oracle/_ref
+    the records come from our dosplitalign over the device double, checked against the reference's digest first."""
     from synth import files
-    ref_split, ref_eval = oracle_mod.ref_tool("ref_dosplitalign"), oracle_mod.ref_tool("ref_evalsplitalign")
-    if not ref_split or not ref_eval:
-        pytest.skip("oracle/_ref tools not built")
     d = str(tmp_path / "d")
     args = files.make_split_dataset(d, **kw)
-    _run([ref_split] + args + ["-a", os.path.join(d, "raw.alignments")])
-    files.sort_alignments(os.path.join(d, "raw.alignments"), os.path.join(d, "sorted.alignments"))
+    raw = os.path.join(d, "raw.alignments")
+    want_raw = util.reference_tool_digest(oracle_mod, "dosplitalign_tool/%(seed)d" % kw, "ref_dosplitalign",
+                                          lambda ref: _output_file([ref] + args + ["-a", raw], raw))
+    if not oracle_mod.ref_tool("ref_dosplitalign"):
+        _run([_tool("dosplitalign")] + args + ["-a", raw], env=dict(os.environ, LD_PRELOAD=device_double))
+    assert util.digest(open(raw, "rb").read()) == want_raw
+    files.sort_alignments(raw, os.path.join(d, "sorted.alignments"))
     common, ev = files.downstream_args(args, d)
-    ours, theirs = _eval(_tool("evalsplitalign"), ev, d, "ours"), _eval(ref_eval, ev, d, "ref")
-    assert len(theirs["seq"].splitlines()) > 10
-    assert ours == theirs
+    ours = _eval(_tool("evalsplitalign"), ev, d, "ours")
+    theirs = util.reference_tool_digest(oracle_mod, "evalsplitalign_tool/%(seed)d" % kw, "ref_evalsplitalign",
+                                        lambda ref: _eval_bytes(_eval(ref, ev, d, "ref")))
+    assert len(ours["seq"].splitlines()) > 10
+    assert util.digest(*_eval_bytes(ours)) == theirs
 
 
 def test_evalsplitalign_errors(tmp_path):
@@ -101,22 +121,23 @@ def test_splitseq_vs_reference_tool(oracle_mod, tmp_path, kw):
     reference tools fed the same files.  splitseq is run on the full sorted alignments too (every record re-aligned and
     back-traced), not only on the predicted ones."""
     from synth import files
-    refs = {n: oracle_mod.ref_tool("ref_" + n) for n in ("dosplitalign", "evalsplitalign", "splitseq")}
-    if not all(refs.values()):
-        pytest.skip("oracle/_ref tools not built")
     d = str(tmp_path / "d")
     args = files.make_split_dataset(d, **kw)
     _run([_tool("dosplitalign")] + args + ["-a", os.path.join(d, "raw.alignments")])
     files.sort_alignments(os.path.join(d, "raw.alignments"), os.path.join(d, "sorted.alignments"))
     common, ev = files.downstream_args(args, d)
-    ours, theirs = _eval(_tool("evalsplitalign"), ev, d, "ours"), _eval(refs["evalsplitalign"], ev, d, "ref")
-    assert ours == theirs
+    ours = _eval(_tool("evalsplitalign"), ev, d, "ours")
+    theirs = util.reference_tool_digest(oracle_mod, "evalsplitalign_tool/%(seed)d" % kw, "ref_evalsplitalign",
+                                        lambda ref: _eval_bytes(_eval(ref, ev, d, "ref")))
+    assert util.digest(*_eval_bytes(ours)) == theirs
     prefix = files.write_read_index(d)
-    for name in ("ref.predalign", "sorted.alignments"):
+    for name in ("ours.predalign", "sorted.alignments"):   # (ours.predalign has the reference's bytes: checked above)
         tail = common + ["-p", prefix, "-a", os.path.join(d, name)]
-        a, b = _run([_tool("splitseq")] + tail), _run([refs["splitseq"]] + tail)
-        assert len(b) > 1000
-        assert a == b, name
+        a = _run([_tool("splitseq")] + tail)
+        b = util.reference_tool_digest(oracle_mod, "splitseq_tool/%d/%s" % (kw["seed"], name.split(".")[1]), "ref_splitseq",
+                                       lambda ref: (_run([ref] + tail),))
+        assert len(a) > 1000
+        assert util.digest(a) == b, name
 
 
 @pytest.mark.gpu
@@ -128,17 +149,20 @@ def test_fused_align_evaluate_vs_reference_pipeline(oracle_mod, tmp_path, kw):
     outputs must be byte-identical; with -a the alignments file is still written and equals the reference's; several
     small GPU batches and small evaluation regions give the same bytes."""
     from synth import files
-    ref_split, ref_eval = oracle_mod.ref_tool("ref_dosplitalign"), oracle_mod.ref_tool("ref_evalsplitalign")
-    if not ref_split or not ref_eval:
-        pytest.skip("oracle/_ref tools not built")
     d = str(tmp_path / "d")
     args = files.make_split_dataset(d, **kw)
-    _run([ref_split] + args + ["-a", os.path.join(d, "raw.alignments")])
-    p = subprocess.run("LC_ALL=C sort -n -k 1 %s > %s" % (os.path.join(d, "raw.alignments"), os.path.join(d, "sorted.alignments")), shell=True)
-    assert p.returncode == 0
     common, ev = files.downstream_args(args, d)
-    theirs = _eval(ref_eval, ev, d, "ref")
-    assert len(theirs["seq"].splitlines()) > 10
+
+    def reference_pipeline(ref_split):
+        _run([ref_split] + args + ["-a", os.path.join(d, "raw.alignments")])
+        p = subprocess.run("LC_ALL=C sort -n -k 1 %s > %s" % (os.path.join(d, "raw.alignments"), os.path.join(d, "sorted.alignments")),
+                           shell=True)
+        assert p.returncode == 0
+        return _eval_bytes(_eval(oracle_mod.ref_tool("ref_evalsplitalign"), ev, d, "ref"))
+
+    theirs = util.reference_tool_digest(oracle_mod, "evalsplitalign_pipeline/%(seed)d" % kw, "ref_dosplitalign", reference_pipeline)
+    want_raw = util.reference_tool_digest(oracle_mod, "dosplitalign_tool/%(seed)d" % kw, "ref_dosplitalign",
+                                          lambda ref: (open(os.path.join(d, "raw.alignments"), "rb").read(),))
 
     def fused(tag, extra=(), env=None):
         names = {k: os.path.join(d, "%s.%s" % (tag, k)) for k in ("seq", "break", "predalign")}
@@ -146,10 +170,12 @@ def test_fused_align_evaluate_vs_reference_pipeline(oracle_mod, tmp_path, kw):
              env=dict(os.environ, **env) if env else None)
         return {k: open(v).read() for k, v in names.items()}
 
-    assert fused("fused") == theirs
-    assert fused("fused_a", ["-a", os.path.join(d, "fused.alignments")]) == theirs
-    assert open(os.path.join(d, "fused.alignments"), "rb").read() == open(os.path.join(d, "raw.alignments"), "rb").read()
-    assert fused("fused_small", env={"DFB_TOOL_BATCH": "700", "DFB_TOOL_CHUNK_MIN": "400"}) == theirs
+    got = fused("fused")
+    assert len(got["seq"].splitlines()) > 10
+    assert util.digest(*_eval_bytes(got)) == theirs
+    assert util.digest(*_eval_bytes(fused("fused_a", ["-a", os.path.join(d, "fused.alignments")]))) == theirs
+    assert util.digest(open(os.path.join(d, "fused.alignments"), "rb").read()) == want_raw
+    assert util.digest(*_eval_bytes(fused("fused_small", env={"DFB_TOOL_BATCH": "700", "DFB_TOOL_CHUNK_MIN": "400"}))) == theirs
 
 
 def test_evalsplitalign_score_ties_follow_the_reference_container_order(oracle_mod, tmp_path):
@@ -158,9 +184,6 @@ def test_evalsplitalign_score_ties_follow_the_reference_container_order(oracle_m
     per fusion, summed scores tied on purpose, enough keys to force rehashes.  Host-only, so it runs without a GPU."""
     import numpy as np
     from synth import files
-    ref_eval = oracle_mod.ref_tool("ref_evalsplitalign")
-    if not ref_eval:
-        pytest.skip("oracle/_ref tools not built")
     d = str(tmp_path / "d")
     args = files.make_split_dataset(d, seed=71, n_clusters=40, pairs_per_cluster=2)
     common, ev = files.downstream_args(args, d)
@@ -184,9 +207,11 @@ def test_evalsplitalign_score_ties_follow_the_reference_container_order(oracle_m
     order = rng.permutation(len(lines))
     text = "".join(l for _, l in sorted((lines[k] for k in order), key=lambda x: x[0]))
     open(os.path.join(d, "sorted.alignments"), "w").write(text)
-    ours, theirs = _eval(_tool("evalsplitalign"), ev, d, "ours"), _eval(ref_eval, ev, d, "ref")
-    assert len(theirs["seq"].splitlines()) == 40
-    assert ours == theirs
+    ours = _eval(_tool("evalsplitalign"), ev, d, "ours")
+    theirs = util.reference_tool_digest(oracle_mod, "evalsplitalign_tool/score_ties", "ref_evalsplitalign",
+                                        lambda ref: _eval_bytes(_eval(ref, ev, d, "ref")))
+    assert len(ours["seq"].splitlines()) == 40
+    assert util.digest(*_eval_bytes(ours)) == theirs
 
 
 def _eval_rc(tool, ev, d, tag, env=None):
@@ -214,9 +239,6 @@ def test_evalsplitalign_dies_where_the_reference_dies(oracle_mod, tmp_path):
     evaluates the current one -- a bad first line of a fusion also drops the fusion in front of it.  Same sequence and
     break files as the compiled tool for every cut of the file (prediction records are buffered by the reference and
     lost at exit, so they are not compared)."""
-    ref_eval = oracle_mod.ref_tool("ref_evalsplitalign")
-    if not ref_eval:
-        pytest.skip("oracle/_ref tools not built")
     g, d, common, ev = _golden_dataset(tmp_path)
     lines = g["sorted"].splitlines(keepends=True)
     ids = [l.split("\t")[0] for l in lines]
@@ -228,12 +250,17 @@ def test_evalsplitalign_dies_where_the_reference_dies(oracle_mod, tmp_path):
     for name, at in cases.items():
         bad = lines[:at] + ["12\t3\t0\n"] + lines[at:]
         open(os.path.join(d, "sorted.alignments"), "w").write("".join(bad))
-        pr, theirs = _eval_rc(ref_eval, ev, d, "ref")
-        assert pr.returncode == 1 and b"Format error" in pr.stderr, name
+
+        def reference(ref_eval):
+            pr, theirs = _eval_rc(ref_eval, ev, d, "ref")
+            assert pr.returncode == 1 and b"Format error" in pr.stderr, name
+            stderr = b"".join(l for l in pr.stderr.splitlines(keepends=True) if not l.startswith(b"[fai_load]"))  # samtools' notice
+            return stderr.replace(d.encode(), b"<dir>"), theirs["seq"].encode(), theirs["break"].encode()
+
+        want = util.reference_tool_digest(oracle_mod, "evalsplitalign_tool/dies/" + name, "ref_evalsplitalign", reference)
         for env in (dict(DFB_TOOL_THREADS="1"), dict(DFB_TOOL_THREADS="4", DFB_TOOL_CHUNK_MIN="100"),
                     dict(DFB_TOOL_THREADS="8", DFB_TOOL_CHUNK_MIN="1500")):
             po, ours = _eval_rc(_tool("evalsplitalign"), ev, d, "ours", env)
-            assert po.returncode == 1, (name, env)
-            want = b"".join(l for l in pr.stderr.splitlines(keepends=True) if not l.startswith(b"[fai_load]"))  # samtools' notice
-            assert po.stderr == want, (name, env, po.stderr, want)
-            assert ours["seq"] == theirs["seq"] and ours["break"] == theirs["break"], (name, env)
+            assert po.returncode == 1 and b"Format error" in po.stderr, (name, env)
+            assert util.digest(po.stderr.replace(d.encode(), b"<dir>"), ours["seq"].encode(), ours["break"].encode()) == want, \
+                (name, env, po.stderr)

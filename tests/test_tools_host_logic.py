@@ -16,19 +16,10 @@ import pytest
 
 import test_tools_downstream as td
 import test_tools_gpu as tg
+import util
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
-
-
-@pytest.fixture(scope="session")
-def device_double(tmp_path_factory):
-    out = tmp_path_factory.mktemp("device_double")
-    obj, lib = str(out / "dp_oracle.o"), str(out / "libdevice_double.so")
-    subprocess.run(["gcc", "-O2", "-fPIC", "-c", os.path.join(ROOT, "oracle", "dp_oracle.c"), "-o", obj], check=True)
-    subprocess.run(["g++", "-O2", "-std=c++17", "-fPIC", "-shared", "-I" + os.path.join(ROOT, "include"), "-o", lib,
-                    os.path.join(HERE, "device_double", "device_double.cpp"), obj, "-lpthread", "-Wl,--no-undefined"], check=True)
-    return lib
 
 
 # the compiled reference tool needs half a minute for this one; the two smaller parameter sets stay
@@ -62,7 +53,7 @@ def test_tool_host_logic(body, kwargs, device_double, oracle_mod, tmp_path, monk
         pytest.skip("tools not built")
     monkeypatch.setenv("LD_PRELOAD", device_double)
     monkeypatch.delenv("DFB_DEVICE", raising=False)
-    available = {"oracle_mod": oracle_mod, "tmp_path": tmp_path}
+    available = {"oracle_mod": oracle_mod, "tmp_path": tmp_path, "device_double": device_double}
     args = {k: available[k] for k in inspect.signature(body).parameters if k in available}
     body(**args, **kwargs)
 
@@ -108,8 +99,11 @@ def test_input_fuzz_agrees_with_the_reference_tool(tool, oracle_mod):
     our tool over the device double against the compiled reference tool -- exit codes, outputs, messages."""
     import json
     import sys
-    if not oracle_mod.ref_tool("ref_" + tool) or not os.path.exists(os.path.join(tg.BIN, tool)):
+    if not os.path.exists(os.path.join(tg.BIN, tool)):
         pytest.skip("tools not built")
+    if not oracle_mod.ref_tool("ref_" + tool):
+        # (the reference's outcomes on malformed inputs -- signals, its own DebugCheck messages -- are not ours to derive)
+        pytest.skip("needs the compiled reference tools (oracle/_ref)")
     p = subprocess.run([sys.executable, os.path.join(ROOT, "scripts", "cpu_fuzz_tools.py"), tool, "5", "120", "60"],
                        capture_output=True, timeout=600)
     report = json.loads(p.stdout.decode())
@@ -121,32 +115,32 @@ def test_dosplitalign_baseline_config_0(device_double, oracle_mod, tmp_path, mon
     """BASELINE.json configs[0] ("dosplitalign on synthetic 2k read pairs x 200 planted-fusion breakpoint clusters, 100 bp
     reads"): the whole tool against the compiled reference tool, byte for byte, raw and after the pipeline's sort."""
     from synth import files
-    ref = oracle_mod.ref_tool("ref_dosplitalign")
-    if not ref or not os.path.exists(os.path.join(tg.BIN, "dosplitalign")):
+    if not os.path.exists(os.path.join(tg.BIN, "dosplitalign")):
         pytest.skip("tools not built")
     monkeypatch.setenv("LD_PRELOAD", device_double)
     d = str(tmp_path / "c0")
     args = files.make_split_dataset(d, seed=1, n_clusters=200, pairs_per_cluster=10, L=100, n_chrom=4, genes_per_chrom=10)
     ours, theirs = os.path.join(d, "ours.tmp"), os.path.join(d, "ref.tmp")
+    want = util.reference_tool_digest(oracle_mod, "dosplitalign_tool/baseline_config_0", "ref_dosplitalign",
+                         lambda ref: tg._output_file([ref] + args + ["-a", theirs], theirs))
     tg._run([os.path.join(tg.BIN, "dosplitalign")] + args + ["-a", ours])
-    tg._run([ref] + args + ["-a", theirs])
-    a, b = open(ours).read(), open(theirs).read()
-    assert len(b.splitlines()) > 200 and a == b
+    a = open(ours, "rb").read()
+    assert len(a.splitlines()) > 200 and util.digest(a) == want
 
 
 def test_dosplitalign_stress_shape(device_double, oracle_mod, tmp_path, monkeypatch):
     """BASELINE.json configs[4] shape at file level: 250-bp reads (-n 230 -x 270 with jitter), 600-bp fragments, N and
     lower-case runs in the reference -- windows, candidates and records against the compiled reference tool."""
     from synth import files
-    ref = oracle_mod.ref_tool("ref_dosplitalign")
-    if not ref or not os.path.exists(os.path.join(tg.BIN, "dosplitalign")):
+    if not os.path.exists(os.path.join(tg.BIN, "dosplitalign")):
         pytest.skip("tools not built")
     monkeypatch.setenv("LD_PRELOAD", device_double)
     d = str(tmp_path / "c4")
     args = files.make_split_dataset(d, seed=5, n_clusters=30, pairs_per_cluster=16, L=250, frag_mean=600, read_len_jitter=20,
                                     lower_frac=0.01, n_rate=0.01)
     ours, theirs = os.path.join(d, "ours.tmp"), os.path.join(d, "ref.tmp")
+    want = util.reference_tool_digest(oracle_mod, "dosplitalign_tool/stress_shape", "ref_dosplitalign",
+                         lambda ref: tg._output_file([ref] + args + ["-a", theirs], theirs))
     tg._run([os.path.join(tg.BIN, "dosplitalign")] + args + ["-a", ours])
-    tg._run([ref] + args + ["-a", theirs])
-    a, b = open(ours).read(), open(theirs).read()
-    assert len(b.splitlines()) > 50 and a == b
+    a = open(ours, "rb").read()
+    assert len(a.splitlines()) > 50 and util.digest(a) == want

@@ -1,5 +1,12 @@
-"""Seeded synthetic tasks shared by the parity tests (no reference code involved)."""
+"""Seeded synthetic tasks shared by the parity tests (no reference code involved), and the stored digests of the
+reference's outputs."""
+import hashlib
+import json
+import os
+
 import numpy as np
+
+REFERENCE_DIGESTS = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_digests.json")
 
 ACGT = np.frombuffer(b"ACGT", dtype=np.uint8)
 
@@ -133,3 +140,44 @@ def check_random_parameter_round(rng, rnd, oracle, ctx, check_split, check_simpl
     tr = rng.integers(0, len(refs), len(reads)).astype(np.int32)
     check_simple(oracle, ctx, refs, reads, tr, trd, m, x, g)
     return int(keep.sum()) + len(trd)
+
+
+def digest(*parts):
+    """SHA-256 over byte strings and arrays (with their dtype and shape), in order."""
+    h = hashlib.sha256()
+    for p in parts:
+        if isinstance(p, (bytes, bytearray)):
+            p = np.frombuffer(bytes(p), np.uint8)
+        p = np.ascontiguousarray(p)
+        h.update(("%s%s" % (p.dtype.str, p.shape)).encode())
+        h.update(p.tobytes())
+    return h.hexdigest()
+
+
+def reference_digest(key, compute=None):
+    """The stored digest of the unmodified reference's output for case `key` (tests/golden/reference_digests.json).
+    Where the compiled reference is built (oracle/_ref), `compute` returns the digest of its output now: it must equal
+    the stored one, or replaces it when DFB_RECORD_DIGESTS=1.
+
+    How the file was made: digests of the outputs of the C restatement (oracle/dp_oracle.c) and of the tools
+    (defuse_b200/host, over tests/device_double) at commit f0d5442, where oracle/, synth/, defuse_b200/ and this module
+    were as in the last runs that compared them byte for byte with the compiled reference, and they agreed."""
+    with open(REFERENCE_DIGESTS) as f:
+        stored = json.load(f)
+    if compute is None:
+        return stored[key]
+    d = compute()
+    if os.environ.get("DFB_RECORD_DIGESTS") == "1":
+        stored[key] = d
+        with open(REFERENCE_DIGESTS, "w") as f:
+            json.dump(dict(sorted(stored.items())), f, indent=0)
+    else:
+        assert stored.get(key) == d, "%s: the compiled reference's output differs from its stored digest" % key
+    return d
+
+
+def reference_tool_digest(oracle_mod, key, name, run):
+    """reference_digest() of what the compiled reference tool `name` gives in case `key`: where oracle/_ref has the tool,
+    `run(path)` runs it and returns the byte strings compared (stdout, output files, ...)."""
+    path = oracle_mod.ref_tool(name)
+    return reference_digest(key, (lambda: digest(*run(path))) if path else None)
