@@ -208,7 +208,7 @@ struct dfb_ctx
 	PinnedBuf h_out;             // results on their way back
 	cudaStream_t copy_stream = nullptr; // device->host result copies, ordered after a plan's kernels by an event
 	cudaStream_t upload_stream = nullptr; // uploads + packing of the next chunk of a pipelined batch
-	cudaStream_t upload_stream2 = nullptr; // device-built chunks alternate between the two: chunk k+1's uploads do not hold up chunk k's packing
+	cudaStream_t upload_stream2 = nullptr; // host-built chunks alternate between the two: chunk k+1's uploads do not hold up chunk k's packing
 	// first-sweep state (checkpoints, probe targets, read symbols) of the chunk of a pipelined batch that is on the GPU:
 	// ONE buffer for all chunks and batches -- chunk k+1's first sweep is queued behind chunk k's probe sweep on the compute
 	// stream, so they never overlap --, grown when a chunk needs more.  (Allocated per chunk, a chunk slightly larger than
@@ -973,15 +973,9 @@ static cudaError_t h2d_any(dfb_ctx* ctx, cudaStream_t up, void* dst, const void*
 		else if ((e = cudaEventSynchronize(ctx->ring_ev[slot])) != cudaSuccess) return e; // the block's last transfer is over
 		uint8_t* stage = (uint8_t*)ctx->h_ring.p + (size_t)slot * dfb_ctx::kRingBlock;
 		const uint8_t* from = (const uint8_t*)src + off;
-		// (a thread per megabyte of the block; a thread per 512 or 256 KB -- DFB_STAGE_SHIFT=19 / 18 -- made the matealign shape
-		// from pageable arrays slower, 36 against 32 ms: call r04l)
-		static int shift = 0;
-		if (!shift)
-		{
-			const char* e = getenv("DFB_STAGE_SHIFT");
-			shift = (e && atoi(e) >= 12 && atoi(e) <= 24) ? atoi(e) : 20;
-		}
-		const int T = (int)std::max<size_t>(1, std::min<size_t>((size_t)ctx->host_threads, n >> shift));
+		// (a thread per megabyte of the block; a thread per 512 or 256 KB made the matealign shape from pageable arrays
+		// slower, 36 against 32 ms: call r04l)
+		const int T = (int)std::max<size_t>(1, std::min<size_t>((size_t)ctx->host_threads, n >> 20));
 		parallel_for(ctx->pool, T, [&](int tid) {
 			const size_t a = n * (size_t)tid / (size_t)T, b = n * ((size_t)tid + 1) / (size_t)T;
 			memcpy(stage + a, from + a, b - a);
@@ -1212,47 +1206,50 @@ static int finish_create(dfb_plan* pl)
 	return DFB_OK;
 }
 
-// ---- SimpleAligner plan ------------------------------------------------------------------
+// ---- job lists built on the host ------------------------------------------------------------------
 
-// `refs` / `seqs` may be views into larger tables (off[0] != 0) whose first entries are reference `ref_base` / sequence
-// `seq_base` of the caller's numbering; `async` skips the final stream synchronisation and uploads on the upload
-// stream (chunks of a pipelined batch).
-static int simple_plan_create_impl(dfb_ctx* ctx, const dfb_simple_params* params, const dfb_seq_table* refs,
-                                   const dfb_seq_table* seqs, const int32_t* task_ref, const int32_t* task_seq,
-                                   int64_t n_tasks, int32_t ref_base, int32_t seq_base, int stage_slot, cudaStream_t up_stream, dfb_plan** out)
+// One builder for both aligners (`simple`: SimpleAligner).  Table A holds the references (simple) or two windows per
+// cluster (split), table B the sequences or reads; task_a / task_b name an entry of each, task_min_score is null for
+// simple, whose `params` carry the scoring triple only.  Either table may be a view into a larger one (off[0] != 0)
+// whose first entry is number `a_base` / `b_base` of the caller's numbering.  `up_stream` null: uploads on the compute
+// stream and a final synchronisation; else uploads on `up_stream` and none (chunks of a pipelined batch).
+static int plan_create_host(dfb_ctx* ctx, bool simple, const dfb_split_params* params, const dfb_seq_table* A,
+                            const dfb_seq_table* B, const int32_t* task_a, const int32_t* task_b, const int32_t* task_min_score,
+                            int64_t n_tasks, int32_t a_base, int32_t b_base, int stage_slot, cudaStream_t up_stream, dfb_plan** out)
 {
-	const bool async = up_stream != nullptr;
 	*out = nullptr;
 	int rc;
 	CK(ctx, cudaSetDevice(ctx->device));
 	dfb_plan* pl = new (std::nothrow) dfb_plan();
 	if (!pl) return set_err(ctx, DFB_ERR_NOMEM, "out of host memory");
+	auto fail = [&](int code) {
+		dfb_plan_destroy(pl);
+		return code;
+	};
 	pl->ctx = ctx;
-	pl->split = false;
+	pl->split = !simple;
+	pl->early_release = !simple && up_stream; // (a chunk of a pipelined batch: its sweep state lives in the context's arena)
+	pl->sp = *params;
 	pl->n_tasks = n_tasks;
 	pl->stats.n_tasks = n_tasks;
-	pl->sp.match = params->match;
-	pl->sp.mismatch = params->mismatch;
-	pl->sp.gap = params->gap;
-	classify_params(pl, params->match, params->mismatch, params->gap, true);
+	classify_params(pl, params->match, params->mismatch, params->gap, simple || (params->end_gaps == 0 && params->min_split_score >= 1));
 	pl->up = up_stream;
 	Trace tr;
-	if ((rc = upload_raw(pl, refs, seqs)))
-	{
-		dfb_plan_destroy(pl);
-		return rc;
-	}
-	tr.lap("simple.create: raw upload");
+	if ((rc = upload_raw(pl, A, B))) return fail(rc);
+	tr.lap("host build: raw upload");
 
-	// pass 1 (host threads): classify every task, count per (thread, class, reference-length bin)
+	// pass 1 (host threads): class and reference-length bin of every task, per-thread bin counts
+	const int64_t n_a = simple ? A->n : A->n / 2; // references / clusters
 	const int T = (int)std::max<int64_t>(1, std::min<int64_t>(ctx->host_threads, n_tasks / 65536 + 1));
 	const size_t n_bins = (size_t)kNumClasses * kRBins;
 	std::vector<int32_t> bin_of((size_t)n_tasks);
-	std::vector<int64_t> bin_pos(n_bins * (size_t)T, 0);
+	std::vector<int64_t> bin_pos(n_bins * (size_t)T, 0); // [thread][bin]
+	if (!simple) pl->task_L.resize((size_t)n_tasks);
 	struct Part
 	{
 		int64_t cells = 0, n_gen = 0, bad = -1;
 		uint32_t gen_max_R = 0;
+		uint32_t cls_max_R[kNumClasses] = {0};
 	};
 	std::vector<Part> part((size_t)T);
 	parallel_for(ctx->pool, T, [&](int tid) {
@@ -1260,18 +1257,25 @@ static int simple_plan_create_impl(dfb_ctx* ctx, const dfb_simple_params* params
 		int64_t* cnt = bin_pos.data() + n_bins * (size_t)tid;
 		for (int64_t t = n_tasks * tid / T; t < n_tasks * (tid + 1) / T; t++)
 		{
-			const int32_t r = task_ref[t] - ref_base, sq = task_seq[t] - seq_base;
-			if (r < 0 || r >= refs->n || sq < 0 || sq >= seqs->n)
+			const int64_t ia = (int64_t)task_a[t] - a_base, ib = (int64_t)task_b[t] - b_base;
+			if (ia < 0 || ia >= n_a || ib < 0 || ib >= B->n)
 			{
 				if (pt.bad < 0) pt.bad = t;
 				bin_of[t] = -1;
 				continue;
 			}
-			const int64_t R = refs->off[r + 1] - refs->off[r];
-			const int64_t L = seqs->off[sq + 1] - seqs->off[sq];
-			pt.cells += R * L;
-			int32_t bin = -1; // no interior cell: score 0 (d_out is zero-initialised)
-			if (R > 0 && L > 0)
+			// simple: the reference (R1); split: both windows, the longer one decides the bin and the class limit
+			const int64_t a0 = simple ? ia : 2 * ia;
+			const int64_t R1 = A->off[a0 + 1] - A->off[a0];
+			const int64_t R2 = simple ? 0 : A->off[a0 + 2] - A->off[a0 + 1];
+			const int64_t R = std::max(R1, R2);
+			const int64_t L = B->off[ib + 1] - B->off[ib];
+			if (!simple) pl->task_L[t] = (int32_t)L;
+			pt.cells += (R1 + R2) * L;
+			// no DP cell -- simple: score 0 (d_out is zero-initialised); split: an empty read, every row maximum is 0, no
+			// split (SplitReadAligner.cpp:224-227)
+			int32_t bin = -1;
+			if (L > 0 && (R > 0 || !simple))
 			{
 				int c = (L <= kMaxFastRows && R <= 65535) ? class_for_rows((int)L) : -1;
 				if (c >= 0 && !pl->fast_ok[c]) c = -1;
@@ -1285,27 +1289,24 @@ static int simple_plan_create_impl(dfb_ctx* ctx, const dfb_simple_params* params
 				{
 					bin = c * kRBins + (kRBins - 1 - (int)std::min<int64_t>(R >> 4, kRBins - 1));
 					cnt[bin]++;
+					pt.cls_max_R[c] = std::max<uint32_t>(pt.cls_max_R[c], (uint32_t)R);
 				}
 			}
 			bin_of[t] = bin;
 		}
 	});
-	int64_t n_gen = 0;
+	int64_t n_gen_tasks = 0;
 	uint32_t gen_max_R = 0;
 	for (int k = 0; k < T; k++)
 	{
-		if (part[(size_t)k].bad >= 0)
-		{
-			const long long bad = (long long)part[(size_t)k].bad;
-			dfb_plan_destroy(pl);
-			return set_err(ctx, DFB_ERR_ARG, "task %lld: table index out of range", bad);
-		}
+		if (part[(size_t)k].bad >= 0) return fail(set_err(ctx, DFB_ERR_ARG, "task %lld: table index out of range", (long long)part[(size_t)k].bad));
 		pl->stats.cells += part[(size_t)k].cells;
-		n_gen += part[(size_t)k].n_gen;
+		n_gen_tasks += part[(size_t)k].n_gen;
 		gen_max_R = std::max(gen_max_R, part[(size_t)k].gen_max_R);
+		for (int c = 0; c < kNumClasses; c++) pl->cls[c].max_R = std::max(pl->cls[c].max_R, part[(size_t)k].cls_max_R[c]);
 	}
-	// two tasks share a job (low / high half): task position p inside its class -> job p/2, half p%2.
-	// counts -> positions: class by class, bin by bin, thread by thread (keeps task order inside a bin)
+	// counts -> positions inside the class: class by class, bin by bin, thread by thread (keeps task order inside a bin).
+	// Simple: two tasks share a job (low / high half), task position p -> job p/2, half p%2.  Split: a job per task.
 	int64_t n_jobs_cls[kNumClasses], job_base[kNumClasses];
 	int64_t n_fast_jobs = 0;
 	for (int c = 0; c < kNumClasses; c++)
@@ -1320,296 +1321,99 @@ static int simple_plan_create_impl(dfb_ctx* ctx, const dfb_simple_params* params
 				tasks_c += cnt;
 			}
 		job_base[c] = n_fast_jobs;
-		n_jobs_cls[c] = (tasks_c + 1) / 2;
+		n_jobs_cls[c] = simple ? (tasks_c + 1) / 2 : tasks_c;
 		n_fast_jobs += n_jobs_cls[c];
 	}
+	const int64_t gen_per_task = simple ? 1 : 2; // split: one generic job per window
+	tr.lap("host build: classify");
 
-	tr.lap("simple.create: classify");
 	Staging st;
-	cudaError_t e = stage_layout(ctx, stage_slot, st, refs->n, seqs->n, n_fast_jobs, n_gen);
-	if (e != cudaSuccess)
-	{
-		dfb_plan_destroy(pl);
-		return set_err(ctx, DFB_ERR_NOMEM, "pinned staging buffer: %s", cudaGetErrorString(e));
-	}
-	tr.lap("simple.create: staging");
+	cudaError_t e = stage_layout(ctx, stage_slot, st, A->n, B->n, n_fast_jobs, gen_per_task * n_gen_tasks);
+	if (e != cudaSuccess) return fail(set_err(ctx, DFB_ERR_NOMEM, "pinned staging buffer: %s", cudaGetErrorString(e)));
+	// split: reference 1 of every cluster forward, reference 2 reversed (SplitReadAligner.cpp:80-81); every read forward
+	// and reversed (:84-85)
+	const int mode_a = simple ? PACK_FWD : PACK_REV_ODD, mode_b = simple ? PACK_FWD : PACK_BOTH;
 	uint32_t words_a_end = 0;
 	bool overflow = false;
-	const uint32_t total_words = layout_words(ctx, refs, PACK_FWD, seqs, PACK_FWD, st.desc_a, st.desc_b, &words_a_end, &overflow);
-	if (overflow)
-	{
-		dfb_plan_destroy(pl);
-		return set_err(ctx, DFB_ERR_ARG, "batch too large: more than 2^32 packed words; split it");
-	}
-	// pass 2 (host threads): place every task into its job slot
-	parallel_for(ctx->pool, T, [&](int tid) {
-		for (int64_t j = n_fast_jobs * tid / T; j < n_fast_jobs * (tid + 1) / T; j++)
-		{
-			JobPair& jp = st.jobs[j];
-			memset(&jp, 0, sizeof(jp));
-			jp.out0 = jp.out1 = -1;
-		}
-	});
+	const uint32_t total_words = layout_words(ctx, A, mode_a, B, mode_b, st.desc_a, st.desc_b, &words_a_end, &overflow);
+	if (overflow) return fail(set_err(ctx, DFB_ERR_ARG, "batch too large: more than 2^32 packed words; split it"));
+	tr.lap("host build: layout");
+	// pass 2 (host threads): every task into its job slot
+	if (simple)
+		parallel_for(ctx->pool, T, [&](int tid) {
+			for (int64_t j = n_fast_jobs * tid / T; j < n_fast_jobs * (tid + 1) / T; j++)
+			{
+				JobPair& jp = st.jobs[j];
+				memset(&jp, 0, sizeof(jp));
+				jp.out0 = jp.out1 = -1;
+			}
+		});
 	parallel_for(ctx->pool, T, [&](int tid) {
 		int64_t* pos = bin_pos.data() + n_bins * (size_t)tid;
 		for (int64_t t = n_tasks * tid / T; t < n_tasks * (tid + 1) / T; t++)
 		{
 			const int32_t bin = bin_of[t];
 			if (bin < 0) continue;
-			const int32_t r = task_ref[t] - ref_base, sq = task_seq[t] - seq_base;
+			const int64_t ia = (int64_t)task_a[t] - a_base;
+			const SeqDesc& bd = st.desc_b[task_b[t] - b_base];
 			const int64_t p = pos[bin]++;
-			JobPair& jp = st.jobs[job_base[bin / kRBins] + (p >> 1)];
-			const int h = (int)(p & 1);
-			jp.ref_w[h] = st.desc_a[r].word;
-			jp.read_w[h] = st.desc_b[sq].word;
-			jp.R[h] = (uint16_t)st.desc_a[r].len;
-			jp.L[h] = (uint16_t)st.desc_b[sq].len;
-			if (h == 0) jp.out0 = (int32_t)t; else jp.out1 = (int32_t)t;
+			const int64_t j0 = job_base[bin / kRBins];
+			if (simple)
+			{
+				JobPair& jp = st.jobs[j0 + (p >> 1)];
+				const int h = (int)(p & 1);
+				jp.ref_w[h] = st.desc_a[ia].word;
+				jp.read_w[h] = bd.word;
+				jp.R[h] = (uint16_t)st.desc_a[ia].len;
+				jp.L[h] = (uint16_t)bd.len;
+				if (h == 0) jp.out0 = (int32_t)t; else jp.out1 = (int32_t)t;
+			}
+			else
+			{
+				JobPair& jp = st.jobs[j0 + p];
+				jp.ref_w[0] = st.desc_a[2 * ia].word;
+				jp.ref_w[1] = st.desc_a[2 * ia + 1].word;
+				jp.read_w[0] = bd.word;
+				jp.read_w[1] = bd.word + (bd.len + 15) / 16;
+				jp.R[0] = (uint16_t)st.desc_a[2 * ia].len;
+				jp.R[1] = (uint16_t)st.desc_a[2 * ia + 1].len;
+				jp.L[0] = jp.L[1] = (uint16_t)bd.len;
+				jp.out0 = (int32_t)t;
+				jp.out1 = task_min_score[t];
+			}
 		}
 	});
-	if (n_gen)
+	int64_t gi = 0;
+	for (int64_t t = 0; n_gen_tasks && t < n_tasks; t++)
 	{
-		int64_t gi = 0;
-		for (int64_t t = 0; t < n_tasks; t++)
+		if (bin_of[t] != -2) continue;
+		const int64_t ia = (int64_t)task_a[t] - a_base;
+		const SeqDesc& bd = st.desc_b[task_b[t] - b_base];
+		for (int h = 0; h < gen_per_task; h++)
 		{
-			if (bin_of[t] != -2) continue;
-			const int32_t r = task_ref[t] - ref_base, sq = task_seq[t] - seq_base;
+			const SeqDesc& ad = st.desc_a[simple ? ia : 2 * ia + h];
 			GenJob& j = st.gen[gi++];
-			j.ref_w = st.desc_a[r].word;
-			j.read_w = st.desc_b[sq].word;
-			j.R = st.desc_a[r].len;
-			j.L = st.desc_b[sq].len;
+			j.ref_w = ad.word;
+			j.read_w = h ? bd.word + (bd.len + 15) / 16 : bd.word;
+			j.R = ad.len;
+			j.L = bd.len;
 			j.task = (int32_t)t;
-			j.half = 0;
+			j.half = h;
 			j.row_off = 0;
-		}
-	}
-	pl->n_gen_jobs = n_gen;
-	tr.lap("simple.create: jobs");
-
-	rc = upload_and_pack(pl, refs, PACK_FWD, seqs, PACK_FWD, st, words_a_end, total_words);
-	tr.lap("simple.create: enqueue pack");
-	if (!rc) rc = alloc_work(pl, (JobPair*)(pl->d_stage + st.off_jobs), (GenJob*)(pl->d_stage + st.off_gen), n_jobs_cls, false, gen_max_R);
-	tr.lap("simple.create: alloc");
-	if (!rc)
-	{
-		for (int c = 0; c < kNumClasses; c++)
-			if (pl->cls[c].n_jobs) fill_fast_params(pl, c, params->match, params->mismatch, params->gap, 0);
-		if (!async) rc = finish_create(pl);
-	}
-	tr.lap("simple.create: sync");
-	if (rc)
-	{
-		dfb_plan_destroy(pl);
-		return rc;
-	}
-	*out = pl;
-	return DFB_OK;
-}
-
-static int dfb_simple_plan_create_body(dfb_ctx* ctx, const dfb_simple_params* params, const dfb_seq_table* refs,
-                                      const dfb_seq_table* seqs, const int32_t* task_ref, const int32_t* task_seq,
-                                      int64_t n_tasks, dfb_plan** out)
-{
-	if (!ctx) return DFB_ERR_ARG;
-	if (!params || !out || n_tasks < 0 || (n_tasks > 0 && (!task_ref || !task_seq)))
-		return set_err(ctx, DFB_ERR_ARG, "dfb_simple_plan_create: null argument");
-	*out = nullptr;
-	int rc;
-	if ((rc = check_table(ctx, refs, "refs")) || (rc = check_table(ctx, seqs, "seqs"))) return rc;
-	if (n_tasks > 0x7fffff00LL) return set_err(ctx, DFB_ERR_ARG, "too many tasks in one batch");
-	return simple_plan_create_impl(ctx, params, refs, seqs, task_ref, task_seq, n_tasks, 0, 0, 0, nullptr, out);
-}
-
-// ---- SplitReadAligner plan ------------------------------------------------------------------
-
-// `reads` may be a view into a larger table (off[0] != 0) whose first entry is read `read_base` of the caller's
-// numbering, `refs` likewise a view whose first window pair is cluster `cluster_base`; `async` skips the final
-// stream synchronisation (chunks of a pipelined batch).
-static int split_plan_create_impl(dfb_ctx* ctx, const dfb_split_params* params, const dfb_seq_table* refs,
-                                  const dfb_seq_table* reads, const int32_t* task_cluster, const int32_t* task_read,
-                                  const int32_t* task_min_score, int64_t n_tasks, int32_t read_base, int stage_slot,
-                                  bool async, dfb_plan** out, int32_t cluster_base = 0)
-{
-	*out = nullptr;
-	int rc;
-	const int64_t n_clusters = refs->n / 2;
-	CK(ctx, cudaSetDevice(ctx->device));
-	dfb_plan* pl = new (std::nothrow) dfb_plan();
-	if (!pl) return set_err(ctx, DFB_ERR_NOMEM, "out of host memory");
-	pl->ctx = ctx;
-	pl->split = true;
-	pl->early_release = async; // (a chunk of a pipelined batch: its sweep state lives in the context's arena)
-	pl->sp = *params;
-	pl->n_tasks = n_tasks;
-	pl->stats.n_tasks = n_tasks;
-	classify_params(pl, params->match, params->mismatch, params->gap, params->end_gaps == 0 && params->min_split_score >= 1);
-	pl->up = async ? ((stage_slot & 1) ? ctx->upload_stream2 : ctx->upload_stream) : nullptr;
-	if ((rc = upload_raw(pl, refs, reads)))
-	{
-		dfb_plan_destroy(pl);
-		return rc;
-	}
-
-	Trace tr;
-	// pass 1 (host threads): class and reference-length bin of every task, per-thread bin counts
-	const int T = (int)std::max<int64_t>(1, std::min<int64_t>(ctx->host_threads, n_tasks / 65536 + 1));
-	const size_t n_bins = (size_t)kNumClasses * kRBins;
-	std::vector<int32_t> bin_of((size_t)n_tasks);
-	std::vector<int64_t> bin_pos(n_bins * (size_t)T, 0); // [thread][bin]
-	pl->task_L.resize((size_t)n_tasks);
-	struct Part
-	{
-		int64_t cells = 0, n_gen = 0, bad = -1;
-		uint32_t gen_max_R = 0;
-		uint32_t cls_max_R[kNumClasses] = {0};
-	};
-	std::vector<Part> part((size_t)T);
-	parallel_for(ctx->pool, T, [&](int tid) {
-		const int64_t t0 = n_tasks * tid / T, t1 = n_tasks * (tid + 1) / T;
-		Part& pt = part[tid];
-		int64_t* cnt = bin_pos.data() + n_bins * (size_t)tid;
-		for (int64_t t = t0; t < t1; t++)
-		{
-			const int64_t c0 = (int64_t)task_cluster[t] - cluster_base, rd = (int64_t)task_read[t] - read_base;
-			if (c0 < 0 || c0 >= n_clusters || rd < 0 || rd >= reads->n)
+			if (!simple)
 			{
-				if (pt.bad < 0) pt.bad = t;
-				bin_of[t] = -1;
-				continue;
-			}
-			const int64_t c2 = 2 * (int64_t)c0;
-			const int64_t R1 = refs->off[c2 + 1] - refs->off[c2];
-			const int64_t R2 = refs->off[c2 + 2] - refs->off[c2 + 1];
-			const int64_t L = reads->off[rd + 1] - reads->off[rd];
-			pl->task_L[t] = (int32_t)L;
-			pt.cells += (R1 + R2) * L;
-			int32_t bin = -1; // empty read: every row maximum is 0, no split (SplitReadAligner.cpp:224-227)
-			if (L > 0)
-			{
-				int c = (L <= kMaxFastRows && R1 <= 65535 && R2 <= 65535) ? class_for_rows((int)L) : -1;
-				if (c >= 0 && !pl->fast_ok[c]) c = -1;
-				if (c < 0)
-				{
-					bin = -2;
-					pt.n_gen++;
-					pt.gen_max_R = std::max<uint32_t>(pt.gen_max_R, (uint32_t)std::max(R1, R2));
-				}
-				else
-				{
-					bin = c * kRBins + (kRBins - 1 - (int)std::min<int64_t>(std::max(R1, R2) >> 4, kRBins - 1));
-					cnt[bin]++;
-					pt.cls_max_R[c] = std::max<uint32_t>(pt.cls_max_R[c], (uint32_t)std::max(R1, R2));
-				}
-			}
-			bin_of[t] = bin;
-		}
-	});
-	int64_t n_gen_tasks = 0;
-	uint32_t gen_max_R = 0;
-	for (int k = 0; k < T; k++)
-	{
-		if (part[k].bad >= 0)
-		{
-			const long long bad = (long long)part[k].bad;
-			dfb_plan_destroy(pl);
-			return set_err(ctx, DFB_ERR_ARG, "task %lld: table index out of range", bad);
-		}
-		pl->stats.cells += part[k].cells;
-		n_gen_tasks += part[k].n_gen;
-		gen_max_R = std::max(gen_max_R, part[k].gen_max_R);
-		for (int c = 0; c < kNumClasses; c++) pl->cls[c].max_R = std::max(pl->cls[c].max_R, part[k].cls_max_R[c]);
-	}
-	// counts -> write positions: class by class, bin by bin, thread by thread (keeps task order inside a bin)
-	int64_t n_jobs_cls[kNumClasses];
-	int64_t n_fast_jobs = 0;
-	for (int c = 0; c < kNumClasses; c++)
-	{
-		int64_t in_class = 0;
-		for (int b = 0; b < kRBins; b++)
-		{
-			for (int k = 0; k < T; k++)
-			{
-				int64_t& slot = bin_pos[n_bins * (size_t)k + (size_t)c * kRBins + b];
-				const int64_t cnt = slot;
-				slot = n_fast_jobs + in_class;
-				in_class += cnt;
-			}
-		}
-		n_jobs_cls[c] = in_class;
-		n_fast_jobs += in_class;
-	}
-
-	tr.lap("split.create: classify");
-	Staging st;
-	cudaError_t e = stage_layout(ctx, stage_slot, st, refs->n, reads->n, n_fast_jobs, 2 * n_gen_tasks);
-	if (e != cudaSuccess)
-	{
-		dfb_plan_destroy(pl);
-		return set_err(ctx, DFB_ERR_NOMEM, "pinned staging buffer: %s", cudaGetErrorString(e));
-	}
-	// reference 1 of every cluster forward, reference 2 reversed (SplitReadAligner.cpp:80-81);
-	// every read forward and reversed (:84-85)
-	uint32_t words_a_end = 0;
-	bool overflow = false;
-	const uint32_t total_words = layout_words(ctx, refs, PACK_REV_ODD, reads, PACK_BOTH, st.desc_a, st.desc_b, &words_a_end, &overflow);
-	if (overflow)
-	{
-		dfb_plan_destroy(pl);
-		return set_err(ctx, DFB_ERR_ARG, "batch too large: more than 2^32 packed words; split it");
-	}
-	tr.lap("split.create: layout");
-	// pass 2 (host threads): every task into its job slot
-	parallel_for(ctx->pool, T, [&](int tid) {
-		const int64_t t0 = n_tasks * tid / T, t1 = n_tasks * (tid + 1) / T;
-		int64_t* pos = bin_pos.data() + n_bins * (size_t)tid;
-		for (int64_t t = t0; t < t1; t++)
-		{
-			const int32_t bin = bin_of[t];
-			if (bin < 0) continue;
-			const int64_t c2 = 2 * ((int64_t)task_cluster[t] - cluster_base);
-			const SeqDesc& rdd = st.desc_b[task_read[t] - read_base];
-			JobPair& jp = st.jobs[pos[bin]++];
-			jp.ref_w[0] = st.desc_a[c2].word;
-			jp.ref_w[1] = st.desc_a[c2 + 1].word;
-			jp.read_w[0] = rdd.word;
-			jp.read_w[1] = rdd.word + (rdd.len + 15) / 16;
-			jp.R[0] = (uint16_t)st.desc_a[c2].len;
-			jp.R[1] = (uint16_t)st.desc_a[c2 + 1].len;
-			jp.L[0] = jp.L[1] = (uint16_t)rdd.len;
-			jp.out0 = (int32_t)t;
-			jp.out1 = task_min_score[t];
-		}
-	});
-	if (n_gen_tasks)
-	{
-		int64_t gi = 0;
-		for (int64_t t = 0; t < n_tasks; t++)
-		{
-			if (bin_of[t] != -2) continue;
-			const int64_t c2 = 2 * ((int64_t)task_cluster[t] - cluster_base);
-			const SeqDesc& rdd = st.desc_b[task_read[t] - read_base];
-			const uint32_t rev_w = rdd.word + (rdd.len + 15) / 16;
-			for (int h = 0; h < 2; h++)
-			{
-				GenJob& j = st.gen[gi++];
-				j.ref_w = st.desc_a[c2 + h].word;
-				j.read_w = h ? rev_w : rdd.word;
-				j.R = st.desc_a[c2 + h].len;
-				j.L = rdd.len;
-				j.task = (int32_t)t;
-				j.half = h;
+				// (split: the row maxima of both windows, one row list per job)
 				j.row_off = pl->gen_rows_total;
 				pl->gen_rows_total += (int64_t)j.L + 1;
 			}
 		}
 	}
-	pl->n_gen_jobs = 2 * n_gen_tasks;
-	tr.lap("split.create: jobs");
+	pl->n_gen_jobs = gi;
+	tr.lap("host build: jobs");
 
-	rc = upload_and_pack(pl, refs, PACK_REV_ODD, reads, PACK_BOTH, st, words_a_end, total_words);
-	tr.lap("split.create: enqueue h2d+pack");
-	if (!rc)
+	rc = upload_and_pack(pl, A, mode_a, B, mode_b, st, words_a_end, total_words);
+	tr.lap("host build: enqueue h2d+pack");
+	if (!rc && !simple)
 	{
 		pl->ev_cap = (unsigned long long)std::max<int64_t>(n_tasks, 1 << 20);
 		cudaError_t e2 = dalloc(ctx, (void**)&pl->d_events, (size_t)pl->ev_cap * sizeof(Event));
@@ -1623,53 +1427,83 @@ static int split_plan_create_impl(dfb_ctx* ctx, const dfb_split_params* params, 
 		}
 		if (e2 != cudaSuccess) rc = set_err(ctx, DFB_ERR_CUDA, "output allocation failed: %s", cudaGetErrorString(e2));
 	}
-	if (!rc) rc = alloc_work(pl, (JobPair*)(pl->d_stage + st.off_jobs), (GenJob*)(pl->d_stage + st.off_gen), n_jobs_cls, true, gen_max_R);
+	if (!rc) rc = alloc_work(pl, (JobPair*)(pl->d_stage + st.off_jobs), (GenJob*)(pl->d_stage + st.off_gen), n_jobs_cls, !simple, gen_max_R);
 	if (!rc)
 	{
 		for (int c = 0; c < kNumClasses; c++)
 			if (pl->cls[c].n_jobs)
-				fill_fast_params(pl, c, params->match, params->mismatch, params->gap, params->min_split_score);
-		tr.lap("split.create: alloc");
-		if (!async) rc = finish_create(pl);
-		tr.lap("split.create: sync");
+				fill_fast_params(pl, c, params->match, params->mismatch, params->gap, simple ? 0 : params->min_split_score);
+		tr.lap("host build: alloc");
+		if (!up_stream) rc = finish_create(pl);
+		tr.lap("host build: sync");
 	}
-	if (rc)
-	{
-		dfb_plan_destroy(pl);
-		return rc;
-	}
+	if (rc) return fail(rc);
 	*out = pl;
 	return DFB_OK;
 }
 
-// ---- SplitReadAligner plan, job lists built on the device (dfb_build.cuh) ---------------------------------------
-// Chunks of a pipelined batch: the caller's offsets and task arrays are uploaded as they are; descriptors, class /
-// length bins and the 32-byte job records are made by kernels on the upload stream.  One small read-back (jobs per
-// class, longest reference per class, total pool words) separates the classify pass from the allocations that
-// depend on it.  Returns DFB_BUILD_ON_HOST when the chunk holds tasks only the s32 kernels can take: the caller
-// builds that chunk on the host instead.
-static const int DFB_BUILD_ON_HOST = 1000;
-
-// Upload stream of device-built chunk k.  These streams carry copies only, so one stream serves every chunk in order
-// and chunk 0's upload has the link to itself (two alternating streams share it: the first sweep of a batch started
-// 0.4 ms later on the split path, 5 ms later at the matealign shape).  DFB_UPLOAD_STREAMS=2 alternates (A/B runs).
-static cudaStream_t device_build_upload_stream(dfb_ctx* ctx, int k)
+// The argument checks of a batch, shared by the resident plan and the one-call form of each aligner
+static int check_simple_args(dfb_ctx* ctx, const dfb_simple_params* params, const dfb_seq_table* refs, const dfb_seq_table* seqs,
+                             const int32_t* task_ref, const int32_t* task_seq, int64_t n_tasks)
 {
-	static int n = -1;
-	if (n < 0)
-	{
-		const char* e = getenv("DFB_UPLOAD_STREAMS");
-		n = (e && atoi(e) == 2) ? 2 : 1;
-	}
-	return (n == 2 && (k & 1)) ? ctx->upload_stream2 : ctx->upload_stream;
+	if (!params || n_tasks < 0 || (n_tasks > 0 && (!task_ref || !task_seq)))
+		return set_err(ctx, DFB_ERR_ARG, "dfb_simple_plan_create: null argument");
+	int rc;
+	if ((rc = check_table_parallel(ctx, refs, "refs")) || (rc = check_table_parallel(ctx, seqs, "seqs"))) return rc;
+	if (n_tasks > 0x7fffff00LL) return set_err(ctx, DFB_ERR_ARG, "too many tasks in one batch");
+	return DFB_OK;
 }
 
-// (`simple`: a SimpleAligner batch -- task_cluster names the reference, task_min_score is null, `params` carries the scoring
-// triple only, `ref_base` is the first reference of the view)
-static int split_build_enqueue(dfb_ctx* ctx, const dfb_split_params* params, const dfb_seq_table* refs,
-                               const dfb_seq_table* reads, const int32_t* task_cluster, const int32_t* task_read,
-                               const int32_t* task_min_score, int64_t n_tasks, int32_t read_base, int stage_slot, cudaStream_t up_stream,
-                               dfb_plan** out, bool simple = false, int32_t ref_base = 0)
+static int check_split_args(dfb_ctx* ctx, const dfb_split_params* params, const dfb_seq_table* refs, const dfb_seq_table* reads,
+                            const int32_t* task_cluster, const int32_t* task_read, const int32_t* task_min_score, int64_t n_tasks)
+{
+	if (!params || n_tasks < 0 || (n_tasks > 0 && (!task_cluster || !task_read || !task_min_score)))
+		return set_err(ctx, DFB_ERR_ARG, "dfb_split_plan_create: null argument");
+	int rc;
+	if ((rc = check_table_parallel(ctx, refs, "refs")) || (rc = check_table_parallel(ctx, reads, "reads"))) return rc;
+	if (refs->n & 1) return set_err(ctx, DFB_ERR_ARG, "refs must hold two windows per cluster (n is odd)");
+	if (n_tasks > 0x7fffff00LL) return set_err(ctx, DFB_ERR_ARG, "too many tasks in one batch");
+	return DFB_OK;
+}
+
+static int dfb_simple_plan_create_body(dfb_ctx* ctx, const dfb_simple_params* params, const dfb_seq_table* refs,
+                                      const dfb_seq_table* seqs, const int32_t* task_ref, const int32_t* task_seq,
+                                      int64_t n_tasks, dfb_plan** out)
+{
+	if (!ctx) return DFB_ERR_ARG;
+	if (!out) return set_err(ctx, DFB_ERR_ARG, "dfb_simple_plan_create: null argument");
+	*out = nullptr;
+	if (int rc = check_simple_args(ctx, params, refs, seqs, task_ref, task_seq, n_tasks)) return rc;
+	const dfb_split_params sp{params->match, params->mismatch, params->gap, 0, 0};
+	return plan_create_host(ctx, true, &sp, refs, seqs, task_ref, task_seq, nullptr, n_tasks, 0, 0, 0, nullptr, out);
+}
+
+static int dfb_split_plan_create_body(dfb_ctx* ctx, const dfb_split_params* params, const dfb_seq_table* refs,
+                                     const dfb_seq_table* reads, const int32_t* task_cluster, const int32_t* task_read,
+                                     const int32_t* task_min_score, int64_t n_tasks, dfb_plan** out)
+{
+	if (!ctx) return DFB_ERR_ARG;
+	if (!out) return set_err(ctx, DFB_ERR_ARG, "dfb_split_plan_create: null argument");
+	*out = nullptr;
+	if (int rc = check_split_args(ctx, params, refs, reads, task_cluster, task_read, task_min_score, n_tasks)) return rc;
+	return plan_create_host(ctx, false, params, refs, reads, task_cluster, task_read, task_min_score, n_tasks, 0, 0, 0, nullptr, out);
+}
+
+// ---- job lists built on the device (dfb_build.cuh) ----------------------------------------------------------
+// Chunks of a pipelined batch of either aligner (`simple`, tables and tasks as for plan_create_host): the caller's
+// offsets and task arrays are uploaded as they are; descriptors, class / length bins and the 32-byte job records are
+// made by kernels.  One small read-back (jobs per class, longest reference per class, total pool words) separates the
+// classify pass from the allocations that depend on it.  device_build_finish returns DFB_BUILD_ON_HOST when the chunk
+// holds tasks only the s32 kernels can take: the caller builds that chunk on the host instead.
+static const int DFB_BUILD_ON_HOST = 1000;
+
+// The uploads go on ctx->upload_stream for every chunk.  The upload streams carry copies only, so one stream serves every
+// chunk in order and chunk 0's upload has the link to itself (two alternating streams share it: the first sweep of a
+// batch started 0.4 ms later on the split path, 5 ms later at the matealign shape).
+static int device_build_enqueue(dfb_ctx* ctx, bool simple, const dfb_split_params* params, const dfb_seq_table* refs,
+                                const dfb_seq_table* reads, const int32_t* task_cluster, const int32_t* task_read,
+                                const int32_t* task_min_score, int64_t n_tasks, int32_t ref_base, int32_t read_base, int stage_slot,
+                                dfb_plan** out)
 {
 	static_assert(kNumClasses <= DFB_BUILD_MAX_CLASSES && kRBins == DFB_BUILD_RBINS, "dfb_build.cuh tables");
 	*out = nullptr;
@@ -1687,7 +1521,7 @@ static int split_build_enqueue(dfb_ctx* ctx, const dfb_split_params* params, con
 	pl->h_task_read = task_read;
 	pl->h_read_base = read_base;
 	classify_params(pl, params->match, params->mismatch, params->gap, simple || (params->end_gaps == 0 && params->min_split_score >= 1));
-	pl->up = up_stream;
+	pl->up = ctx->upload_stream;
 	cudaStream_t up = pl->up;
 	auto fail = [&](int code) {
 		dfb_plan_destroy(pl);
@@ -1805,7 +1639,7 @@ static int split_build_enqueue(dfb_ctx* ctx, const dfb_split_params* params, con
 	pl->pending.d_stats = d_stats;
 	pl->pending.d_words_a_end = d_words_a_end;
 	pl->pending.h_stats = h_stats;
-	tr.lap("split.create(dev): uploads queued");
+	tr.lap("device build: uploads queued");
 	*out = pl;
 	return DFB_OK;
 }
@@ -1814,7 +1648,7 @@ static int split_build_enqueue(dfb_ctx* ctx, const dfb_split_params* params, con
 // of small dependent kernels on another stream would wait for a kernel boundary per link.  Queued between the first
 // sweep and the probe sweep of the previous chunk, the chain costs the GPU a few tens of microseconds and its class
 // counts are back on the host long before that chunk's probe sweep ends.
-static int split_build_kernels(dfb_plan* pl)
+static int device_build_kernels(dfb_plan* pl)
 {
 	dfb_ctx* ctx = pl->ctx;
 	cudaStream_t cs = ctx->stream;
@@ -1848,7 +1682,7 @@ static int split_build_kernels(dfb_plan* pl)
 }
 
 // second half: the class counts are back (or will be: the wait sleeps); everything that depends on them
-static int split_build_finish(dfb_plan* pl)
+static int device_build_finish(dfb_plan* pl)
 {
 	dfb_ctx* ctx = pl->ctx;
 	const dfb_split_params* params = &pl->sp;
@@ -1867,7 +1701,7 @@ static int split_build_finish(dfb_plan* pl)
 	const BuildStats* h_stats = pl->pending.h_stats;
 	const unsigned task_blocks = (unsigned)((n_tasks + DFB_BUILD_BLOCK - 1) / DFB_BUILD_BLOCK);
 	int rc;
-	tr.lap("split.create(dev): classify done");
+	tr.lap("device build: classify done");
 	if (h_stats->bad_table) return fail(set_err(ctx, DFB_ERR_ARG, "a table's offsets decrease or a sequence is too long"));
 	if (h_stats->bad_task != ~0ull) return fail(set_err(ctx, DFB_ERR_ARG, "task %llu: table index out of range", h_stats->bad_task));
 	if (h_stats->n_gen) return fail(DFB_BUILD_ON_HOST);
@@ -1930,23 +1764,8 @@ static int split_build_finish(dfb_plan* pl)
 	if ((rc = alloc_work(pl, bp.jobs, nullptr, n_jobs_cls, !simple, 0))) return fail(rc);
 	for (int c = 0; c < kNumClasses; c++)
 		if (pl->cls[c].n_jobs) fill_fast_params(pl, c, params->match, params->mismatch, params->gap, simple ? 0 : params->min_split_score);
-	tr.lap("split.create(dev): pack, scatter, alloc");
+	tr.lap("device build: pack, scatter, alloc");
 	return DFB_OK;
-}
-
-static int dfb_split_plan_create_body(dfb_ctx* ctx, const dfb_split_params* params, const dfb_seq_table* refs,
-                                     const dfb_seq_table* reads, const int32_t* task_cluster, const int32_t* task_read,
-                                     const int32_t* task_min_score, int64_t n_tasks, dfb_plan** out)
-{
-	if (!ctx) return DFB_ERR_ARG;
-	if (!params || !out || n_tasks < 0 || (n_tasks > 0 && (!task_cluster || !task_read || !task_min_score)))
-		return set_err(ctx, DFB_ERR_ARG, "dfb_split_plan_create: null argument");
-	*out = nullptr;
-	int rc;
-	if ((rc = check_table(ctx, refs, "refs")) || (rc = check_table(ctx, reads, "reads"))) return rc;
-	if (refs->n & 1) return set_err(ctx, DFB_ERR_ARG, "refs must hold two windows per cluster (n is odd)");
-	if (n_tasks > 0x7fffff00LL) return set_err(ctx, DFB_ERR_ARG, "too many tasks in one batch");
-	return split_plan_create_impl(ctx, params, refs, reads, task_cluster, task_read, task_min_score, n_tasks, 0, 0, false, out);
 }
 
 // ---- run / fetch -------------------------------------------------------------------------------
@@ -2547,146 +2366,234 @@ extern "C" int dfb_plan_get_stats(const dfb_plan* pl, dfb_plan_stats* stats)
 
 // ---- one-call forms -------------------------------------------------------------------------------
 
-// Large batches whose task_seq is non-decreasing are cut into chunks: chunk k+1 is uploaded and packed (upload stream)
-// underneath chunk k's sweep, the scores of chunk k-1 go back on the copy stream meanwhile.  A chunk takes a view of
-// the sequences it names; of the references too when task_ref is non-decreasing as well (matealign: one window per
-// task), else the whole reference table (localalign: few references, named in any order).
-static int simple_align_pipelined(dfb_ctx* ctx, const dfb_simple_params* params, const dfb_seq_table* refs,
+// Batches of at least this many tasks whose table-B indices (sequences, reads) do not decrease are cut into chunks
+static int64_t pipeline_min_tasks()
+{
+	if (const char* e = getenv("DFB_PIPELINE_MIN_TASKS")) return std::max<long long>(2, atoll(e)); // tests
+	return 1 << 18;
+}
+
+static bool env_on(const char* name)
+{
+	const char* e = getenv(name);
+	return e && *e && *e != '0';
+}
+
+// Whether task array `b` does not decrease (*b_ok) and, if it does not, whether `a` does not either (*a_ok)
+static void tasks_non_decreasing(dfb_ctx* ctx, const int32_t* b, const int32_t* a, int64_t n_tasks, bool* b_ok, bool* a_ok)
+{
+	const int T = (int)std::max<int64_t>(1, std::min<int64_t>(ctx->host_threads, n_tasks / 262144 + 1));
+	std::vector<char> ok_b((size_t)T, 1), ok_a((size_t)T, 1);
+	parallel_for(ctx->pool, T, [&](int tid) {
+		const int64_t t0 = std::max<int64_t>(1, n_tasks * tid / T), t1 = n_tasks * (tid + 1) / T;
+		bool mb = true, ma = true;
+		for (int64_t t = t0; t < t1 && mb; t++)
+		{
+			mb = b[t] >= b[t - 1];
+			ma = ma && a[t] >= a[t - 1];
+		}
+		ok_b[(size_t)tid] = mb;
+		ok_a[(size_t)tid] = ma;
+	});
+	*b_ok = *a_ok = true;
+	for (int k = 0; k < T; k++)
+	{
+		*b_ok = *b_ok && ok_b[(size_t)k];
+		*a_ok = *a_ok && ok_a[(size_t)k];
+	}
+}
+
+// First task of every chunk (and n_tasks behind the last): chunk k's share of the batch is weight[k] / sum(weight)
+static std::vector<int64_t> chunk_starts(int64_t n_tasks, const std::vector<double>& weight)
+{
+	const int K = (int)weight.size();
+	std::vector<int64_t> t0((size_t)K + 1, 0);
+	double total = 0, run = 0;
+	for (double w : weight) total += w;
+	for (int k = 0; k < K; k++)
+	{
+		run += weight[(size_t)k];
+		t0[(size_t)k + 1] = k + 1 == K ? n_tasks : (int64_t)((double)n_tasks * run / total);
+	}
+	return t0;
+}
+
+// Where the job lists of a chunked batch are built.  Never on the device when no class of the s16x2 kernels takes this
+// scoring (every task is generic then and the host path lists them).  Simple: on the device otherwise -- a simple batch is
+// host-bound on the host path (one pass over the tasks and two over the tables per chunk against 4 ms of sweep).  Split:
+// on the device, 31 ms of host CPU time per 2 M-task batch, but the build kernels sit on the compute stream (0.2 ms per
+// chunk with their launch gaps); on the host, 72 ms of CPU time over the context's workers, fully hidden under the GPU
+// when the host has the threads -- 1.7 ms per batch faster then (A/B on one box, profiles/r03l_ab_e2e.txt).  So the
+// device unless this context has 16 or more host threads to itself (one process per GPU on a shared host caps them with
+// DFB_HOST_THREADS; bench.py does under torchrun).  DFB_DEVICE_BUILD / DFB_HOST_BUILD force either (tests).
+static bool device_build_chosen(dfb_ctx* ctx, bool simple, const dfb_split_params* params)
+{
+	dfb_plan probe;
+	classify_params(&probe, params->match, params->mismatch, params->gap, simple || (params->end_gaps == 0 && params->min_split_score >= 1));
+	bool any_fast = false;
+	for (int c = 0; c < kNumClasses; c++) any_fast = any_fast || probe.fast_ok[c];
+	bool device = any_fast && (simple || ctx->host_threads < 16);
+	if (env_on("DFB_DEVICE_BUILD")) device = any_fast;
+	if (env_on("DFB_HOST_BUILD")) device = false;
+	return device;
+}
+
+// A batch of either aligner (tables and tasks as for plan_create_host) cut into the chunks that start at t0, whose
+// table-B indices do not decrease.  A chunk sees a view of table B (its own entries) and, when the batch's table-A
+// indices do not decrease either (`a_monotone`), a view of table A too -- else the whole table.  Device-built chunks
+// (three beats per chunk): the uploads of chunk k+1 are queued on the upload stream while chunk k is finished --
+// allocations, packing and job scatter once its class counts are back -- and launched; the job-build kernels of chunk
+// k+1 ride on the compute stream between chunk k's two sweeps, so their counts are on the host before chunk k's probe
+// sweep ends and the GPU never waits for this thread.  The plans land in `plans`; chunk_queued(k) runs once chunk k is
+// on the GPU (a non-zero return stops the batch), batch_done(rc) once no more is queued: it waits for what is in flight
+// and returns the batch's result.  The plans are destroyed on return.
+static int pipeline_run(dfb_ctx* ctx, bool simple, const dfb_split_params* params, const dfb_seq_table* A, const dfb_seq_table* B,
+                        const int32_t* task_a, const int32_t* task_b, const int32_t* task_min_score, bool a_monotone,
+                        const std::vector<int64_t>& t0, std::vector<dfb_plan*>& plans, const std::function<int(int)>& chunk_queued,
+                        const std::function<int(int)>& batch_done)
+{
+	const int K = (int)t0.size() - 1;
+	const int64_t per = simple ? 1 : 2; // table-A entries per task index (split: the two windows of a cluster)
+	struct View
+	{
+		dfb_seq_table a, b;
+		int32_t a_lo = 0, b_lo = 0;
+	};
+	auto chunk_of = [&](int k, View& v) -> int {
+		const int64_t t_lo = t0[(size_t)k], t_hi = t0[(size_t)k + 1];
+		if (t_hi <= t_lo) return set_err(ctx, DFB_ERR_STATE, "empty chunk in a pipelined batch");
+		const int64_t b_lo = task_b[t_lo], b_hi = (int64_t)task_b[t_hi - 1] + 1;
+		if (b_lo < 0 || b_hi > B->n) return set_err(ctx, DFB_ERR_ARG, "task %lld: table index out of range", (long long)t_lo);
+		int64_t a_lo = 0, a_hi = A->n / per;
+		if (a_monotone)
+		{
+			a_lo = task_a[t_lo];
+			a_hi = (int64_t)task_a[t_hi - 1] + 1;
+			if (a_lo < 0 || per * a_hi > A->n)
+				return set_err(ctx, DFB_ERR_ARG, "task %lld: table index out of range", (long long)(simple || a_lo < 0 ? t_lo : t_hi - 1));
+		}
+		v.a = dfb_seq_table{A->bytes, A->off + per * a_lo, per * (a_hi - a_lo)};
+		v.b = dfb_seq_table{B->bytes, B->off + b_lo, b_hi - b_lo};
+		v.a_lo = (int32_t)a_lo;
+		v.b_lo = (int32_t)b_lo;
+		return DFB_OK;
+	};
+	auto min_score_of = [&](int64_t t) -> const int32_t* { return simple ? nullptr : task_min_score + t; };
+	std::vector<dfb_plan*> staged((size_t)K, nullptr);
+	auto upload = [&](int k) -> int {
+		View v;
+		const int64_t a = t0[(size_t)k];
+		int rc = chunk_of(k, v);
+		return rc ? rc : device_build_enqueue(ctx, simple, params, &v.a, &v.b, task_a + a, task_b + a, min_score_of(a), t0[(size_t)k + 1] - a,
+		                                      v.a_lo, v.b_lo, k, &staged[(size_t)k]);
+	};
+	const bool device_build = device_build_chosen(ctx, simple, params);
+	// DFB_TRACE: the device's side of the batch -- when every chunk's uploads, first sweep and (split) probe sweep +
+	// assembly ended, measured from an event recorded on the (idle) compute stream now
+	cudaEvent_t trace_base = nullptr;
+	if (trace_on() && cudaEventCreate(&trace_base) == cudaSuccess) cudaEventRecord(trace_base, ctx->stream);
+	int rc = DFB_OK;
+	if (device_build)
+	{
+		rc = upload(0);
+		if (!rc) rc = device_build_kernels(staged[0]); // (the GPU is idle: straight away)
+	}
+	for (int k = 0; k < K && !rc; k++)
+	{
+		if (device_build && k + 1 < K && (rc = upload(k + 1))) break;
+		dfb_plan* pk = staged[(size_t)k];
+		staged[(size_t)k] = nullptr;
+		rc = DFB_BUILD_ON_HOST;
+		if (pk && (rc = device_build_finish(pk)))
+		{
+			dfb_plan_destroy(pk);
+			pk = nullptr;
+		}
+		if (rc == DFB_BUILD_ON_HOST)
+		{
+			View v;
+			const int64_t a = t0[(size_t)k];
+			if (!(rc = chunk_of(k, v)))
+				rc = plan_create_host(ctx, simple, params, &v.a, &v.b, task_a + a, task_b + a, min_score_of(a), t0[(size_t)k + 1] - a, v.a_lo,
+				                      v.b_lo, k, (k & 1) ? ctx->upload_stream2 : ctx->upload_stream, &pk);
+		}
+		if (rc) break;
+		plans[(size_t)k] = pk;
+		if (!simple) pk->result_slot = k;
+		if (trace_base) pk->timing = true;
+		// the next chunk's build kernels ride behind this chunk's first sweep on the compute stream
+		dfb_plan* next = (k + 1 < K) ? staged[(size_t)k + 1] : nullptr;
+		const std::function<int()> hook = [&]() -> int { return next ? device_build_kernels(next) : DFB_OK; };
+		rc = plan_run_impl(pk, &hook);
+		if (!rc) rc = chunk_queued(k);
+	}
+	for (dfb_plan* sp : staged)
+		if (sp)
+		{
+			cudaStreamSynchronize(sp->up); // (its uploads read the caller's arrays)
+			dfb_plan_destroy(sp);
+		}
+	rc = batch_done(rc);
+	if (trace_base)
+	{
+		for (int k = 0; k < K && !rc; k++)
+		{
+			const dfb_plan* pk = plans[(size_t)k];
+			float up = -1, a = -1, b = -1, c = -1;
+			if (pk->pending.uploaded) cudaEventElapsedTime(&up, trace_base, pk->pending.uploaded);
+			cudaEventElapsedTime(&a, trace_base, pk->ev[0]);
+			cudaEventElapsedTime(&b, trace_base, pk->ev[1]);
+			fprintf(stderr, "[dfb] device: chunk %d (%lld tasks) uploaded %.3f | %s %.3f .. %.3f", k, (long long)pk->n_tasks, up,
+			        simple ? "sweep" : "first sweep", a, b);
+			if (!simple)
+			{
+				cudaEventElapsedTime(&c, trace_base, pk->ev[2]);
+				fprintf(stderr, " | probe + assembly .. %.3f", c);
+			}
+			fprintf(stderr, " ms\n");
+		}
+		cudaEventDestroy(trace_base);
+	}
+	for (dfb_plan* pk : plans)
+		if (pk) dfb_plan_destroy(pk);
+	return rc;
+}
+
+// Large batches whose task_seq is non-decreasing go through pipeline_run: chunk k+1 is uploaded and packed underneath
+// chunk k's sweep, the scores of chunk k-1 go back on the copy stream meanwhile.  A chunk takes a view of the sequences it
+// names; of the references too when task_ref is non-decreasing as well (matealign: one window per task), else the whole
+// reference table (localalign: few references, named in any order).
+static int simple_align_pipelined(dfb_ctx* ctx, const dfb_split_params* params, const dfb_seq_table* refs,
                                   const dfb_seq_table* seqs, const int32_t* task_ref, const int32_t* task_seq,
                                   int64_t n_tasks, bool refs_monotone, int32_t* out_score)
 {
 	// chunks: a batch whose references come in task order (matealign: one window per task) uploads every byte once however
 	// it is cut, and is bound by the upload -- short chunks keep the wait for the first and the sweep of the last short;
 	// one whose references are named in any order re-uploads the reference table with every chunk: fewer, longer chunks
-	int64_t per_chunk = refs_monotone ? 80000 : 150000;
-	if (const char* e = getenv("DFB_SIMPLE_CHUNK_TASKS")) per_chunk = std::max<long long>(1000, atoll(e)); // tuning runs
+	const int64_t per_chunk = refs_monotone ? 80000 : 150000;
 	const int K = (int)std::max<int64_t>(2, std::min<int64_t>(dfb_ctx::kStageSlots, n_tasks / per_chunk));
-	std::vector<dfb_plan*> plans((size_t)K, nullptr), staged((size_t)K, nullptr);
-	std::vector<int64_t> t0((size_t)K + 1, 0);
-	{
-		std::vector<double> weight((size_t)K, 1.0);
-		weight[0] = 0.4; // a short first chunk puts the GPU to work early
-		double total = 0, run = 0;
-		for (double w : weight) total += w;
-		for (int k = 0; k < K; k++)
-		{
-			run += weight[(size_t)k];
-			t0[(size_t)k + 1] = k + 1 == K ? n_tasks : (int64_t)((double)n_tasks * run / total);
-		}
-	}
-	// Job lists on the device (dfb_build.cuh) whenever the s16x2 kernels take this scoring: a simple batch is host-bound
-	// otherwise (one pass over the tasks and two over the tables per chunk against 4 ms of sweep).  DFB_HOST_BUILD forces
-	// the host path (A/B runs, tests).
-	dfb_split_params sp{params->match, params->mismatch, params->gap, 0, 0};
-	bool device_build = false;
-	{
-		dfb_plan probe;
-		classify_params(&probe, params->match, params->mismatch, params->gap, true);
-		for (int c = 0; c < kNumClasses; c++) device_build = device_build || probe.fast_ok[c];
-		if (const char* e = getenv("DFB_HOST_BUILD"))
-			if (*e && *e != '0') device_build = false;
-	}
-	struct View
-	{
-		dfb_seq_table refs, seqs;
-		int32_t r_lo, s_lo;
-	};
-	auto chunk_of = [&](int k, View& v) -> int {
-		const int64_t a = t0[(size_t)k], b = t0[(size_t)k + 1];
-		if (b <= a) return set_err(ctx, DFB_ERR_STATE, "empty chunk in a pipelined batch");
-		const int32_t s_lo = task_seq[a], s_hi = task_seq[b - 1] + 1;
-		int32_t r_lo = 0, r_hi = (int32_t)refs->n;
-		if (refs_monotone) { r_lo = task_ref[a]; r_hi = task_ref[b - 1] + 1; }
-		if (s_lo < 0 || s_hi > seqs->n || r_lo < 0 || r_hi > refs->n || s_hi < s_lo || r_hi < r_lo)
-			return set_err(ctx, DFB_ERR_ARG, "task %lld: table index out of range", (long long)a);
-		v.seqs = dfb_seq_table{seqs->bytes, seqs->off + s_lo, (int64_t)(s_hi - s_lo)};
-		v.refs = dfb_seq_table{refs->bytes, refs->off + r_lo, (int64_t)(r_hi - r_lo)};
-		v.r_lo = r_lo;
-		v.s_lo = s_lo;
-		return DFB_OK;
-	};
-	auto upload = [&](int k) -> int {
-		View v;
-		int arc = chunk_of(k, v);
-		if (arc) return arc;
-		const int64_t a = t0[(size_t)k], b = t0[(size_t)k + 1];
-		return split_build_enqueue(ctx, &sp, &v.refs, &v.seqs, task_ref + a, task_seq + a, nullptr, b - a, v.s_lo, k,
-		                           device_build_upload_stream(ctx, k), &staged[(size_t)k], true, v.r_lo);
-	};
-	int rc = DFB_OK;
-	cudaEvent_t trace_base = nullptr; // DFB_TRACE: the device's side of the batch (see split_align_pipelined)
-	if (trace_on() && cudaEventCreate(&trace_base) == cudaSuccess) cudaEventRecord(trace_base, ctx->stream);
+	std::vector<double> weight((size_t)K, 1.0);
+	weight[0] = 0.4; // a short first chunk puts the GPU to work early
+	const std::vector<int64_t> t0 = chunk_starts(n_tasks, weight);
+	std::vector<dfb_plan*> plans((size_t)K, nullptr);
 	Trace trp;
-	if (device_build)
-	{
-		rc = upload(0);
-		if (!rc) rc = split_build_kernels(staged[0]);
-	}
-	for (int k = 0; k < K && !rc; k++)
-	{
-		if (device_build && k + 1 < K && (rc = upload(k + 1))) break;
+	auto copy_scores = [&](int k) -> int {
+		// scores straight into the caller's array, behind this chunk's kernels only
 		const int64_t a = t0[(size_t)k], b = t0[(size_t)k + 1];
-		dfb_plan* pk = staged[(size_t)k];
-		staged[(size_t)k] = nullptr;
-		rc = DFB_BUILD_ON_HOST;
-		if (pk)
-		{
-			rc = split_build_finish(pk);
-			if (rc)
-			{
-				dfb_plan_destroy(pk);
-				pk = nullptr;
-			}
-		}
-		if (rc == DFB_BUILD_ON_HOST)
-		{
-			View v;
-			if (!(rc = chunk_of(k, v)))
-				rc = simple_plan_create_impl(ctx, params, &v.refs, &v.seqs, task_ref + a, task_seq + a, b - a, v.r_lo, v.s_lo, k,
-				                             (k & 1) ? ctx->upload_stream2 : ctx->upload_stream, &pk);
-		}
-		if (rc) break;
-		plans[(size_t)k] = pk;
-		if (trace_base) pk->timing = true;
-		// the next chunk's build kernels ride behind this chunk's sweep on the compute stream
-		dfb_plan* next = (k + 1 < K) ? staged[(size_t)k + 1] : nullptr;
-		const std::function<int()> hook = [&]() -> int { return next ? split_build_kernels(next) : DFB_OK; };
-		rc = plan_run_impl(pk, &hook);
-		if (!rc)
-		{
-			// scores straight into the caller's array, behind this chunk's kernels only
-			cudaError_t e = cudaStreamWaitEvent(ctx->copy_stream, pk->done_ev, 0);
-			if (e == cudaSuccess)
-				e = cudaMemcpyAsync(out_score + a, pk->d_out, (size_t)(b - a) * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->copy_stream);
-			if (e != cudaSuccess) rc = set_err(ctx, DFB_ERR_CUDA, "score copy failed: %s", cudaGetErrorString(e));
-		}
-	}
-	cudaError_t e = cudaStreamSynchronize(ctx->copy_stream);
-	if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-	if (!rc && e != cudaSuccess) rc = set_err(ctx, DFB_ERR_CUDA, "pipelined batch failed: %s", cudaGetErrorString(e));
-	if (!rc) rc = bounds_check_status(ctx);
-	trp.lap("simple pipelined: done");
-	if (trace_base)
-	{
-		for (int k = 0; k < K && !rc; k++)
-		{
-			float up = -1, a = -1, b2 = -1;
-			if (plans[(size_t)k]->pending.uploaded) cudaEventElapsedTime(&up, trace_base, plans[(size_t)k]->pending.uploaded);
-			cudaEventElapsedTime(&a, trace_base, plans[(size_t)k]->ev[0]);
-			cudaEventElapsedTime(&b2, trace_base, plans[(size_t)k]->ev[1]);
-			fprintf(stderr, "[dfb] device: chunk %d (%lld tasks) uploaded %.3f | sweep %.3f .. %.3f ms\n", k, (long long)plans[(size_t)k]->n_tasks, up, a, b2);
-		}
-		cudaEventDestroy(trace_base);
-	}
-	for (dfb_plan* sp2 : staged)
-		if (sp2)
-		{
-			cudaStreamSynchronize(sp2->up); // (its uploads read the caller's arrays)
-			dfb_plan_destroy(sp2);
-		}
-	for (dfb_plan* pk : plans)
-		if (pk) dfb_plan_destroy(pk);
-	return rc;
+		cudaError_t e = cudaStreamWaitEvent(ctx->copy_stream, plans[(size_t)k]->done_ev, 0);
+		if (e == cudaSuccess)
+			e = cudaMemcpyAsync(out_score + a, plans[(size_t)k]->d_out, (size_t)(b - a) * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->copy_stream);
+		return e == cudaSuccess ? DFB_OK : set_err(ctx, DFB_ERR_CUDA, "score copy failed: %s", cudaGetErrorString(e));
+	};
+	auto wait_all = [&](int rc) -> int {
+		cudaError_t e = cudaStreamSynchronize(ctx->copy_stream);
+		if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+		if (!rc && e != cudaSuccess) rc = set_err(ctx, DFB_ERR_CUDA, "pipelined batch failed: %s", cudaGetErrorString(e));
+		if (!rc) rc = bounds_check_status(ctx);
+		trp.lap("simple pipelined: done");
+		return rc;
+	};
+	return pipeline_run(ctx, true, params, refs, seqs, task_ref, task_seq, nullptr, refs_monotone, t0, plans, copy_scores, wait_all);
 }
 
 static int dfb_simple_align_batch_body(dfb_ctx* ctx, const dfb_simple_params* params, const dfb_seq_table* refs,
@@ -2694,34 +2601,18 @@ static int dfb_simple_align_batch_body(dfb_ctx* ctx, const dfb_simple_params* pa
                                       int64_t n_tasks, int32_t* out_score)
 {
 	if (!ctx) return DFB_ERR_ARG;
-	int64_t pipeline_min = 1 << 18;
-	if (const char* e = getenv("DFB_PIPELINE_MIN_TASKS")) pipeline_min = std::max<long long>(2, atoll(e)); // tests
-	if (n_tasks >= pipeline_min && params && refs && seqs && task_ref && task_seq && out_score)
+	int rc = check_simple_args(ctx, params, refs, seqs, task_ref, task_seq, n_tasks);
+	if (rc) return rc;
+	const dfb_split_params sp{params->match, params->mismatch, params->gap, 0, 0};
+	if (n_tasks >= pipeline_min_tasks() && out_score)
 	{
-		int rc;
-		if ((rc = check_table_parallel(ctx, refs, "refs")) || (rc = check_table_parallel(ctx, seqs, "seqs"))) return rc;
-		if (n_tasks > 0x7fffff00LL) return set_err(ctx, DFB_ERR_ARG, "too many tasks in one batch");
-		const int T = (int)std::max<int64_t>(1, std::min<int64_t>(ctx->host_threads, n_tasks / 262144 + 1));
-		std::vector<char> ok_s((size_t)T, 1), ok_r((size_t)T, 1);
-		parallel_for(ctx->pool, T, [&](int tid) {
-			const int64_t a = std::max<int64_t>(1, n_tasks * tid / T), b = n_tasks * (tid + 1) / T;
-			bool ms = true, mr = true;
-			for (int64_t t = a; t < b && ms; t++)
-			{
-				ms = task_seq[t] >= task_seq[t - 1];
-				mr = mr && task_ref[t] >= task_ref[t - 1];
-			}
-			ok_s[(size_t)tid] = ms;
-			ok_r[(size_t)tid] = mr;
-		});
-		bool seq_monotone = true, ref_monotone = true;
-		for (char c : ok_s) seq_monotone = seq_monotone && c;
-		for (char c : ok_r) ref_monotone = ref_monotone && c;
-		if (seq_monotone) return simple_align_pipelined(ctx, params, refs, seqs, task_ref, task_seq, n_tasks, ref_monotone, out_score);
+		bool seq_monotone, ref_monotone;
+		tasks_non_decreasing(ctx, task_seq, task_ref, n_tasks, &seq_monotone, &ref_monotone);
+		if (seq_monotone) return simple_align_pipelined(ctx, &sp, refs, seqs, task_ref, task_seq, n_tasks, ref_monotone, out_score);
 	}
 	dfb_plan* pl = nullptr;
 	Trace tr;
-	int rc = dfb_simple_plan_create(ctx, params, refs, seqs, task_ref, task_seq, n_tasks, &pl);
+	rc = plan_create_host(ctx, true, &sp, refs, seqs, task_ref, task_seq, nullptr, n_tasks, 0, 0, 0, nullptr, &pl);
 	if (rc) return rc;
 	tr.lap("simple: create");
 	rc = dfb_plan_run(pl);
@@ -2732,58 +2623,45 @@ static int dfb_simple_align_batch_body(dfb_ctx* ctx, const dfb_simple_params* pa
 	return rc;
 }
 
-// Large batches whose task_read is non-decreasing (the usual case: reads are listed in task order) are cut
-// into chunks that flow through the GPU back to back while the host builds the next chunk and assembles the
-// previous one.  Results are merged into one task-ordered row list.
-static const int64_t kPipelineMinTasks = 1 << 18;
-
+// Large batches whose task_read is non-decreasing (the usual case: reads are listed in task order) go through
+// pipeline_run: chunks flow through the GPU back to back while the host builds the next chunk and assembles the previous
+// one.  Results are merged into one task-ordered row list.  A chunk sees views of both tables: its own reads and -- when
+// the batch's clusters do not decrease, the order dosplitalign emits -- its own window pairs, so that every window is
+// uploaded and packed once per batch (plus one shared cluster per chunk boundary) instead of once per chunk.
 static int split_align_pipelined(dfb_ctx* ctx, const dfb_split_params* params, const dfb_seq_table* refs,
                                  const dfb_seq_table* reads, const int32_t* task_cluster, const int32_t* task_read,
                                  const int32_t* task_min_score, int64_t n_tasks, int32_t* out_best, bool clusters_monotone)
 {
-	int K = (int)std::max<int64_t>(2, std::min<int64_t>(std::min<int64_t>(dfb_ctx::kStageSlots, n_tasks), n_tasks / 330000));
-	if (const char* e = getenv("DFB_PIPELINE_CHUNKS")) // tuning runs
-		K = (int)std::max<int64_t>(2, std::min<int64_t>(std::min<int64_t>(dfb_ctx::kStageSlots, n_tasks), atoi(e)));
-	std::vector<dfb_plan*> plans((size_t)K, nullptr);
+	const int K = (int)std::max<int64_t>(2, std::min<int64_t>(std::min<int64_t>(dfb_ctx::kStageSlots, n_tasks), n_tasks / 330000));
 	// chunk boundaries: short chunks in front put the GPU to work early, chunks that taper off at the end keep the part
 	// of the result assembly that nothing overlaps small (lane 2 finishes chunk k while the GPU runs chunk k+1); the
 	// chunks in between share the rest
-	std::vector<int64_t> t0((size_t)K + 1);
+	std::vector<double> weight((size_t)K, 1.0);
+	if (K >= 8)
 	{
-		std::vector<double> weight((size_t)K, 1.0);
-		if (K >= 8)
-		{
-			// the fetch lane needs about 0.8 of a chunk's GPU time for that chunk: a tail that shrinks by no more than
-			// that factor per chunk keeps it from falling behind, so only the last, smallest chunk's fetch is left uncovered
-			weight[0] = 0.3;
-			weight[1] = 0.7;
-			weight[(size_t)K - 4] = 0.8;
-			weight[(size_t)K - 3] = 0.62;
-			weight[(size_t)K - 2] = 0.48;
-			weight[(size_t)K - 1] = 0.36;
-		}
-		else if (K >= 6)
-		{
-			weight[0] = 0.25;
-			weight[1] = 0.6;
-			weight[(size_t)K - 2] = 0.6;
-			weight[(size_t)K - 1] = 0.3;
-		}
-		else if (K >= 4)
-		{
-			weight[0] = 0.4;
-			weight[(size_t)K - 1] = 0.45;
-		}
-		double total = 0, run = 0;
-		for (double w : weight) total += w;
-		t0[0] = 0;
-		for (int k = 0; k < K; k++)
-		{
-			run += weight[(size_t)k];
-			t0[(size_t)k + 1] = k + 1 == K ? n_tasks : (int64_t)((double)n_tasks * run / total);
-		}
+		// the fetch lane needs about 0.8 of a chunk's GPU time for that chunk: a tail that shrinks by no more than
+		// that factor per chunk keeps it from falling behind, so only the last, smallest chunk's fetch is left uncovered
+		weight[0] = 0.3;
+		weight[1] = 0.7;
+		weight[(size_t)K - 4] = 0.8;
+		weight[(size_t)K - 3] = 0.62;
+		weight[(size_t)K - 2] = 0.48;
+		weight[(size_t)K - 1] = 0.36;
 	}
-	int rc = DFB_OK;
+	else if (K >= 6)
+	{
+		weight[0] = 0.25;
+		weight[1] = 0.6;
+		weight[(size_t)K - 2] = 0.6;
+		weight[(size_t)K - 1] = 0.3;
+	}
+	else if (K >= 4)
+	{
+		weight[0] = 0.4;
+		weight[(size_t)K - 1] = 0.45;
+	}
+	const std::vector<int64_t> t0 = chunk_starts(n_tasks, weight);
+	std::vector<dfb_plan*> plans((size_t)K, nullptr);
 	{
 		// the pinned buffer the chunks' results land in: sized for the largest chunk now (growing it chunk by chunk frees and
 		// pins it again each time, at 0.6 ms per MB either way)
@@ -2792,32 +2670,6 @@ static int split_align_pipelined(dfb_ctx* ctx, const dfb_split_params* params, c
 		ctx->h_out.ensure((size_t)largest * 72);
 	}
 	Trace trp;
-	// DFB_TRACE: the device's side of the batch -- when every chunk's uploads, first sweep and probe sweep + assembly
-	// ended, measured from an event recorded on the (idle) compute stream now
-	cudaEvent_t trace_base = nullptr;
-	if (trace_on() && cudaEventCreate(&trace_base) == cudaSuccess) cudaEventRecord(trace_base, ctx->stream);
-	// Where the job lists are built.  On the device: 31 ms of host CPU time per 2 M-task batch, but the build kernels sit
-	// on the compute stream (0.2 ms per chunk with their launch gaps).  On the host: 72 ms of CPU time over the context's
-	// workers, fully hidden under the GPU when the host has the threads -- 1.7 ms per batch faster then (A/B on one box,
-	// profiles/r03l_ab_e2e.txt).  So: the device unless this context has 16 or more host threads to itself (one process
-	// per GPU on a shared host caps them with DFB_HOST_THREADS; bench.py does under torchrun); never when no class of the
-	// s16x2 kernels takes this scoring (every task is generic then and the host path lists them).  DFB_HOST_BUILD /
-	// DFB_DEVICE_BUILD force either (A/B runs, tests).
-	bool device_build = false;
-	{
-		dfb_plan probe;
-		classify_params(&probe, params->match, params->mismatch, params->gap, params->end_gaps == 0 && params->min_split_score >= 1);
-		for (int c = 0; c < kNumClasses; c++) device_build = device_build || probe.fast_ok[c];
-		if (ctx->host_threads >= 16) device_build = false;
-		if (const char* e = getenv("DFB_DEVICE_BUILD"))
-			if (*e && *e != '0')
-			{
-				device_build = false;
-				for (int c = 0; c < kNumClasses; c++) device_build = device_build || probe.fast_ok[c];
-			}
-		if (const char* e = getenv("DFB_HOST_BUILD"))
-			if (*e && *e != '0') device_build = false;
-	}
 	// the batch's result holder: every chunk's rows go straight behind the previous chunk's
 	dfb_plan* holder = new (std::nothrow) dfb_plan();
 	if (!holder) return set_err(ctx, DFB_ERR_NOMEM, "out of host memory");
@@ -2846,7 +2698,7 @@ static int split_align_pipelined(dfb_ctx* ctx, const dfb_split_params* params, c
 				cv.wait(lk, [&] { return queued > k || abort; });
 				if (queued <= k) return;
 			}
-			sink.task_shift = (int32_t)t0[(size_t)k];
+			sink.task_shift = (int32_t)t0[k];
 			int frc = split_fetch_impl(plans[k], out_best ? out_best + t0[k] : nullptr, nullptr, nullptr, ctx->pool_fetch, &sink);
 			if (frc)
 			{
@@ -2864,141 +2716,50 @@ static int split_align_pipelined(dfb_ctx* ctx, const dfb_split_params* params, c
 			fetch_rc = set_err(ctx, DFB_ERR_NOMEM, "out of host memory in the fetch lane");
 		}
 	});
-	// Device-built chunks (lane 1 in three beats per chunk): the uploads of chunk k+1 are queued on an upload stream
-	// while chunk k is finished -- allocations, packing and job scatter once its class counts are back -- and launched;
-	// the job-build kernels of chunk k+1 ride on the compute stream between chunk k's two sweeps, so their counts are
-	// on the host before chunk k's probe sweep ends and the GPU never waits for this thread.
-	std::vector<dfb_plan*> staged((size_t)K, nullptr);
-	// a chunk sees views of both tables: its own reads and -- when the batch's clusters do not decrease, the order
-	// dosplitalign emits -- its own window pairs, so that every window is uploaded and packed once per batch (plus
-	// one shared cluster per chunk boundary) instead of once per chunk
-	struct View
-	{
-		dfb_seq_table reads, refs;
-		int32_t r_lo = 0, c_lo = 0;
-	};
-	auto chunk_of = [&](int k, View& v) -> int {
-		const int64_t a = t0[k], b = t0[k + 1];
-		if (b <= a) return set_err(ctx, DFB_ERR_STATE, "empty chunk in a pipelined batch");
-		v.r_lo = task_read[a];
-		const int32_t r_hi = task_read[b - 1] + 1;
-		if (v.r_lo < 0 || r_hi > reads->n) return set_err(ctx, DFB_ERR_ARG, "task %lld: table index out of range", (long long)a);
-		v.reads = dfb_seq_table{reads->bytes, reads->off + v.r_lo, (int64_t)(r_hi - v.r_lo)};
-		v.refs = *refs;
-		v.c_lo = 0;
-		if (clusters_monotone)
-		{
-			const int64_t c_lo = task_cluster[a], c_hi = (int64_t)task_cluster[b - 1] + 1;
-			if (c_lo < 0 || 2 * c_hi > refs->n)
-				return set_err(ctx, DFB_ERR_ARG, "task %lld: table index out of range", (long long)(c_lo < 0 ? a : b - 1));
-			v.c_lo = (int32_t)c_lo;
-			v.refs = dfb_seq_table{refs->bytes, refs->off + 2 * c_lo, 2 * (c_hi - c_lo)};
-		}
-		return DFB_OK;
-	};
-	auto upload = [&](int k) -> int {
-		View v;
-		int arc = chunk_of(k, v);
-		if (arc) return arc;
-		const int64_t a = t0[k], b = t0[k + 1];
-		return split_build_enqueue(ctx, params, &v.refs, &v.reads, task_cluster + a, task_read + a, task_min_score + a, b - a, v.r_lo, k,
-		                           device_build_upload_stream(ctx, k), &staged[(size_t)k], false, v.c_lo);
-	};
-	if (device_build)
-	{
-		rc = upload(0);
-		if (!rc) rc = split_build_kernels(staged[0]); // (the GPU is idle: straight away)
-	}
-	for (int k = 0; k < K && !rc && !fetch_rc.load(); k++)
-	{
-		if (device_build && k + 1 < K && (rc = upload(k + 1))) break;
-		const int64_t a = t0[k], b = t0[k + 1];
-		dfb_plan* pk = staged[(size_t)k];
-		staged[(size_t)k] = nullptr;
-		rc = DFB_BUILD_ON_HOST;
-		if (pk)
-		{
-			rc = split_build_finish(pk);
-			if (rc)
-			{
-				dfb_plan_destroy(pk);
-				pk = nullptr;
-			}
-		}
-		if (rc == DFB_BUILD_ON_HOST)
-		{
-			View v;
-			if (!(rc = chunk_of(k, v)))
-				rc = split_plan_create_impl(ctx, params, &v.refs, &v.reads, task_cluster + a, task_read + a, task_min_score + a, b - a, v.r_lo, k,
-				                            true, &pk, v.c_lo);
-		}
-		if (rc) break;
-		pk->result_slot = k;
-		pk->early_release = true;
-		if (trace_base) pk->timing = true;
-		dfb_plan* next = (k + 1 < K) ? staged[(size_t)k + 1] : nullptr;
-		const std::function<int()> hook = [&]() -> int { return next ? split_build_kernels(next) : DFB_OK; };
-		rc = plan_run_impl(pk, &hook);
+	auto hand_to_lane2 = [&](int k) -> int {
 		{
 			std::lock_guard<std::mutex> lk(mu);
-			plans[k] = pk;
-			if (!rc) queued = k + 1;
+			queued = k + 1;
 		}
 		cv.notify_all();
-	}
-	for (dfb_plan* sp : staged)
-		if (sp)
+		return fetch_rc.load();
+	};
+	auto join_lane2 = [&](int rc) -> int {
 		{
-			cudaStreamSynchronize(sp->up); // (its uploads read the caller's arrays)
-			dfb_plan_destroy(sp);
+			std::lock_guard<std::mutex> lk(mu);
+			if (rc) abort = true;
 		}
-	{
-		std::lock_guard<std::mutex> lk(mu);
-		if (rc) abort = true;
-	}
-	cv.notify_all();
-	trp.lap("pipelined: lane 1 done");
-	lane2.join();
-	trp.lap("pipelined: lane 2 joined");
-	if (!rc) rc = fetch_rc.load();
-	if (!rc)
-	{
-		holder->fetched = true;
-		holder->ran = true;
-		for (int k = 0; k < K; k++)
+		cv.notify_all();
+		trp.lap("pipelined: lane 1 done");
+		lane2.join();
+		trp.lap("pipelined: lane 2 joined");
+		if (!rc) rc = fetch_rc.load();
+		if (!rc)
 		{
-			holder->stats.events += plans[k]->stats.events;
-			holder->stats.probe_jobs += plans[k]->stats.probe_jobs;
-			holder->stats.d2h_bytes += plans[k]->stats.d2h_bytes;
-			holder->stats.h2d_bytes += plans[k]->stats.h2d_bytes;
-			holder->stats.cells += plans[k]->stats.cells;
-			holder->stats.fast_jobs += plans[k]->stats.fast_jobs;
-			holder->stats.generic_jobs += plans[k]->stats.generic_jobs;
-			holder->stats.kernel_launches += plans[k]->stats.kernel_launches;
-			holder->stats.raw_bytes += plans[k]->stats.raw_bytes;
-			holder->stats.packed_bytes += plans[k]->stats.packed_bytes;
+			holder->fetched = true;
+			holder->ran = true;
+			for (int k = 0; k < K; k++)
+			{
+				holder->stats.events += plans[k]->stats.events;
+				holder->stats.probe_jobs += plans[k]->stats.probe_jobs;
+				holder->stats.d2h_bytes += plans[k]->stats.d2h_bytes;
+				holder->stats.h2d_bytes += plans[k]->stats.h2d_bytes;
+				holder->stats.cells += plans[k]->stats.cells;
+				holder->stats.fast_jobs += plans[k]->stats.fast_jobs;
+				holder->stats.generic_jobs += plans[k]->stats.generic_jobs;
+				holder->stats.kernel_launches += plans[k]->stats.kernel_launches;
+				holder->stats.raw_bytes += plans[k]->stats.raw_bytes;
+				holder->stats.packed_bytes += plans[k]->stats.packed_bytes;
+			}
 		}
-	}
-	if (trace_base)
-	{
-		for (int k = 0; k < K && !rc; k++)
-		{
-			float up = -1, a = -1, b = -1, c = -1;
-			if (plans[k]->pending.uploaded) cudaEventElapsedTime(&up, trace_base, plans[k]->pending.uploaded);
-			cudaEventElapsedTime(&a, trace_base, plans[k]->ev[0]);
-			cudaEventElapsedTime(&b, trace_base, plans[k]->ev[1]);
-			cudaEventElapsedTime(&c, trace_base, plans[k]->ev[2]);
-			fprintf(stderr, "[dfb] device: chunk %d (%lld tasks) uploaded %.3f | first sweep %.3f .. %.3f | probe + assembly .. %.3f ms\n", k,
-			        (long long)plans[k]->n_tasks, up, a, b, c);
-		}
-		cudaEventDestroy(trace_base);
-	}
-	for (int k = 0; k < K; k++)
-		if (plans[k]) dfb_plan_destroy(plans[k]);
+		return rc;
+	};
+	const int rc = pipeline_run(ctx, false, params, refs, reads, task_cluster, task_read, task_min_score, clusters_monotone, t0, plans,
+	                            hand_to_lane2, join_lane2);
 	trp.lap("pipelined: chunks destroyed");
 	if (rc)
 	{
-		if (holder) dfb_plan_destroy(holder);
+		dfb_plan_destroy(holder);
 		return rc;
 	}
 	ctx->last_split = holder;
@@ -3015,40 +2776,20 @@ static int dfb_split_align_batch_body(dfb_ctx* ctx, const dfb_split_params* para
 		dfb_plan_destroy(ctx->last_split);
 		ctx->last_split = nullptr;
 	}
-	int64_t pipeline_min = kPipelineMinTasks;
-	if (const char* e = getenv("DFB_PIPELINE_MIN_TASKS")) pipeline_min = std::max<long long>(2, atoll(e)); // tests
 	Trace tre;
 	tre.lap("split: entry");
-	if (n_tasks >= pipeline_min && params && refs && reads && task_cluster && task_read && task_min_score)
+	int rc = check_split_args(ctx, params, refs, reads, task_cluster, task_read, task_min_score, n_tasks);
+	if (rc) return rc;
+	if (n_tasks >= pipeline_min_tasks())
 	{
-		int rc;
-		if ((rc = check_table(ctx, refs, "refs")) || (rc = check_table_parallel(ctx, reads, "reads"))) return rc;
-		if (refs->n & 1) return set_err(ctx, DFB_ERR_ARG, "refs must hold two windows per cluster (n is odd)");
-		if (n_tasks > 0x7fffff00LL) return set_err(ctx, DFB_ERR_ARG, "too many tasks in one batch");
-		bool monotone = true, clusters_monotone = true;
-		{
-			const int T = (int)std::max<int64_t>(1, std::min<int64_t>(ctx->host_threads, n_tasks / 262144 + 1));
-			std::vector<char> ok((size_t)T, 1), okc((size_t)T, 1);
-			parallel_for(ctx->pool, T, [&](int tid) {
-				const int64_t a = std::max<int64_t>(1, n_tasks * tid / T), b = n_tasks * (tid + 1) / T;
-				bool m = true, mc = true;
-				for (int64_t t = a; t < b && m; t++)
-				{
-					m = task_read[t] >= task_read[t - 1];
-					mc = mc && task_cluster[t] >= task_cluster[t - 1];
-				}
-				ok[(size_t)tid] = m;
-				okc[(size_t)tid] = mc;
-			});
-			for (char c : ok) monotone = monotone && c;
-			for (char c : okc) clusters_monotone = clusters_monotone && c;
-		}
+		bool monotone, clusters_monotone;
+		tasks_non_decreasing(ctx, task_read, task_cluster, n_tasks, &monotone, &clusters_monotone);
 		tre.lap("split: validated");
 		if (monotone)
 			return split_align_pipelined(ctx, params, refs, reads, task_cluster, task_read, task_min_score, n_tasks, out_best, clusters_monotone);
 	}
 	dfb_plan* pl = nullptr;
-	int rc = dfb_split_plan_create(ctx, params, refs, reads, task_cluster, task_read, task_min_score, n_tasks, &pl);
+	rc = plan_create_host(ctx, false, params, refs, reads, task_cluster, task_read, task_min_score, n_tasks, 0, 0, 0, nullptr, &pl);
 	if (rc) return rc;
 	rc = dfb_plan_run(pl);
 	if (!rc) rc = dfb_split_plan_fetch(pl, out_best, nullptr, nullptr);
