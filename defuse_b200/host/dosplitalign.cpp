@@ -15,6 +15,15 @@
 // into evalsplitalign's evaluation (eval_core.h): the three outputs are byte-identical to
 // dosplitalign | sort | evalsplitalign, without the multi-gigabyte intermediate file, the sort and the second parse.
 // One process must see every read of the fusions it evaluates (one fastq split, or all of them).
+//
+// Built with -DDFB_MULTI_SPLIT it is dosplitalign_multi, every fastq split of a run in one process:
+//   dosplitalign_multi -f ref.fa -e exons.regions -u <mean> -s <sd> -n <minread> -x <maxread> -r clusters.regions -l splits.tsv
+// where each line of splits.tsv is "seq1.fastq <TAB> seq2.fastq <TAB> improper.sam <TAB> out.alignments".  Files,
+// stdout, stderr and exit code are those of the stock tool run once per line, in order, stopping at the first run that
+// fails; the set-up every split shares (regions, reference, exons, tasks, window table, bins, GPU contexts) is done once.
+#if defined(DFB_FUSED_EVAL) && defined(DFB_MULTI_SPLIT)
+#error "dosplitalign_eval and dosplitalign_multi are separate tools"
+#endif
 #include "split_tasks.h"
 #include "fast_io.h"
 #ifdef DFB_FUSED_EVAL
@@ -25,6 +34,7 @@
 #include <fstream>
 #include <map>
 #include <memory>
+#include <set>
 #include <thread>
 #include <unordered_map>
 #include <unordered_set>
@@ -99,36 +109,47 @@ std::string SortRecordsLikeThePipeline(const std::string& text)
 }
 #endif
 
-}  // namespace
-
-int main(int argc, char* argv[])
+// Where a split's messages go: straight to the streams, or -- for a split whose ingest runs while the split before it
+// is still being aligned and written -- held until Release(), which writes them in the order they were said.
+class Messages
 {
-	CommandLine cmd("Fusion sequence prediction by split reads", {
-	    {'f', "fasta", "Reference Fasta", true, "string", "", false},
-	    {'e', "exons", "Exon Regions Filename", true, "string", "", false},
-	    {'u', "ufrag", "Fragment Length Mean", true, "float", "", false},
-	    {'s', "sfrag", "Fragment Length Standard Deviation", true, "float", "", false},
-	    {'n', "minread", "Minimum Read Length", true, "integer", "", false},
-	    {'x', "maxread", "Maximum Read Length", true, "integer", "", false},
-	    {'r', "regions", "Fusion Regions Filename", true, "string", "", false},
-	    {'i', "improper", "Improper Alignments Sam Filename", true, "string", "", false},
-	    {'1', "seq1", "End 1 Sequences", true, "string", "", false},
-	    {'2', "seq2", "End 2 Sequences", true, "string", "", false},
-#ifdef DFB_FUSED_EVAL
-	    {'a', "align", "Split Alignments Filename (optional here)", false, "string", "", false},
-	    {'q', "seq", "Sequences Filename", true, "string", "", false},
-	    {'b', "break", "Break Positions Filename", true, "string", "", false},
-	    {'p', "predalign", "Prediction Split Alignments Filename", true, "string", "", false},
-#else
-	    {'a', "align", "Split Alignments Filename", true, "string", "", false},
-#endif
-	});
-	cmd.Parse(argc, argv);
-	PhaseTimer timer;
+public:
+	explicit Messages(bool hold) : mHold(hold) {}
+	void Out(const std::string& s) { Say(&std::cout, s); }
+	void Err(const std::string& s) { Say(&std::cerr, s); }
+	void Release()
+	{
+		for (const auto& m : mHeld) *m.first << m.second << std::flush;
+		mHeld.clear();
+	}
+
+private:
+	void Say(std::ostream* stream, const std::string& s)
+	{
+		if (s.empty()) return;
+		if (mHold) mHeld.emplace_back(stream, s);
+		else *stream << s << std::flush;
+	}
+	bool mHold;
+	std::vector<std::pair<std::ostream*, std::string>> mHeld;
+};
+
+// What every split reads and nothing changes after the set-up: the GPU contexts, the tasks, the window table (window
+// pair 2k, 2k+1 of cluster slot k) and the 2 000-bp bins of the mate regions.
+struct SharedSetup
+{
+	std::vector<std::unique_ptr<Gpu>> gpus;
+	std::unordered_map<int, ClusterTask> tasks; // its iteration order is the order mate regions are registered in
+	BinnedRegions binned{2000};
+	std::unordered_map<int, int> cluster_slot; // fusion id -> dense index (window pair 2k, 2k+1)
+	TableBuilder windows;
+};
+
+void ReadSharedSetup(const CommandLine& cmd, SharedSetup& s, PhaseTimer& timer)
+{
 	// one context per GPU (DFB_DEVICES), created in the background while the inputs are parsed; candidates are
 	// dealt out by cluster, no exchange between GPUs
-	std::vector<std::unique_ptr<Gpu>> gpus;
-	for (int dev : DeviceList()) gpus.emplace_back(new Gpu(dev));
+	for (int dev : DeviceList()) s.gpus.emplace_back(new Gpu(dev));
 	const double frag_mean = cmd.Double('u', 0.0), frag_sd = cmd.Double('s', 0.0);
 	const int min_read = cmd.Int('n'), max_read = cmd.Int('x');
 
@@ -146,33 +167,76 @@ int main(int argc, char* argv[])
 			ExitNow(1);
 		}
 	}
-	std::unordered_map<int, ClusterTask> tasks; // its iteration order is the order mate regions are registered in
 	for (const auto& kv : regions)
-		InitializeTask(tasks[kv.first], kv.first, kv.second, reference, exons, frag_mean, frag_sd, min_read, max_read);
+		InitializeTask(s.tasks[kv.first], kv.first, kv.second, reference, exons, frag_mean, frag_sd, min_read, max_read);
 
 	timer.Lap("regions, fasta, exons, tasks");
-	BinnedRegions binned(2000);
-	std::unordered_map<int, int> cluster_slot; // fusion id -> dense index (window pair 2k, 2k+1)
-	TableBuilder windows;
-	for (const auto& kv : tasks)
+	for (const auto& kv : s.tasks)
 	{
 		const ClusterTask& t = kv.second;
-		cluster_slot[t.fusion_id] = (int)(windows.Count() / 2);
-		windows.Add(t.window[0]);
-		windows.Add(t.window[1]);
+		s.cluster_slot[t.fusion_id] = (int)(s.windows.Count() / 2);
+		s.windows.Add(t.window[0]);
+		s.windows.Add(t.window[1]);
 		for (int end = 0; end <= 1; end++)
-			for (const Location& loc : t.mate_regions[end]) binned.Add(PackId(t.fusion_id, end), loc);
+			for (const Location& loc : t.mate_regions[end]) s.binned.Add(PackId(t.fusion_id, end), loc);
 	}
+	timer.Lap("bins");
+}
 
-	// ---- reads: both fastq files indexed in place on a helper thread while the SAM file is parsed ----
+// the four paths of one split (`write_align` false: dosplitalign_eval without -a)
+struct SplitPaths
+{
+	std::string seq1, seq2, improper, align;
+	bool write_align = true;
+};
+
+// what a split's ingest leaves for its alignment: both fastq files indexed in place, the candidates in order
+struct SplitInput
+{
 	FastqIndex fastq[2];
-	const bool ok0 = fastq[0].Open(cmd.Str('1'));
-	const bool ok1 = fastq[1].Open(cmd.Str('2'));
-	std::cerr << fastq[0].Message() << fastq[1].Message();
+	std::unique_ptr<Candidate[]> candidates;
+	size_t n_candidates = 0;
+};
+
+// Host buffers of the batches, kept from batch to batch and from split to split.
+struct Shard
+{
+	// the batch's reads as a CSR table; the bytes are a plain array that the worker threads touch first
+	std::unique_ptr<char[]> read_bytes;
+	size_t read_bytes_cap = 0;
+	std::vector<int64_t> read_off;
+	std::vector<int32_t> task_cluster, task_read, task_min_score, best, read_len, ref2_len;
+	std::vector<int64_t> row_begin; // first result row of each task (n_rows when it has none)
+	const dfb_split_row* rows = nullptr;
+	const int32_t* cols = nullptr;
+	int64_t n_rows = 0, n_cols = 0;
+	int rc = DFB_OK;
+};
+struct BatchBuffers
+{
+	explicit BatchBuffers(int n_gpus) : shards((size_t)n_gpus), out_parts((size_t)ToolThreads()) {}
+	std::vector<Shard> shards;
+	std::vector<int> gpu_of;
+	std::vector<int32_t> local_of;        // index of a candidate inside its shard
+	std::vector<const char*> cand_seq;    // the candidate's read in the mapped fastq (forward orientation)
+	std::vector<uint32_t> cand_len;
+	std::vector<int32_t> cand_slot;
+	std::vector<std::string> out_parts;
+};
+
+// One split up to its candidates: FASTQ index, SAM parse, overlaps, de-duplication.  false: the split fails here, its
+// messages said (the stock tool exits 1 at that point).
+bool IngestSplit(const SharedSetup& s, const SplitPaths& paths, SplitInput& in, Messages& msg, PhaseTimer& timer)
+{
+	// ---- reads: both fastq files indexed in place on a helper thread while the SAM file is parsed ----
+	FastqIndex* const fastq = in.fastq;
+	const bool ok0 = fastq[0].Open(paths.seq1);
+	const bool ok1 = fastq[1].Open(paths.seq2);
+	msg.Err(fastq[0].Message() + fastq[1].Message());
 	if (!ok0 || !ok1)
 	{
-		std::cout << "Error: unable to read sequences" << std::endl;
-		ExitNow(1);
+		msg.Out("Error: unable to read sequences\n");
+		return false;
 	}
 	const int T = ToolThreads();
 	std::thread fastq_thread([&] {
@@ -183,32 +247,32 @@ int main(int argc, char* argv[])
 	// The reference reads both fastq files to the end before it opens the SAM file (tools/dosplitalign.cpp:93-110), so
 	// whatever the fastq streams have to say -- and a fatal fragment name -- comes before any SAM error.
 	auto finish_fastq = [&]() {
-		if (!fastq_thread.joinable()) return;
+		if (!fastq_thread.joinable()) return true;
 		fastq_thread.join();
 		for (int file = 0; file <= 1; file++)
 		{
-			std::cerr << fastq[file].Message();
-			if (fastq[file].Fatal()) ExitNow(1);
+			msg.Err(fastq[file].Message());
+			if (fastq[file].Fatal()) return false;
 		}
+		return true;
 	};
 
-	timer.Lap("bins");
-	const int n_gpus = (int)gpus.size();
+	timer.Lap("fastq open");
 
 	// ---- candidates, in the reference's order (SplitAlignment.cpp:266-303): SAM record order x iteration order of
 	//      the overlap set; once per (cluster, read id, revComp).  Chunks of lines are parsed in parallel (every chunk
 	//      keeps, per record, the overlap set in its iteration order), then merged in file order. ----
 	// (plain arrays below: a std::vector would zero hundreds of megabytes on one thread before the workers fill them)
-	std::unique_ptr<Candidate[]> candidates;
-	size_t n_candidates = 0;
+	std::unique_ptr<Candidate[]>& candidates = in.candidates;
+	size_t& n_candidates = in.n_candidates;
 	{
 		MappedInput sam;
-		const bool opened = cmd.Str('i') == "-" ? sam.OpenStdin() : sam.OpenFile(cmd.Str('i'));
+		const bool opened = paths.improper == "-" ? sam.OpenStdin() : sam.OpenFile(paths.improper);
 		if (!opened)
 		{
-			finish_fastq();
-			std::cerr << "Error: Unable to open sam file " << cmd.Str('i') << std::endl;
-			ExitNow(1);
+			if (!finish_fastq()) return false;
+			msg.Err("Error: Unable to open sam file " + paths.improper + "\n");
+			return false;
 		}
 		const char* const base = sam.data();
 		std::vector<LineChunk> chunks = SplitLines(base, sam.size(), T);
@@ -225,9 +289,9 @@ int main(int argc, char* argv[])
 			const char* const end = base + chunks[(size_t)c].end;
 			int64_t line_number = chunks[(size_t)c].first_line;
 			std::string ref_name;
-			auto fail = [&](const std::string& msg) {
+			auto fail = [&](const std::string& what) {
 				part.error_line = line_number;
-				part.error = msg;
+				part.error = what;
 			};
 			while (a < end)
 			{
@@ -280,7 +344,7 @@ int main(int argc, char* argv[])
 				const Region r{pos, pos + (int)(f[10] - 1 - f[9]) - 1};
 				ref_name.assign(f[2], f[3] - 1);
 				std::unordered_set<int> overlapping;
-				binned.Overlapping(ref_name, strand, r, overlapping);
+				s.binned.Overlapping(ref_name, strand, r, overlapping);
 				if (overlapping.empty()) continue;
 				int fragment_index = 0;
 				if (!ParseIntRange(qb, fragment_end, fragment_index))
@@ -295,9 +359,9 @@ int main(int argc, char* argv[])
 			if (part.error_line >= 0)
 			{
 				// (chunks are in file order: this is the first line a sequential reader would have died on)
-				finish_fastq();
-				std::cerr << part.error << std::endl;
-				ExitNow(1);
+				if (!finish_fastq()) return false;
+				msg.Err(part.error + "\n");
+				return false;
 			}
 		timer.Lap("sam parse + overlaps");
 		// expand the per-chunk streams into one candidate list (file order), then keep the first occurrence of every
@@ -405,31 +469,41 @@ int main(int argc, char* argv[])
 					candidates[at++] = Candidate{(int)(uint32_t)(keys[k] >> 33), (int)(uint32_t)((keys[k] >> 1) & 0xFFFFFFFFull), (int)(keys[k] & 1)};
 		});
 	}
-
 	timer.Lap("candidates (dedupe)");
+	if (!finish_fastq()) return false;
+	timer.Lap("fastq (wait)");
+	return true;
+}
+
+// One split from its candidates to its finished alignments file; `records` (the fused tool) also gets every record.
+// false: the output cannot be opened, the message said.  A GPU that fails ends the process here, as in the stock tool;
+// every split before this one is finished by then.
+bool AlignSplit(const SharedSetup& s, const SplitPaths& paths, const SplitInput& in, BatchBuffers& buf, Messages& msg,
+                PhaseTimer& timer, std::string* records)
+{
 	// ---- the reads the candidates need (the reference keeps every read of both files, SplitAlignment.cpp:253-264, the
 	//      second file overwriting the first; a read id that is absent aligns as the empty string, :286) ----
-	finish_fastq();
+	const FastqIndex* const fastq = in.fastq;
 	auto find_read = [&](int id, const char*& seq, uint32_t& len) {
 		if (fastq[1].Find(id, seq, len) || fastq[0].Find(id, seq, len)) return;
 		seq = nullptr;
 		len = 0;
 	};
+	const Candidate* const candidates = in.candidates.get();
+	const size_t n_candidates = in.n_candidates;
+	const std::vector<std::unique_ptr<Gpu>>& gpus = s.gpus;
+	const int n_gpus = (int)gpus.size();
+	const std::unordered_map<int, int>& cluster_slot = s.cluster_slot;
+	const TableBuilder& windows = s.windows;
+	const int T = ToolThreads();
 
-	timer.Lap("fastq (wait)");
-#ifdef DFB_FUSED_EVAL
-	const bool write_align = cmd.IsSet('a');
+	const bool write_align = paths.write_align;
 	std::ofstream out;
-	if (write_align) out.open(cmd.Str('a').c_str());
-	std::string fused_text; // every record of the run, in emission order
-#else
-	const bool write_align = true;
-	std::ofstream out(cmd.Str('a').c_str());
-#endif
+	if (write_align) out.open(paths.align.c_str());
 	if (write_align && !out.good())
 	{
-		std::cerr << "Error: Unable to open " << cmd.Str('a') << std::endl;
-		ExitNow(1);
+		msg.Err("Error: Unable to open " + paths.align + "\n");
+		return false;
 	}
 
 	// ---- align in batches, write records in candidate order ----
@@ -437,26 +511,13 @@ int main(int argc, char* argv[])
 	const dfb_seq_table window_table = windows.View();
 	size_t kBatch = (size_t)(1u << 20) * (size_t)n_gpus; // (a batch twice as large costs the process another ~0.4 s of first-use device allocation)
 	if (const char* e = getenv("DFB_TOOL_BATCH")) kBatch = (size_t)std::max(1, atoi(e)); // tests: force several batches
-	struct Shard
-	{
-		// the batch's reads as a CSR table; the bytes are a plain array that the worker threads touch first
-		std::unique_ptr<char[]> read_bytes;
-		size_t read_bytes_cap = 0;
-		std::vector<int64_t> read_off;
-		std::vector<int32_t> task_cluster, task_read, task_min_score, best, read_len, ref2_len;
-		std::vector<int64_t> row_begin; // first result row of each task (n_rows when it has none)
-		const dfb_split_row* rows = nullptr;
-		const int32_t* cols = nullptr;
-		int64_t n_rows = 0, n_cols = 0;
-		int rc = DFB_OK;
-	};
-	std::vector<Shard> shards((size_t)n_gpus);
-	std::vector<int> gpu_of;
-	std::vector<int32_t> local_of;        // index of a candidate inside its shard
-	std::vector<const char*> cand_seq;    // the candidate's read in the mapped fastq (forward orientation)
-	std::vector<uint32_t> cand_len;
-	std::vector<int32_t> cand_slot;
-	std::vector<std::string> out_parts((size_t)T);
+	std::vector<Shard>& shards = buf.shards;
+	std::vector<int>& gpu_of = buf.gpu_of;
+	std::vector<int32_t>& local_of = buf.local_of;
+	std::vector<const char*>& cand_seq = buf.cand_seq;
+	std::vector<uint32_t>& cand_len = buf.cand_len;
+	std::vector<int32_t>& cand_slot = buf.cand_slot;
+	std::vector<std::string>& out_parts = buf.out_parts;
 	timer.Lap("open output");
 	static unsigned char complement[256];
 	for (int k = 0; k < 256; k++) complement[k] = (unsigned char)k;
@@ -705,9 +766,8 @@ int main(int argc, char* argv[])
 		timer.Add("batch: format");
 		if (write_align)
 			for (const std::string& part : out_parts) out.write(part.data(), (std::streamsize)part.size());
-#ifdef DFB_FUSED_EVAL
-		for (const std::string& part : out_parts) fused_text += part;
-#endif
+		if (records)
+			for (const std::string& part : out_parts) *records += part;
 		timer.Add("batch: write");
 	}
 	if (write_align)
@@ -715,6 +775,82 @@ int main(int argc, char* argv[])
 		out.flush();
 		out.close();
 	}
+	return true;
+}
+
+#ifdef DFB_MULTI_SPLIT
+// The split manifest: one split per line, four TAB-separated paths (seq1.fastq, seq2.fastq, improper.sam, output).
+// Anything malformed ends the run before a split is read or an output created.
+std::vector<SplitPaths> ReadManifest(const std::string& path)
+{
+	auto fail = [](const std::string& what) {
+		std::cerr << "Error: " << what << std::endl;
+		ExitNow(1);
+	};
+	std::ifstream in(path.c_str());
+	if (!in.good()) fail("Unable to read splits manifest " + path);
+	std::vector<SplitPaths> splits;
+	std::set<std::string> outputs;
+	std::string line;
+	std::vector<std::string> f;
+	while (std::getline(in, line))
+	{
+		const std::string where = "splits manifest " + path + " line " + std::to_string(splits.size() + 1);
+		SplitChar(line, '\t', f);
+		if (f.size() != 4 || f[0].empty() || f[1].empty() || f[2].empty() || f[3].empty())
+			fail("Expected four non-empty tab-separated fields (seq1, seq2, improper sam, output) on " + where);
+		for (const std::string& p : f)
+			if (p == "-") fail("'-' names standard input or output, which cannot serve several splits, on " + where);
+		if (!outputs.insert(f[3]).second) fail("Output " + f[3] + " is named a second time on " + where);
+		splits.push_back(SplitPaths{f[0], f[1], f[2], f[3]});
+	}
+	if (in.bad()) fail("Unable to read splits manifest " + path);
+	if (splits.empty()) fail("Splits manifest " + path + " has no lines");
+	return splits;
+}
+#endif
+
+}  // namespace
+
+#ifndef DFB_MULTI_SPLIT
+int main(int argc, char* argv[])
+{
+	CommandLine cmd("Fusion sequence prediction by split reads", {
+	    {'f', "fasta", "Reference Fasta", true, "string", "", false},
+	    {'e', "exons", "Exon Regions Filename", true, "string", "", false},
+	    {'u', "ufrag", "Fragment Length Mean", true, "float", "", false},
+	    {'s', "sfrag", "Fragment Length Standard Deviation", true, "float", "", false},
+	    {'n', "minread", "Minimum Read Length", true, "integer", "", false},
+	    {'x', "maxread", "Maximum Read Length", true, "integer", "", false},
+	    {'r', "regions", "Fusion Regions Filename", true, "string", "", false},
+	    {'i', "improper", "Improper Alignments Sam Filename", true, "string", "", false},
+	    {'1', "seq1", "End 1 Sequences", true, "string", "", false},
+	    {'2', "seq2", "End 2 Sequences", true, "string", "", false},
+#ifdef DFB_FUSED_EVAL
+	    {'a', "align", "Split Alignments Filename (optional here)", false, "string", "", false},
+	    {'q', "seq", "Sequences Filename", true, "string", "", false},
+	    {'b', "break", "Break Positions Filename", true, "string", "", false},
+	    {'p', "predalign", "Prediction Split Alignments Filename", true, "string", "", false},
+#else
+	    {'a', "align", "Split Alignments Filename", true, "string", "", false},
+#endif
+	});
+	cmd.Parse(argc, argv);
+	PhaseTimer timer;
+	SharedSetup shared;
+	ReadSharedSetup(cmd, shared, timer);
+	SplitPaths paths{cmd.Str('1'), cmd.Str('2'), cmd.Str('i'), cmd.Str('a')};
+	std::string* records = nullptr;
+#ifdef DFB_FUSED_EVAL
+	paths.write_align = cmd.IsSet('a');
+	std::string fused_text; // every record of the run, in emission order
+	records = &fused_text;
+#endif
+	Messages direct(false);
+	SplitInput in;
+	if (!IngestSplit(shared, paths, in, direct, timer)) ExitNow(1);
+	BatchBuffers buf((int)shared.gpus.size());
+	if (!AlignSplit(shared, paths, in, buf, direct, timer, records)) ExitNow(1);
 #ifdef DFB_FUSED_EVAL
 	{
 		// align -> evaluate without the file in between (tools/evalsplitalign.cpp:96-114 on the sorted records)
@@ -727,7 +863,7 @@ int main(int argc, char* argv[])
 			}
 		const std::string sorted = SortRecordsLikeThePipeline(fused_text);
 		timer.Lap("fused: sort records");
-		const bool ok = EvaluateSortedRecords(sorted.data(), sorted.data() + sorted.size(), tasks, seq_file, break_file, pred_file);
+		const bool ok = EvaluateSortedRecords(sorted.data(), sorted.data() + sorted.size(), shared.tasks, seq_file, break_file, pred_file);
 		timer.Lap("fused: evaluate");
 		if (!ok) ExitNow(1);
 	}
@@ -736,3 +872,68 @@ int main(int argc, char* argv[])
 	timer.Lap("close");
 	FinishProcess(0);
 }
+#else
+int main(int argc, char* argv[])
+{
+	CommandLine cmd("Fusion sequence prediction by split reads, every fastq split of a run in one process", {
+	    {'f', "fasta", "Reference Fasta", true, "string", "", false},
+	    {'e', "exons", "Exon Regions Filename", true, "string", "", false},
+	    {'u', "ufrag", "Fragment Length Mean", true, "float", "", false},
+	    {'s', "sfrag", "Fragment Length Standard Deviation", true, "float", "", false},
+	    {'n', "minread", "Minimum Read Length", true, "integer", "", false},
+	    {'x', "maxread", "Maximum Read Length", true, "integer", "", false},
+	    {'r', "regions", "Fusion Regions Filename", true, "string", "", false},
+	    {'l', "splits", "Splits Manifest Filename (per line: seq1 <TAB> seq2 <TAB> improper sam <TAB> alignments)", true, "string", "", false},
+	});
+	cmd.Parse(argc, argv);
+	const std::vector<SplitPaths> splits = ReadManifest(cmd.Str('l'));
+	PhaseTimer timer;
+	SharedSetup shared;
+	ReadSharedSetup(cmd, shared, timer); // (says nothing unless it fails, and then it exits: said once, as by the first stock run)
+	BatchBuffers buf((int)shared.gpus.size());
+	// Split k+1's ingest runs on a helper thread while split k is aligned and written, its messages held until split k
+	// is done; at most two splits' inputs are mapped at once.  DFB_SPLIT_OVERLAP=0: one split after the other.
+	const bool overlap = !(getenv("DFB_SPLIT_OVERLAP") && atoi(getenv("DFB_SPLIT_OVERLAP")) == 0);
+	auto label = [](size_t k) { return "split " + std::to_string(k + 1) + ": "; };
+	Messages direct(false);
+	std::unique_ptr<SplitInput> current(new SplitInput);
+	std::unique_ptr<PhaseTimer> split_timer(new PhaseTimer(label(0)));
+	if (!IngestSplit(shared, splits[0], *current, direct, *split_timer)) ExitNow(1);
+	for (size_t k = 0; k < splits.size(); k++)
+	{
+		const bool last = k + 1 == splits.size();
+		std::unique_ptr<SplitInput> next;
+		std::unique_ptr<PhaseTimer> next_timer;
+		Messages held(true);
+		bool next_ok = true;
+		std::thread ahead;
+		if (overlap && !last)
+		{
+			next.reset(new SplitInput);
+			next_timer.reset(new PhaseTimer(label(k + 1)));
+			ahead = std::thread([&] { next_ok = IngestSplit(shared, splits[k + 1], *next, held, *next_timer); });
+		}
+		split_timer->Restart();
+		if (!AlignSplit(shared, splits[k], *current, buf, direct, *split_timer, nullptr)) ExitNow(1);
+		split_timer->Report();
+		current.reset(); // (split k's inputs are unmapped before split k+2's ingest maps more)
+		if (last) break;
+		if (overlap)
+		{
+			ahead.join();
+			held.Release();
+			if (!next_ok) ExitNow(1);
+			current = std::move(next);
+			split_timer = std::move(next_timer);
+		}
+		else
+		{
+			current.reset(new SplitInput);
+			split_timer.reset(new PhaseTimer(label(k + 1)));
+			if (!IngestSplit(shared, splits[k + 1], *current, direct, *split_timer)) ExitNow(1);
+		}
+	}
+	timer.Lap("close");
+	FinishProcess(0);
+}
+#endif

@@ -440,19 +440,26 @@ inline std::vector<int> DeviceList()
 	return out;
 }
 
-// DFB_TRACE=1: phase timings of a tool on stderr (stdout / the -a file stay byte-exact)
+// DFB_TRACE=1: phase timings of a tool on stderr (stdout / the -a file stay byte-exact); `label` goes in front of
+// every line (dosplitalign_multi: which split)
 class PhaseTimer
 {
 public:
-	PhaseTimer() : mOn(getenv("DFB_TRACE") && *getenv("DFB_TRACE") && *getenv("DFB_TRACE") != '0') { clock_gettime(CLOCK_MONOTONIC, &mT); }
+	explicit PhaseTimer(std::string label = "")
+	    : mOn(getenv("DFB_TRACE") && *getenv("DFB_TRACE") && *getenv("DFB_TRACE") != '0'), mLabel(std::move(label))
+	{
+		clock_gettime(CLOCK_MONOTONIC, &mT);
+	}
 	void Lap(const char* what)
 	{
 		if (!mOn) return;
 		timespec t;
 		clock_gettime(CLOCK_MONOTONIC, &t);
-		fprintf(stderr, "[tool] %-28s %9.3f ms\n", what, (t.tv_sec - mT.tv_sec) * 1e3 + (t.tv_nsec - mT.tv_nsec) * 1e-6);
+		fprintf(stderr, "[tool] %s%-28s %9.3f ms\n", mLabel.c_str(), what, (t.tv_sec - mT.tv_sec) * 1e3 + (t.tv_nsec - mT.tv_nsec) * 1e-6);
 		mT = t;
 	}
+	// the next lap starts now (time spent waiting elsewhere is charged to no phase)
+	void Restart() { clock_gettime(CLOCK_MONOTONIC, &mT); }
 
 	// accumulating form for phases that repeat per batch: Add("name") charges the time since the last call to a
 	// named bucket, Report() prints the buckets
@@ -473,12 +480,13 @@ public:
 	}
 	void Report()
 	{
-		for (auto& b : mBuckets) fprintf(stderr, "[tool] %-28s %9.3f ms\n", b.first.c_str(), b.second);
+		for (auto& b : mBuckets) fprintf(stderr, "[tool] %s%-28s %9.3f ms\n", mLabel.c_str(), b.first.c_str(), b.second);
 		mBuckets.clear();
 	}
 
 private:
 	bool mOn;
+	std::string mLabel;
 	timespec mT;
 	std::vector<std::pair<std::string, double>> mBuckets;
 };

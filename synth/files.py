@@ -151,6 +151,37 @@ def make_split_dataset(outdir, seed=1, n_clusters=40, pairs_per_cluster=30, L=10
             "-2", os.path.join(outdir, "reads.2.fastq")]
 
 
+def cut_splits(outdir, n_splits):
+    """Cut the reads of a make_split_dataset directory into n_splits fastq splits, as split_fastq.pl does with real
+    reads: fragment f goes to split f % n_splits, file order is kept, every split's SAM starts with the header.  Writes
+    split.K.1.fastq, split.K.2.fastq and split.K.improper.sam (K = 0 .. n_splits-1) and returns, per split, the list
+    [seq1, seq2, improper sam].  Every split sees every cluster."""
+    def fragment(name):  # "@12/1" (fastq) or "12/1" (SAM qname)
+        return int(name.lstrip(b"@").split(b"/", 1)[0])
+
+    fq = []
+    for end in (1, 2):
+        lines = open(os.path.join(outdir, "reads.%d.fastq" % end), "rb").read().splitlines(keepends=True)
+        parts = [[] for _ in range(n_splits)]
+        for k in range(0, len(lines), 4):
+            parts[fragment(lines[k]) % n_splits] += lines[k:k + 4]
+        fq.append(parts)
+    header, sam = [], [[] for _ in range(n_splits)]
+    for line in open(os.path.join(outdir, "improper.sam"), "rb").read().splitlines(keepends=True):
+        if line.startswith(b"@"):
+            header.append(line)
+        else:
+            sam[fragment(line.split(b"\t", 1)[0]) % n_splits].append(line)
+    out = []
+    for k in range(n_splits):
+        paths = [os.path.join(outdir, "split.%d.%s" % (k, name)) for name in ("1.fastq", "2.fastq", "improper.sam")]
+        for path, data in zip(paths, (fq[0][k], fq[1][k], header + sam[k])):
+            with open(path, "wb") as f:
+                f.write(b"".join(data))
+        out.append(paths)
+    return out
+
+
 def write_read_index(outdir):
     """<outdir>/reads.fqi for reads.{1,2}.fastq: little-endian int64 offsets of the '@' lines, entry 2*fragment+end
     (tools/ReadIndex.cpp:67-77; writer scripts/index_paired_fastq.pl:56-60).  Returns the reads prefix."""
