@@ -42,6 +42,10 @@ class _SeqTable(ctypes.Structure):
     _fields_ = [("bytes", ctypes.c_void_p), ("off", ctypes.c_void_p), ("n", ctypes.c_int64)]
 
 
+class _DeviceSeqTable(ctypes.Structure):
+    _fields_ = [("bytes", ctypes.c_void_p), ("off", ctypes.c_void_p), ("n", ctypes.c_int64), ("n_bytes", ctypes.c_int64)]
+
+
 class _SimpleParams(ctypes.Structure):
     _fields_ = [("match", ctypes.c_int32), ("mismatch", ctypes.c_int32), ("gap", ctypes.c_int32)]
 
@@ -117,6 +121,10 @@ def load_library():
         "dfb_plan_destroy": ([vp], None),
         "dfb_microbench_issue_rate": ([vp, ctypes.c_int, ctypes.c_int, P(ctypes.c_double), P(ctypes.c_double)], ctypes.c_int),
         "dfb_ctx_memory_info": ([vp, ctypes.c_int, P(i64), P(i64), P(i64)], ctypes.c_int),
+        "dfb_simple_align_device": ([vp, P(_SimpleParams), P(_DeviceSeqTable), P(_DeviceSeqTable), vp, vp, i64, vp], ctypes.c_int),
+        "dfb_split_align_device": ([vp, P(_SplitParams), P(_DeviceSeqTable), P(_DeviceSeqTable), vp, vp, vp, i64, vp, P(i64), P(i64)],
+                                   ctypes.c_int),
+        "dfb_split_result_copy_device": ([vp, vp, vp], ctypes.c_int),
         "dfb_split_backtrace_batch": ([vp, P(_SplitParams), P(_SeqTable), P(_SeqTable), vp, vp, vp, vp, vp, i64, vp, vp, i64,
                                        P(i64)], ctypes.c_int),
     }
@@ -135,7 +143,7 @@ ABI_SYMBOLS = (
     "dfb_plan_set_timing",
     "dfb_simple_plan_fetch", "dfb_split_plan_fetch", "dfb_split_plan_copy", "dfb_plan_get_stats", "dfb_plan_destroy",
     "dfb_microbench_issue_rate", "dfb_split_backtrace_batch", "dfb_ctx_memory_info",
-    "dfb_split_result_stats",
+    "dfb_split_result_stats", "dfb_simple_align_device", "dfb_split_align_device", "dfb_split_result_copy_device",
 )
 
 
@@ -178,6 +186,55 @@ def _i32(a):
     return np.ascontiguousarray(a, dtype=np.int32)
 
 
+def _check_tensor(name, t, dtype, device=None):
+    """A contiguous 1-D CUDA tensor of `dtype` (on `device` when given); TypeError / ValueError otherwise."""
+    import torch
+    if not isinstance(t, torch.Tensor):
+        raise TypeError("%s must be a torch.Tensor, got %s" % (name, type(t).__name__))
+    if t.dtype != dtype:
+        raise TypeError("%s must be %s, got %s" % (name, dtype, t.dtype))
+    if not t.is_cuda:
+        raise ValueError("%s must be a CUDA tensor, got one on %s" % (name, t.device))
+    if device is not None and t.device != device:
+        raise ValueError("%s is on %s, expected %s" % (name, t.device, device))
+    if t.dim() != 1 or not t.is_contiguous():
+        raise ValueError("%s must be a contiguous 1-D tensor" % name)
+    return t
+
+
+def _dptr(t):
+    """Device address of a tensor; a placeholder for an empty one (the library reads nothing through it)."""
+    return t.data_ptr() if t.numel() else 0
+
+
+class DeviceSeqTable:
+    """CSR table of byte strings in GPU memory: `data` (torch.uint8) and `off` (torch.int64, n + 1 entries), contiguous
+    CUDA tensors on one device.  The device-resident aligner calls read them where they are."""
+
+    def __init__(self, data, off):
+        import torch
+        _check_tensor("data", data, torch.uint8)
+        _check_tensor("off", off, torch.int64, data.device)
+        if off.numel() < 1:
+            raise ValueError("off must hold n + 1 >= 1 entries")
+        self.data = data
+        self.off = off
+        self.device = data.device
+
+    @classmethod
+    def from_host(cls, table, device):
+        """The device copy of a SeqTable."""
+        import torch
+        data = table.data if table.data.flags.writeable else table.data.copy()   # (torch refuses read-only arrays)
+        return cls(torch.from_numpy(data).to(device), torch.from_numpy(table.off).to(device))
+
+    def __len__(self):
+        return self.off.numel() - 1
+
+    def c_struct(self):
+        return _DeviceSeqTable(_dptr(self.data), _dptr(self.off), len(self), self.data.numel())
+
+
 # ------------------------------------------------------------------------------------------------
 # context and plans
 # ------------------------------------------------------------------------------------------------
@@ -212,6 +269,19 @@ class Context:
     def set_stream(self, cuda_stream_ptr):
         """Run on a caller's cudaStream_t (e.g. torch.cuda.current_stream().cuda_stream); None resets."""
         self._check(self._lib.dfb_ctx_set_stream(self._h, ctypes.c_void_p(cuda_stream_ptr or 0)))
+        self._stream = cuda_stream_ptr or None
+
+    def _on_torch_stream(self, fn):
+        """fn() with the context on torch's current stream of its device; the context's stream is restored after."""
+        import torch
+        prev = getattr(self, "_stream", None)
+        # torch's default stream is the legacy NULL stream (handle 0); the library takes NULL to mean its own non-blocking
+        # stream, which would not wait for torch's work, so it gets cudaStreamLegacy ((cudaStream_t)1) instead
+        self.set_stream(torch.cuda.current_stream(self.device).cuda_stream or 1)
+        try:
+            return fn()
+        finally:
+            self.set_stream(prev)
 
     def device_info(self):
         info = _DeviceInfo()
@@ -352,6 +422,54 @@ class SplitResult:
         return np.array(out, dtype=np.int32).reshape(-1, 5)
 
 
+class DeviceSplitResult:
+    """Result of SplitReadAligner.align_device, in GPU memory: `best` (int32, per task), `rows` (the 32-byte
+    dfb_split_row records as an (n, 8) int32 tensor; the field accessors below read it) and `cols` (int32 column pool)."""
+
+    def __init__(self, best, rows, cols, lens):
+        self.best = best
+        self.rows = rows
+        self.cols = cols
+        self._lens = lens
+
+    # fields of the records (SPLIT_ROW_DTYPE): task, read_split, score1, score2, col_begin (int64), n1, n2
+    @property
+    def task(self):
+        return self.rows[:, 0]
+
+    @property
+    def read_split(self):
+        return self.rows[:, 1]
+
+    @property
+    def score1(self):
+        return self.rows[:, 2]
+
+    @property
+    def score2(self):
+        return self.rows[:, 3]
+
+    @property
+    def col_begin(self):
+        import torch
+        return self.rows[:, 4:6].contiguous().view(torch.int64).reshape(-1)
+
+    @property
+    def n1(self):
+        return self.rows[:, 6]
+
+    @property
+    def n2(self):
+        return self.rows[:, 7]
+
+    def to_host(self):
+        """The same result as a SplitResult (host arrays), so that alignments() / records() work.  The read and window
+        lengths it needs are read from the batch's tables and task tensors now: call it before reusing them."""
+        rows = np.ascontiguousarray(self.rows.cpu().numpy()).view(SPLIT_ROW_DTYPE).reshape(-1)
+        lens = self._lens()
+        return SplitResult(self.best.cpu().numpy(), rows, self.cols.cpu().numpy(), lambda: lens)
+
+
 def _view_arrays(rows_p, n_rows, cols_p, n_cols, copy):
     """numpy arrays over (or copied from) the library-owned result buffers."""
     if n_rows:
@@ -419,6 +537,28 @@ class SimpleAligner:
                                                              task_ref.size, out.ctypes.data))
         return out
 
+    def align_device(self, refs, seqs, task_ref, task_seq, out=None):
+        """align_batch for a batch in GPU memory (DeviceSeqTable, int32 CUDA tensors) through dfb_simple_align_device:
+        nothing but counters crosses PCIe.  Returns `out` (int32 CUDA tensor), written on torch's current stream."""
+        import torch
+        dev = _device_args(self.ctx, refs, seqs)
+        _check_tensor("task_ref", task_ref, torch.int32, dev)
+        _check_tensor("task_seq", task_seq, torch.int32, dev)
+        if task_ref.numel() != task_seq.numel():
+            raise ValueError("task_ref and task_seq differ in length")
+        n = task_ref.numel()
+        if out is None:
+            out = torch.empty(n, dtype=torch.int32, device=dev)
+        _check_tensor("out", out, torch.int32, dev)
+        if out.numel() < n:
+            raise ValueError("out holds fewer than n_tasks entries")
+        rt, st = refs.c_struct(), seqs.c_struct()
+        lib = self.ctx._lib
+        self.ctx._on_torch_stream(lambda: self.ctx._check(lib.dfb_simple_align_device(
+            self.ctx._h, ctypes.byref(self.params), ctypes.byref(rt), ctypes.byref(st), _dptr(task_ref), _dptr(task_seq), n,
+            _dptr(out))))
+        return out
+
     def Align(self, reference, sequence):
         """int SimpleAligner::Align(const string& reference, const string& sequence)."""
         return int(self.align_batch(SeqTable.from_list([reference]), SeqTable.from_list([sequence]), [0], [0])[0])
@@ -475,6 +615,43 @@ class SplitReadAligner:
         rows, cols = _view_arrays(rp.value, n_rows.value, cp.value, n_cols.value, copy)
         return SplitResult(best, rows, cols, lambda: self._lens(refs, reads, task_cluster, task_read))
 
+    def align_device(self, refs, reads, task_cluster, task_read, task_min_score, out=None):
+        """align_batch for a batch in GPU memory (DeviceSeqTable, int32 CUDA tensors) through dfb_split_align_device.
+        Returns a DeviceSplitResult whose best / rows / cols are CUDA tensors equal to align_batch's arrays; the work
+        runs on torch's current stream and nothing but counters crosses PCIe."""
+        import torch
+        dev = _device_args(self.ctx, refs, reads)
+        for name, t in (("task_cluster", task_cluster), ("task_read", task_read), ("task_min_score", task_min_score)):
+            _check_tensor(name, t, torch.int32, dev)
+        n = task_cluster.numel()
+        if task_read.numel() != n or task_min_score.numel() != n:
+            raise ValueError("task arrays differ in length")
+        if out is None:
+            out = torch.empty(n, dtype=torch.int32, device=dev)
+        _check_tensor("out", out, torch.int32, dev)
+        if out.numel() < n:
+            raise ValueError("out holds fewer than n_tasks entries")
+        rt, st = refs.c_struct(), reads.c_struct()
+        lib, h = self.ctx._lib, self.ctx._h
+        n_rows, n_cols = ctypes.c_int64(), ctypes.c_int64()
+
+        def run():
+            self.ctx._check(lib.dfb_split_align_device(h, ctypes.byref(self.params), ctypes.byref(rt), ctypes.byref(st),
+                                                       _dptr(task_cluster), _dptr(task_read), _dptr(task_min_score), n,
+                                                       _dptr(out), ctypes.byref(n_rows), ctypes.byref(n_cols)))
+            rows = torch.empty((n_rows.value, 8), dtype=torch.int32, device=dev)
+            cols = torch.empty(n_cols.value, dtype=torch.int32, device=dev)
+            self.ctx._check(lib.dfb_split_result_copy_device(h, _dptr(rows), _dptr(cols)))
+            return rows, cols
+
+        rows, cols = self.ctx._on_torch_stream(run)
+
+        def lens():
+            tc, tr = task_cluster.cpu().numpy(), task_read.cpu().numpy()
+            return self._lens(SeqTable(np.zeros(0, np.uint8), refs.off.cpu().numpy()),
+                              SeqTable(np.zeros(0, np.uint8), reads.off.cpu().numpy()), tc, tr)
+        return DeviceSplitResult(out[:n], rows, cols, lens)
+
     def backtrace_batch(self, refs, reads, task_cluster, task_read, ref_split1, ref_split2, read_split):
         """matches1 / matches2 of chosen alignments (GetAlignments(..., backtrace=True), tools/SplitReadAligner.cpp:
         124-154,287-292) through dfb_split_backtrace_batch.  Task t names the alignment of reads[task_read[t]] against
@@ -513,6 +690,18 @@ class SplitReadAligner:
         n = len(al)
         off, pairs = self.backtrace_batch(refs, reads, np.zeros(n, np.int32), np.zeros(n, np.int32), al[:, 0], al[:, 1], al[:, 2])
         return [(al[k], pairs[off[2 * k]:off[2 * k + 1]], pairs[off[2 * k + 1]:off[2 * k + 2]]) for k in range(n)]
+
+
+def _device_args(ctx, *tables):
+    """The CUDA device of the context, which every DeviceSeqTable must be on."""
+    import torch
+    dev = torch.device("cuda", ctx.device)
+    for t in tables:
+        if not isinstance(t, DeviceSeqTable):
+            raise TypeError("tables must be DeviceSeqTable, got %s" % type(t).__name__)
+        if t.device != dev:
+            raise ValueError("table is on %s, the context on %s" % (t.device, dev))
+    return dev
 
 
 def split_min_score(read_len, match=2):

@@ -12,8 +12,8 @@
 //    spread over host threads.
 #include "../../include/defuse_b200.h"
 #include "dfb_kernels.cuh"
-#include "dfb_assemble.cuh"
 #include "dfb_build.cuh"
+#include "dfb_assemble.cuh"
 
 #include <algorithm>
 #include <cstdarg>
@@ -662,6 +662,12 @@ struct dfb_plan
 	unsigned long long* d_asm_sums = nullptr; // [blocks][2] + totals[2] behind them
 	int64_t asm_blocks = 0;
 	int64_t n_fast_tasks = 0;
+	bool dev_inputs = false; // tables (and, for a device build, offsets and tasks) are the caller's device memory
+	// result holder of dfb_split_align_device: the batch's rows and columns in device memory
+	dfb_split_row* d_res_rows = nullptr;
+	int32_t* d_res_cols = nullptr;
+	int64_t d_res_n_rows = 0, d_res_n_cols = 0;
+	bool device_result = false;
 
 	// host
 	std::vector<int32_t> task_L; // read length per task (split)
@@ -771,6 +777,8 @@ static void release_device(dfb_plan* plan)
 	dfree(ctx, plan->d_asm_rows);
 	dfree(ctx, plan->d_asm_cols);
 	dfree(ctx, plan->d_asm_sums);
+	dfree(ctx, plan->d_res_rows);
+	dfree(ctx, plan->d_res_cols);
 }
 
 extern "C" void dfb_plan_destroy(dfb_plan* plan)
@@ -987,17 +995,26 @@ static cudaError_t h2d_any(dfb_ctx* ctx, cudaStream_t up, void* dst, const void*
 }
 
 // Starts the copy of the raw sequence bytes before the host builds descriptors and jobs: with pinned
-// caller buffers the transfer runs underneath that host work.
-static int upload_raw(dfb_plan* pl, const dfb_seq_table* a, const dfb_seq_table* b)
+// caller buffers the transfer runs underneath that host work.  `dev_range` (device-resident tables): the bytes are
+// device memory, [a0, a1) of table A's and [b0, b1) of table B's; they are copied device to device (the pack kernel
+// reads whole 16-byte windows, so it never reads the caller's allocation itself).
+static int upload_raw(dfb_plan* pl, const dfb_seq_table* a, const dfb_seq_table* b, const int64_t* dev_range = nullptr)
 {
 	dfb_ctx* ctx = pl->ctx;
 	cudaStream_t up = pl->up ? pl->up : ctx->stream;
-	const int64_t na = a->off[a->n] - a->off[0], nb = b->off[b->n] - b->off[0];
+	const int64_t a0 = dev_range ? dev_range[0] : a->off[0], b0 = dev_range ? dev_range[2] : b->off[0];
+	const int64_t na = (dev_range ? dev_range[1] : a->off[a->n]) - a0, nb = (dev_range ? dev_range[3] : b->off[b->n]) - b0;
 	// 16 bytes of slack in front, 32 behind (the pack kernel reads whole 16-byte windows)
 	CK(ctx, cudaMallocAsync((void**)&pl->d_raw, std::max<size_t>(256, (size_t)(na + nb + 48)), up));
 	pl->raw_bytes = (unsigned long long)(na + nb + 48);
-	if (na) CK(ctx, h2d_any(ctx, up, pl->d_raw + 16, a->bytes + a->off[0], (size_t)na));
-	if (nb) CK(ctx, h2d_any(ctx, up, pl->d_raw + 16 + na, b->bytes + b->off[0], (size_t)nb));
+	if (dev_range)
+	{
+		if (na) CK(ctx, cudaMemcpyAsync(pl->d_raw + 16, a->bytes + a0, (size_t)na, cudaMemcpyDeviceToDevice, up));
+		if (nb) CK(ctx, cudaMemcpyAsync(pl->d_raw + 16 + na, b->bytes + b0, (size_t)nb, cudaMemcpyDeviceToDevice, up));
+		return DFB_OK;
+	}
+	if (na) CK(ctx, h2d_any(ctx, up, pl->d_raw + 16, a->bytes + a0, (size_t)na));
+	if (nb) CK(ctx, h2d_any(ctx, up, pl->d_raw + 16 + na, b->bytes + b0, (size_t)nb));
 	return DFB_OK;
 }
 
@@ -1039,7 +1056,7 @@ static int upload_and_pack(dfb_plan* pl, const dfb_seq_table* a, int mode_a, con
 		if (!pl->packed_ev) CK(ctx, cudaEventCreateWithFlags(&pl->packed_ev, cudaEventDisableTiming));
 		CK(ctx, cudaEventRecord(pl->packed_ev, up));
 	}
-	pl->stats.h2d_bytes += na + nb + (int64_t)st.total;
+	pl->stats.h2d_bytes += (pl->dev_inputs ? 0 : na + nb) + (int64_t)st.total;
 	pl->stats.raw_bytes = na * (mode_a == PACK_BOTH ? 2 : 1) + nb * (mode_b == PACK_BOTH ? 2 : 1);
 	pl->stats.packed_bytes = (int64_t)total_words * 8;
 	return DFB_OK;
@@ -1215,7 +1232,8 @@ static int finish_create(dfb_plan* pl)
 // stream and a final synchronisation; else uploads on `up_stream` and none (chunks of a pipelined batch).
 static int plan_create_host(dfb_ctx* ctx, bool simple, const dfb_split_params* params, const dfb_seq_table* A,
                             const dfb_seq_table* B, const int32_t* task_a, const int32_t* task_b, const int32_t* task_min_score,
-                            int64_t n_tasks, int32_t a_base, int32_t b_base, int stage_slot, cudaStream_t up_stream, dfb_plan** out)
+                            int64_t n_tasks, int32_t a_base, int32_t b_base, int stage_slot, cudaStream_t up_stream, dfb_plan** out,
+                            bool bytes_on_device = false)
 {
 	*out = nullptr;
 	int rc;
@@ -1234,8 +1252,10 @@ static int plan_create_host(dfb_ctx* ctx, bool simple, const dfb_split_params* p
 	pl->stats.n_tasks = n_tasks;
 	classify_params(pl, params->match, params->mismatch, params->gap, simple || (params->end_gaps == 0 && params->min_split_score >= 1));
 	pl->up = up_stream;
+	pl->dev_inputs = bytes_on_device;
 	Trace tr;
-	if ((rc = upload_raw(pl, A, B))) return fail(rc);
+	const int64_t range[4] = {A->off[0], A->off[A->n], B->off[0], B->off[B->n]};
+	if ((rc = upload_raw(pl, A, B, bytes_on_device ? range : nullptr))) return fail(rc);
 	tr.lap("host build: raw upload");
 
 	// pass 1 (host threads): class and reference-length bin of every task, per-thread bin counts
@@ -1503,7 +1523,7 @@ static const int DFB_BUILD_ON_HOST = 1000;
 static int device_build_enqueue(dfb_ctx* ctx, bool simple, const dfb_split_params* params, const dfb_seq_table* refs,
                                 const dfb_seq_table* reads, const int32_t* task_cluster, const int32_t* task_read,
                                 const int32_t* task_min_score, int64_t n_tasks, int32_t ref_base, int32_t read_base, int stage_slot,
-                                dfb_plan** out)
+                                dfb_plan** out, const int64_t* dev_range = nullptr)
 {
 	static_assert(kNumClasses <= DFB_BUILD_MAX_CLASSES && kRBins == DFB_BUILD_RBINS, "dfb_build.cuh tables");
 	*out = nullptr;
@@ -1517,8 +1537,10 @@ static int device_build_enqueue(dfb_ctx* ctx, bool simple, const dfb_split_param
 	pl->sp = *params;
 	pl->n_tasks = n_tasks;
 	pl->stats.n_tasks = n_tasks;
-	pl->h_read_off = reads->off;
-	pl->h_task_read = task_read;
+	// (dev_range: every input is device memory -- offsets, tasks, bytes --, [off[0], off[n]) of either table given)
+	pl->dev_inputs = dev_range != nullptr;
+	pl->h_read_off = dev_range ? nullptr : reads->off;
+	pl->h_task_read = dev_range ? nullptr : task_read;
 	pl->h_read_base = read_base;
 	classify_params(pl, params->match, params->mismatch, params->gap, simple || (params->end_gaps == 0 && params->min_split_score >= 1));
 	pl->up = ctx->upload_stream;
@@ -1528,7 +1550,7 @@ static int device_build_enqueue(dfb_ctx* ctx, bool simple, const dfb_split_param
 		return code;
 	};
 	Trace tr;
-	if ((rc = upload_raw(pl, refs, reads))) return fail(rc);
+	if ((rc = upload_raw(pl, refs, reads, dev_range))) return fail(rc);
 
 	// arena
 	const int64_t na = refs->n, nb = reads->n;
@@ -1569,13 +1591,14 @@ static int device_build_enqueue(dfb_ctx* ctx, bool simple, const dfb_split_param
 	};
 	cudaError_t e;
 	if ((e = cudaMemcpyAsync(d_stats, h_init, sizeof(BuildStats), cudaMemcpyHostToDevice, up)) != cudaSuccess) return cuda_fail(e, "statistics upload");
-	if ((e = cudaMemcpyAsync(base + o_off_a, refs->off, (size_t)(na + 1) * 8, cudaMemcpyHostToDevice, up)) != cudaSuccess ||
-	    (e = cudaMemcpyAsync(base + o_off_b, reads->off, (size_t)(nb + 1) * 8, cudaMemcpyHostToDevice, up)) != cudaSuccess ||
-	    (e = cudaMemcpyAsync(base + o_tc, task_cluster, (size_t)n_tasks * 4, cudaMemcpyHostToDevice, up)) != cudaSuccess ||
-	    (e = cudaMemcpyAsync(base + o_tr, task_read, (size_t)n_tasks * 4, cudaMemcpyHostToDevice, up)) != cudaSuccess ||
-	    (!simple && (e = cudaMemcpyAsync(base + o_tm, task_min_score, (size_t)n_tasks * 4, cudaMemcpyHostToDevice, up)) != cudaSuccess))
+	const cudaMemcpyKind kind = dev_range ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
+	if ((e = cudaMemcpyAsync(base + o_off_a, refs->off, (size_t)(na + 1) * 8, kind, up)) != cudaSuccess ||
+	    (e = cudaMemcpyAsync(base + o_off_b, reads->off, (size_t)(nb + 1) * 8, kind, up)) != cudaSuccess ||
+	    (e = cudaMemcpyAsync(base + o_tc, task_cluster, (size_t)n_tasks * 4, kind, up)) != cudaSuccess ||
+	    (e = cudaMemcpyAsync(base + o_tr, task_read, (size_t)n_tasks * 4, kind, up)) != cudaSuccess ||
+	    (!simple && (e = cudaMemcpyAsync(base + o_tm, task_min_score, (size_t)n_tasks * 4, kind, up)) != cudaSuccess))
 		return cuda_fail(e, "task upload");
-	const int64_t raw_a = refs->off[refs->n] - refs->off[0];
+	const int64_t raw_a = dev_range ? dev_range[1] - dev_range[0] : refs->off[refs->n] - refs->off[0];
 	// descriptors: windows (one stored copy each), then reads (forward + reversed copy)
 	DescParams da;
 	da.off = (const int64_t*)(base + o_off_a);
@@ -1635,7 +1658,7 @@ static int device_build_enqueue(dfb_ctx* ctx, bool simple, const dfb_split_param
 	pl->pending.blocks_a = blocks_a;
 	pl->pending.blocks_b = blocks_b;
 	pl->pending.raw_a = raw_a;
-	pl->pending.raw_b = reads->off[reads->n] - reads->off[0];
+	pl->pending.raw_b = dev_range ? dev_range[3] - dev_range[2] : reads->off[reads->n] - reads->off[0];
 	pl->pending.d_stats = d_stats;
 	pl->pending.d_words_a_end = d_words_a_end;
 	pl->pending.h_stats = h_stats;
@@ -1750,7 +1773,13 @@ static int device_build_finish(dfb_plan* pl)
 	}
 	else if (n_tasks) split_scatter_kernel<<<task_blocks, DFB_BUILD_BLOCK, 0, up>>>(bp);
 	if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail(e, "pack / scatter kernels");
-	pl->stats.h2d_bytes += raw_a + raw_b + (na + 1 + nb + 1) * 8 + n_tasks * 12 + (int64_t)sizeof(BuildStats);
+	if (pl->dev_inputs)
+	{
+		// (the statistics, both ways, are all that crosses)
+		pl->stats.h2d_bytes += (int64_t)sizeof(BuildStats);
+		pl->stats.d2h_bytes += (int64_t)sizeof(BuildStats);
+	}
+	else pl->stats.h2d_bytes += raw_a + raw_b + (na + 1 + nb + 1) * 8 + n_tasks * 12 + (int64_t)sizeof(BuildStats);
 	pl->stats.raw_bytes = raw_a + (simple ? 1 : 2) * raw_b;
 	pl->stats.packed_bytes = (int64_t)total_words * 8;
 
@@ -2068,29 +2097,19 @@ static int dfb_split_plan_fetch_body(dfb_plan* pl, int32_t* out_best, int64_t* n
 	return split_fetch_impl(pl, out_best, n_rows, n_cols, pl->ctx->pool);
 }
 
-static int split_fetch_impl(dfb_plan* pl, int32_t* out_best, int64_t* n_rows, int64_t* n_cols, HostPool* pool, ResultSink* sink)
+// Step 1 of a split fetch, once the plan's kernels are done (`cs` waits for them): the overflow-list length, the
+// winning tasks per class (h_ctrl) and the row / column totals of the region assembly.  When the probe sweep found more
+// arg-max columns than the overflow list holds, the list is sized exactly and the sweep run again.
+static int fetch_counters(dfb_plan* pl, cudaStream_t cs, int* h_ctrl, unsigned long long* n_ov_out, unsigned long long* asm_totals)
 {
 	dfb_ctx* ctx = pl->ctx;
-	if (!pl->split) return set_err(ctx, DFB_ERR_STATE, "dfb_split_plan_fetch on a simple plan");
-	if (!pl->ran) return set_err(ctx, DFB_ERR_STATE, "dfb_split_plan_fetch before dfb_plan_run");
-	CK(ctx, cudaSetDevice(ctx->device));
-	Trace tr;
-	// result copies run on the copy stream, ordered behind this plan's kernels only (later batches may
-	// already be queued on the compute stream)
-	cudaStream_t cs = ctx->copy_stream;
-	CK(ctx, wait_event(pl->done_ev));
-	CK(ctx, cudaStreamWaitEvent(cs, pl->done_ev, 0));
-
-	// 1. counters: overflow-list length and winning tasks per class
-	int h_ctrl[kNumClasses * 4];
 	unsigned long long n_ov = 0;
-	unsigned long long asm_totals[2] = {0, 0}; // rows, columns assembled on the device
 	for (int attempt = 0;; attempt++)
 	{
 		CK(ctx, cudaMemcpyAsync(&n_ov, pl->d_ev_count, sizeof(n_ov), cudaMemcpyDeviceToHost, cs));
-		CK(ctx, cudaMemcpyAsync(h_ctrl, pl->d_ctrl, sizeof(h_ctrl), cudaMemcpyDeviceToHost, cs));
+		CK(ctx, cudaMemcpyAsync(h_ctrl, pl->d_ctrl, kNumClasses * 4 * sizeof(int), cudaMemcpyDeviceToHost, cs));
 		if (pl->d_asm_sums)
-			CK(ctx, cudaMemcpyAsync(asm_totals, pl->d_asm_sums + 2 * (size_t)pl->asm_blocks, sizeof(asm_totals), cudaMemcpyDeviceToHost, cs));
+			CK(ctx, cudaMemcpyAsync(asm_totals, pl->d_asm_sums + 2 * (size_t)pl->asm_blocks, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, cs));
 		CK(ctx, cudaStreamSynchronize(cs));
 		if (n_ov <= pl->ev_cap) break;
 		if (attempt >= 2) return set_err(ctx, DFB_ERR_STATE, "event buffer overflow persists");
@@ -2127,6 +2146,28 @@ static int split_fetch_impl(dfb_plan* pl, int32_t* out_best, int64_t* n_rows, in
 		if (rc) return rc;
 		CK(ctx, cudaStreamWaitEvent(cs, pl->done_ev, 0));
 	}
+	*n_ov_out = n_ov;
+	return DFB_OK;
+}
+
+static int split_fetch_impl(dfb_plan* pl, int32_t* out_best, int64_t* n_rows, int64_t* n_cols, HostPool* pool, ResultSink* sink)
+{
+	dfb_ctx* ctx = pl->ctx;
+	if (!pl->split) return set_err(ctx, DFB_ERR_STATE, "dfb_split_plan_fetch on a simple plan");
+	if (!pl->ran) return set_err(ctx, DFB_ERR_STATE, "dfb_split_plan_fetch before dfb_plan_run");
+	CK(ctx, cudaSetDevice(ctx->device));
+	Trace tr;
+	// result copies run on the copy stream, ordered behind this plan's kernels only (later batches may
+	// already be queued on the compute stream)
+	cudaStream_t cs = ctx->copy_stream;
+	CK(ctx, wait_event(pl->done_ev));
+	CK(ctx, cudaStreamWaitEvent(cs, pl->done_ev, 0));
+
+	// 1. counters: overflow-list length and winning tasks per class
+	int h_ctrl[kNumClasses * 4];
+	unsigned long long n_ov = 0;
+	unsigned long long asm_totals[2] = {0, 0}; // rows, columns assembled on the device
+	if (int rc = fetch_counters(pl, cs, h_ctrl, &n_ov, asm_totals)) return rc;
 	int64_t n_slots = 0;
 	for (int c = 0; c < kNumClasses; c++)
 		if (pl->cls[c].n_jobs) n_slots += (int64_t)h_ctrl[4 * c + 1] + h_ctrl[4 * c + 3]; // short- and long-window queue slots
@@ -2623,14 +2664,9 @@ static int dfb_simple_align_batch_body(dfb_ctx* ctx, const dfb_simple_params* pa
 	return rc;
 }
 
-// Large batches whose task_read is non-decreasing (the usual case: reads are listed in task order) go through
-// pipeline_run: chunks flow through the GPU back to back while the host builds the next chunk and assembles the previous
-// one.  Results are merged into one task-ordered row list.  A chunk sees views of both tables: its own reads and -- when
-// the batch's clusters do not decrease, the order dosplitalign emits -- its own window pairs, so that every window is
-// uploaded and packed once per batch (plus one shared cluster per chunk boundary) instead of once per chunk.
-static int split_align_pipelined(dfb_ctx* ctx, const dfb_split_params* params, const dfb_seq_table* refs,
-                                 const dfb_seq_table* reads, const int32_t* task_cluster, const int32_t* task_read,
-                                 const int32_t* task_min_score, int64_t n_tasks, int32_t* out_best, bool clusters_monotone)
+// Chunk boundaries of a pipelined split batch (both one-call forms cut a batch at the same tasks: the column pool
+// holds each chunk's region-assembled columns in front of its overflow-list columns, so equal results need equal cuts)
+static std::vector<int64_t> split_chunk_starts(int64_t n_tasks)
 {
 	const int K = (int)std::max<int64_t>(2, std::min<int64_t>(std::min<int64_t>(dfb_ctx::kStageSlots, n_tasks), n_tasks / 330000));
 	// chunk boundaries: short chunks in front put the GPU to work early, chunks that taper off at the end keep the part
@@ -2660,7 +2696,20 @@ static int split_align_pipelined(dfb_ctx* ctx, const dfb_split_params* params, c
 		weight[0] = 0.4;
 		weight[(size_t)K - 1] = 0.45;
 	}
-	const std::vector<int64_t> t0 = chunk_starts(n_tasks, weight);
+	return chunk_starts(n_tasks, weight);
+}
+
+// Large batches whose task_read is non-decreasing (the usual case: reads are listed in task order) go through
+// pipeline_run: chunks flow through the GPU back to back while the host builds the next chunk and assembles the previous
+// one.  Results are merged into one task-ordered row list.  A chunk sees views of both tables: its own reads and -- when
+// the batch's clusters do not decrease, the order dosplitalign emits -- its own window pairs, so that every window is
+// uploaded and packed once per batch (plus one shared cluster per chunk boundary) instead of once per chunk.
+static int split_align_pipelined(dfb_ctx* ctx, const dfb_split_params* params, const dfb_seq_table* refs,
+                                 const dfb_seq_table* reads, const int32_t* task_cluster, const int32_t* task_read,
+                                 const int32_t* task_min_score, int64_t n_tasks, int32_t* out_best, bool clusters_monotone)
+{
+	const std::vector<int64_t> t0 = split_chunk_starts(n_tasks);
+	const int K = (int)t0.size() - 1;
 	std::vector<dfb_plan*> plans((size_t)K, nullptr);
 	{
 		// the pinned buffer the chunks' results land in: sized for the largest chunk now (growing it chunk by chunk frees and
@@ -2816,6 +2865,8 @@ extern "C" int dfb_split_result_size(const dfb_ctx* ctx, int64_t* n_rows, int64_
 {
 	if (!ctx) return DFB_ERR_ARG;
 	if (!ctx->last_split) return set_err(ctx, DFB_ERR_STATE, "no split result on this context");
+	if (ctx->last_split->device_result)
+		return set_err(ctx, DFB_ERR_STATE, "the last split result is in device memory: use dfb_split_result_copy_device");
 	if (n_rows) *n_rows = (int64_t)ctx->last_split->rows.size();
 	if (n_cols) *n_cols = (int64_t)ctx->last_split->cols.size();
 	return DFB_OK;
@@ -2825,6 +2876,8 @@ extern "C" int dfb_split_result_copy(const dfb_ctx* ctx, dfb_split_row* rows, in
 {
 	if (!ctx) return DFB_ERR_ARG;
 	if (!ctx->last_split) return set_err(ctx, DFB_ERR_STATE, "no split result on this context");
+	if (ctx->last_split->device_result)
+		return set_err(ctx, DFB_ERR_STATE, "the last split result is in device memory: use dfb_split_result_copy_device");
 	return dfb_split_plan_copy(ctx->last_split, rows, cols);
 }
 
@@ -2833,6 +2886,8 @@ extern "C" int dfb_split_result_view(const dfb_ctx* ctx, const dfb_split_row** r
 {
 	if (!ctx) return DFB_ERR_ARG;
 	if (!ctx->last_split) return set_err(ctx, DFB_ERR_STATE, "no split result on this context");
+	if (ctx->last_split->device_result)
+		return set_err(ctx, DFB_ERR_STATE, "the last split result is in device memory: use dfb_split_result_copy_device");
 	return dfb_split_plan_view(ctx->last_split, rows, n_rows, cols, n_cols);
 }
 
@@ -2875,6 +2930,541 @@ extern "C" int dfb_split_align_batch(dfb_ctx* ctx, const dfb_split_params* param
                                      const int32_t* task_min_score, int64_t n_tasks, int32_t* out_best)
 {
 	return guarded(ctx, [&] { return dfb_split_align_batch_body(ctx, params, refs, reads, task_cluster, task_read, task_min_score, n_tasks, out_best); });
+}
+
+// ---- device-resident one-call forms ------------------------------------------------------------------------------
+// The batch, the outputs and the results stay in device memory: tables and tasks are read where they are, checked by
+// kernels (dfb_build.cuh), copied device to device into the plan's raw buffer and built into job lists on the device;
+// the overflow list is assembled by the kernels of dfb_assemble.cuh.  What crosses PCIe is counters: the check record,
+// the build statistics and the overflow / assembly totals of every chunk, the batch's row and column totals.  Chunks that
+// hold tasks only the s32 kernels take are built by the host builder from a host copy of their offsets and task arrays
+// (never the bytes).
+
+// Every array of a device-resident call must be memory of the context's device: host memory (pinned or not), managed
+// memory and another GPU's memory are refused before anything is queued.
+static bool is_ctx_device_memory(const dfb_ctx* ctx, const void* p)
+{
+	if (!p) return true; // (null pointers are judged by the argument checks of the host form)
+	cudaPointerAttributes a;
+	if (cudaPointerGetAttributes(&a, p) != cudaSuccess)
+	{
+		cudaGetLastError();
+		return false;
+	}
+	return a.type == cudaMemoryTypeDevice && a.device == ctx->device;
+}
+
+// The argument checks of the host form (check_simple_args / check_split_args, and the builders' task index check) with
+// the same statuses and messages, run on the device; plus off[n] <= n_bytes.  *chk receives the record.
+static int check_device_args(dfb_ctx* ctx, bool simple, const void* params, const dfb_device_seq_table* A, const dfb_device_seq_table* B,
+                             const int32_t* ta, const int32_t* tb, const int32_t* tm, int64_t n_tasks, const void* out, DeviceCheck* chk)
+{
+	const char* names[2] = {"refs", simple ? "seqs" : "reads"};
+	const dfb_device_seq_table* tabs[2] = {A, B};
+	if (!params || n_tasks < 0 || (n_tasks > 0 && (!ta || !tb || (!simple && !tm))))
+		return set_err(ctx, DFB_ERR_ARG, "%s: null argument", simple ? "dfb_simple_plan_create" : "dfb_split_plan_create");
+	for (int k = 0; k < 2; k++)
+		if (!tabs[k] || !tabs[k]->off || tabs[k]->n < 0 || tabs[k]->n_bytes < 0) return set_err(ctx, DFB_ERR_ARG, "%s: null table", names[k]);
+	if (n_tasks > 0 && !out) return set_err(ctx, DFB_ERR_ARG, "null output");
+	const void* ptrs[8] = {A->bytes, A->off, B->bytes, B->off, ta, tb, simple ? nullptr : tm, out};
+	const char* what[8] = {"refs->bytes", "refs->off", simple ? "seqs->bytes" : "reads->bytes", simple ? "seqs->off" : "reads->off",
+	                       simple ? "task_ref" : "task_cluster", simple ? "task_seq" : "task_read", "task_min_score",
+	                       simple ? "out_score" : "out_best"};
+	for (int k = 0; k < 8; k++)
+		if (!is_ctx_device_memory(ctx, ptrs[k]))
+			return set_err(ctx, DFB_ERR_ARG, "%s is not device memory of device %d", what[k], ctx->device);
+	DeviceCheck* d_chk = nullptr;
+	CK(ctx, dalloc(ctx, (void**)&d_chk, sizeof(DeviceCheck)));
+	CK(ctx, ctx->h_out.ensure(sizeof(DeviceCheck)));
+	DeviceCheck* h_chk = (DeviceCheck*)ctx->h_out.p;
+	const int max_grid = ctx->prop.multiProcessorCount * 8;
+	auto grid = [&](int64_t n) { return (unsigned)std::max<int64_t>(1, std::min<int64_t>((n + DFB_BUILD_BLOCK - 1) / DFB_BUILD_BLOCK, max_grid)); };
+	device_check_init_kernel<<<1, 1, 0, ctx->stream>>>(d_chk);
+	for (int k = 0; k < 2; k++) table_check_kernel<<<grid(tabs[k]->n), DFB_BUILD_BLOCK, 0, ctx->stream>>>(tabs[k]->off, tabs[k]->n, &d_chk->tab[k]);
+	if (n_tasks)
+		task_check_kernel<<<grid(n_tasks), DFB_BUILD_BLOCK, 0, ctx->stream>>>(ta, tb, n_tasks, simple ? A->n : A->n / 2, B->n, d_chk);
+	CK(ctx, cudaGetLastError());
+	CK(ctx, cudaMemcpyAsync(h_chk, d_chk, sizeof(DeviceCheck), cudaMemcpyDeviceToHost, ctx->stream));
+	cudaFreeAsync(d_chk, ctx->stream);
+	CK(ctx, cudaStreamSynchronize(ctx->stream));
+	*chk = *h_chk;
+	for (int k = 0; k < 2; k++)
+	{
+		const TableCheck& c = chk->tab[k];
+		if (tabs[k]->n > 0 && !tabs[k]->bytes && c.off_n > 0) return set_err(ctx, DFB_ERR_ARG, "%s: null table", names[k]);
+		if (c.off0 != 0) return set_err(ctx, DFB_ERR_ARG, "%s: off[0] must be 0", names[k]);
+		if (c.first_bad != ~0ull)
+		{
+			if (c.first_bad & 1) return set_err(ctx, DFB_ERR_ARG, "%s: sequence %lld too long", names[k], (long long)(c.first_bad >> 1));
+			return set_err(ctx, DFB_ERR_ARG, "%s: offsets decrease at %lld", names[k], (long long)(c.first_bad >> 1));
+		}
+		if (c.off_n > tabs[k]->n_bytes)
+			return set_err(ctx, DFB_ERR_ARG, "%s: off[n] = %lld exceeds n_bytes = %lld", names[k], (long long)c.off_n, (long long)tabs[k]->n_bytes);
+	}
+	if (!simple && (A->n & 1)) return set_err(ctx, DFB_ERR_ARG, "refs must hold two windows per cluster (n is odd)");
+	if (n_tasks > 0x7fffff00LL) return set_err(ctx, DFB_ERR_ARG, "too many tasks in one batch");
+	if (chk->bad_task != ~0ull) return set_err(ctx, DFB_ERR_ARG, "task %lld: table index out of range", (long long)chk->bad_task);
+	return DFB_OK;
+}
+
+// Work on the upload and copy streams is ordered behind what the caller queued on the context's stream before the call
+static int order_side_streams(dfb_ctx* ctx)
+{
+	cudaEvent_t ev;
+	CK(ctx, cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
+	cudaError_t e = cudaEventRecord(ev, ctx->stream);
+	if (e == cudaSuccess) e = cudaStreamWaitEvent(ctx->upload_stream, ev, 0);
+	if (e == cudaSuccess) e = cudaStreamWaitEvent(ctx->upload_stream2, ev, 0);
+	if (e == cudaSuccess) e = cudaStreamWaitEvent(ctx->copy_stream, ev, 0);
+	cudaEventDestroy(ev);
+	if (e != cudaSuccess) return set_err(ctx, DFB_ERR_CUDA, "stream ordering failed: %s", cudaGetErrorString(e));
+	return DFB_OK;
+}
+
+static bool any_fast_class(bool simple, const dfb_split_params* params)
+{
+	dfb_plan probe;
+	classify_params(&probe, params->match, params->mismatch, params->gap, simple || (params->end_gaps == 0 && params->min_split_score >= 1));
+	for (int c = 0; c < kNumClasses; c++)
+		if (probe.fast_ok[c]) return true;
+	return false;
+}
+
+// A chunk with tasks only the s32 kernels take: its offsets and task arrays come to the host and the host builder makes
+// its job lists; the raw bytes go device to device.  *d2h counts what crossed.
+static int plan_create_from_device(dfb_ctx* ctx, bool simple, const dfb_split_params* params, const dfb_seq_table* A, const dfb_seq_table* B,
+                                   const int32_t* ta, const int32_t* tb, const int32_t* tm, int64_t n_tasks, int32_t a_base, int32_t b_base,
+                                   int stage_slot, cudaStream_t up_stream, int64_t* d2h, dfb_plan** out)
+{
+	std::vector<int64_t> ha((size_t)A->n + 1), hb((size_t)B->n + 1);
+	std::vector<int32_t> hta((size_t)n_tasks), htb((size_t)n_tasks), htm(simple ? 0 : (size_t)n_tasks);
+	cudaStream_t cs = ctx->copy_stream;
+	CK(ctx, cudaMemcpyAsync(ha.data(), A->off, ha.size() * 8, cudaMemcpyDeviceToHost, cs));
+	CK(ctx, cudaMemcpyAsync(hb.data(), B->off, hb.size() * 8, cudaMemcpyDeviceToHost, cs));
+	if (n_tasks)
+	{
+		CK(ctx, cudaMemcpyAsync(hta.data(), ta, (size_t)n_tasks * 4, cudaMemcpyDeviceToHost, cs));
+		CK(ctx, cudaMemcpyAsync(htb.data(), tb, (size_t)n_tasks * 4, cudaMemcpyDeviceToHost, cs));
+		if (!simple) CK(ctx, cudaMemcpyAsync(htm.data(), tm, (size_t)n_tasks * 4, cudaMemcpyDeviceToHost, cs));
+	}
+	CK(ctx, cudaStreamSynchronize(cs));
+	*d2h += (int64_t)(ha.size() + hb.size()) * 8 + n_tasks * (simple ? 8 : 12);
+	const dfb_seq_table a{A->bytes, ha.data(), A->n}, b{B->bytes, hb.data(), B->n};
+	return plan_create_host(ctx, simple, params, &a, &b, hta.data(), htb.data(), simple ? nullptr : htm.data(), n_tasks, a_base, b_base,
+	                        stage_slot, up_stream, out, true);
+}
+
+static int dfb_simple_align_device_body(dfb_ctx* ctx, const dfb_simple_params* params, const dfb_device_seq_table* refs,
+                                        const dfb_device_seq_table* seqs, const int32_t* task_ref, const int32_t* task_seq, int64_t n_tasks,
+                                        int32_t* out_score)
+{
+	if (!ctx) return DFB_ERR_ARG;
+	CK(ctx, cudaSetDevice(ctx->device));
+	DeviceCheck chk;
+	int rc = check_device_args(ctx, true, params, refs, seqs, task_ref, task_seq, nullptr, n_tasks, out_score, &chk);
+	if (rc || n_tasks == 0) return rc;
+	if ((rc = order_side_streams(ctx))) return rc;
+	const dfb_split_params sp{params->match, params->mismatch, params->gap, 0, 0};
+	const dfb_seq_table a{refs->bytes, refs->off, refs->n}, b{seqs->bytes, seqs->off, seqs->n};
+	const int64_t range[4] = {0, chk.tab[0].off_n, 0, chk.tab[1].off_n};
+	// one chunk: a simple batch keeps no first-sweep state
+	dfb_plan* pl = nullptr;
+	rc = DFB_BUILD_ON_HOST;
+	if (any_fast_class(true, &sp))
+	{
+		rc = device_build_enqueue(ctx, true, &sp, &a, &b, task_ref, task_seq, nullptr, n_tasks, 0, 0, 0, &pl, range);
+		if (!rc) rc = device_build_kernels(pl);
+		if (!rc) rc = device_build_finish(pl);
+		if (rc && pl)
+		{
+			dfb_plan_destroy(pl);
+			pl = nullptr;
+		}
+	}
+	int64_t d2h = 0;
+	if (rc == DFB_BUILD_ON_HOST) rc = plan_create_from_device(ctx, true, &sp, &a, &b, task_ref, task_seq, nullptr, n_tasks, 0, 0, 0, nullptr, &d2h, &pl);
+	if (!rc) rc = plan_run_impl(pl, nullptr);
+	if (!rc)
+	{
+		cudaError_t e = cudaMemcpyAsync(out_score, pl->d_out, (size_t)n_tasks * sizeof(int32_t), cudaMemcpyDeviceToDevice, ctx->stream);
+		if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+		if (e != cudaSuccess) rc = set_err(ctx, DFB_ERR_CUDA, "simple device batch failed: %s", cudaGetErrorString(e));
+	}
+	if (!rc) rc = bounds_check_status(ctx);
+	if (pl) dfb_plan_destroy(pl);
+	return rc;
+}
+
+static int bit_width(unsigned long long v)
+{
+	int b = 0;
+	while (v) { b++; v >>= 1; }
+	return b;
+}
+
+// exclusive scan of v[0, n) in place on the context's stream; the total goes to *total (device)
+static int scan_u64(dfb_ctx* ctx, unsigned long long* v, long long n, unsigned long long* sums, unsigned long long* total)
+{
+	const long long blocks = std::max<long long>(1, (n + DFB_BUILD_BLOCK * DFB_BUILD_ITEMS - 1) / (DFB_BUILD_BLOCK * DFB_BUILD_ITEMS));
+	u64_scan_sums_kernel<<<(unsigned)blocks, DFB_BUILD_BLOCK, 0, ctx->stream>>>(v, n, sums);
+	desc_scan_kernel<<<1, DFB_BUILD_BLOCK, 0, ctx->stream>>>(sums, blocks, nullptr, total);
+	u64_scan_write_kernel<<<(unsigned)blocks, DFB_BUILD_BLOCK, 0, ctx->stream>>>(v, n, sums);
+	CK(ctx, cudaGetLastError());
+	return DFB_OK;
+}
+
+// The rows of chunk `pl` into the batch's arrays (dfb_assemble.cuh, "overflow list assembled on the device"): n_ov overflow
+// events, g_rows / g_cols rows and columns of the region assembly; d_base holds the batch's totals before the chunk and
+// is advanced past it.
+static int assemble_chunk_device(dfb_plan* pl, unsigned long long n_ov, long long g_rows, long long g_cols, int32_t task_shift,
+                                 const int64_t* read_off, const int32_t* task_read, OvKey key, int passes, unsigned long long* d_base,
+                                 dfb_split_row* out_rows, int32_t* out_cols)
+{
+	dfb_ctx* ctx = pl->ctx;
+	cudaStream_t s = ctx->stream;
+	const long long n = (long long)n_ov, n_x_bound = n / 2 + 1;
+	unsigned long long* scal = nullptr;
+	dfb_split_row* x_rows = nullptr;
+	Event* tmp = nullptr;
+	unsigned long long *hist = nullptr, *head = nullptr, *sums = nullptr, *g_r = nullptr, *g_c = nullptr;
+	long long* g_first = nullptr;
+	int32_t *g_match = nullptr, *g_mb = nullptr;
+	int rc = DFB_OK;
+	auto cleanup = [&]() {
+		dfree(ctx, scal);
+		dfree(ctx, x_rows);
+		dfree(ctx, tmp);
+		dfree(ctx, hist);
+		dfree(ctx, head);
+		dfree(ctx, sums);
+		dfree(ctx, g_r);
+		dfree(ctx, g_c);
+		dfree(ctx, g_first);
+		dfree(ctx, g_match);
+		dfree(ctx, g_mb);
+	};
+	if (n)
+	{
+		const long long nb = (n + DFB_OV_BLOCK - 1) / DFB_OV_BLOCK;
+		const long long scan_len = std::max<long long>(256 * nb, n);
+		cudaError_t e = cudaSuccess;
+		auto take = [&](void** p, size_t bytes) {
+			if (e == cudaSuccess) e = dalloc(ctx, p, bytes);
+		};
+		take((void**)&scal, 4 * sizeof(unsigned long long));
+		take((void**)&x_rows, (size_t)n_x_bound * sizeof(dfb_split_row));
+		take((void**)&tmp, (size_t)n * sizeof(Event));
+		take((void**)&hist, (size_t)256 * nb * sizeof(unsigned long long));
+		take((void**)&head, (size_t)n * sizeof(unsigned long long));
+		take((void**)&sums, (size_t)(scan_len / (DFB_BUILD_BLOCK * DFB_BUILD_ITEMS) + 2) * sizeof(unsigned long long));
+		take((void**)&g_r, (size_t)n * sizeof(unsigned long long));
+		take((void**)&g_c, (size_t)n * sizeof(unsigned long long));
+		take((void**)&g_first, (size_t)(n + 1) * sizeof(long long));
+		take((void**)&g_match, (size_t)n * sizeof(int32_t));
+		take((void**)&g_mb, (size_t)n * sizeof(int32_t));
+		if (e != cudaSuccess)
+		{
+			cleanup();
+			return set_err(ctx, DFB_ERR_NOMEM, "overflow assembly buffers for %lld events: %s", n, cudaGetErrorString(e));
+		}
+		// 1. radix sort: (matrix, row, column) passes, then task passes
+		Event* src = pl->d_events;
+		Event* dst = tmp;
+		for (int pass = 0; pass < passes && !rc; pass++)
+		{
+			ov_hist_kernel<<<(unsigned)nb, DFB_OV_BLOCK, 0, s>>>(src, n, pass, key, hist, nb);
+			rc = scan_u64(ctx, hist, 256 * nb, sums, scal + 3);
+			ov_scatter_kernel<<<(unsigned)nb, DFB_OV_BLOCK, 0, s>>>(src, dst, n, pass, key, hist, nb);
+			std::swap(src, dst);
+		}
+		OvAsmParams p;
+		p.ev = src;
+		p.n = n;
+		p.head = head;
+		p.scal = scal;
+		p.g_first = g_first;
+		p.g_match = g_match;
+		p.g_matched_by = g_mb;
+		p.g_rows = g_r;
+		p.g_cols = g_c;
+		p.read_off = read_off;
+		p.task_read = task_read;
+		p.task_base = task_shift;
+		p.x_rows = x_rows;
+		p.asm_cols = g_cols;
+		p.cols = out_cols;
+		p.base = d_base;
+		// 2.-4. groups, pairs, rows, columns
+		if (!rc)
+		{
+			ov_head_kernel<<<(unsigned)nb, DFB_OV_BLOCK, 0, s>>>(p);
+			rc = scan_u64(ctx, head, n, sums, scal + 0);
+		}
+		if (!rc)
+		{
+			ov_group_kernel<<<(unsigned)nb, DFB_OV_BLOCK, 0, s>>>(p);
+			cudaMemsetAsync(g_mb, 0xff, (size_t)n * sizeof(int32_t), s);
+			ov_match_kernel<<<(unsigned)nb, DFB_OV_BLOCK, 0, s>>>(p);
+			rc = scan_u64(ctx, g_r, n, sums, scal + 1);
+		}
+		if (!rc) rc = scan_u64(ctx, g_c, n, sums, scal + 2);
+		if (!rc)
+		{
+			ov_rows_kernel<<<(unsigned)nb, DFB_OV_BLOCK, 0, s>>>(p);
+			ov_cols_kernel<<<(unsigned)nb, DFB_OV_BLOCK, 0, s>>>(p);
+		}
+	}
+	// 5. merge by task into the batch's arrays, columns of the region part first
+	const long long items = g_rows + (n ? n_x_bound : 0) + g_cols;
+	if (!rc && items)
+		ov_place_kernel<<<(unsigned)((items + DFB_OV_BLOCK - 1) / DFB_OV_BLOCK), DFB_OV_BLOCK, 0, s>>>(
+		    pl->d_asm_rows, g_rows, pl->d_asm_cols, g_cols, x_rows, n ? n_x_bound : 0, n ? scal : nullptr, task_shift, d_base, out_rows, out_cols);
+	if (!rc) ov_advance_kernel<<<1, 1, 0, s>>>(d_base, g_rows, g_cols, n ? scal : nullptr);
+	if (!rc)
+	{
+		cudaError_t e = cudaGetLastError();
+		if (e != cudaSuccess) rc = set_err(ctx, DFB_ERR_CUDA, "overflow assembly kernels: %s", cudaGetErrorString(e));
+	}
+	cleanup();
+	return rc;
+}
+
+// grows a device array of the batch's results (stream-ordered), keeping its first `cap` entries
+template <class T>
+static int grow_device(dfb_ctx* ctx, T*& p, int64_t& cap, int64_t need)
+{
+	if (need <= cap) return DFB_OK;
+	const int64_t ncap = need + need / 2 + 1024;
+	T* q = nullptr;
+	CK(ctx, dalloc(ctx, (void**)&q, (size_t)ncap * sizeof(T)));
+	if (p) CK(ctx, cudaMemcpyAsync(q, p, (size_t)cap * sizeof(T), cudaMemcpyDeviceToDevice, ctx->stream));
+	dfree(ctx, p);
+	p = q;
+	cap = ncap;
+	return DFB_OK;
+}
+
+static int dfb_split_align_device_body(dfb_ctx* ctx, const dfb_split_params* params, const dfb_device_seq_table* refs,
+                                       const dfb_device_seq_table* reads, const int32_t* task_cluster, const int32_t* task_read,
+                                       const int32_t* task_min_score, int64_t n_tasks, int32_t* out_best, int64_t* n_rows, int64_t* n_cols)
+{
+	if (!ctx) return DFB_ERR_ARG;
+	if (ctx->last_split)
+	{
+		dfb_plan_destroy(ctx->last_split);
+		ctx->last_split = nullptr;
+	}
+	CK(ctx, cudaSetDevice(ctx->device));
+	DeviceCheck chk;
+	int rc = check_device_args(ctx, false, params, refs, reads, task_cluster, task_read, task_min_score, n_tasks, out_best, &chk);
+	if (rc) return rc;
+	if ((rc = order_side_streams(ctx))) return rc;
+	dfb_plan* holder = new (std::nothrow) dfb_plan();
+	if (!holder) return set_err(ctx, DFB_ERR_NOMEM, "out of host memory");
+	holder->ctx = ctx;
+	holder->split = true;
+	holder->n_tasks = n_tasks;
+	holder->stats.n_tasks = n_tasks;
+	holder->device_result = true;
+	holder->stats.d2h_bytes = (int64_t)sizeof(DeviceCheck);
+	auto fail = [&](int code) {
+		dfb_plan_destroy(holder);
+		return code;
+	};
+	// the host form's chunks (split_chunk_starts), so that the column pool comes out the same
+	const bool chunked = n_tasks >= pipeline_min_tasks() && !chk.b_decreases;
+	const std::vector<int64_t> t0 = chunked ? split_chunk_starts(n_tasks) : std::vector<int64_t>{0, n_tasks};
+	const int K = n_tasks ? (int)t0.size() - 1 : 0;
+	static_assert(dfb_ctx::kStageSlots <= DFB_MAX_CHUNKS, "ChunkStarts too small");
+	// chunk views: a_lo, a_hi, b_lo, b_hi and their byte offsets
+	std::vector<long long> bnd((size_t)std::max(K, 1) * 8, 0);
+	if (chunked)
+	{
+		ChunkStarts cs;
+		for (int k = 0; k <= K; k++) cs.t[k] = t0[(size_t)k];
+		long long* d_bnd = nullptr;
+		if (cudaError_t e = dalloc(ctx, (void**)&d_bnd, bnd.size() * sizeof(long long)))
+			return fail(set_err(ctx, DFB_ERR_NOMEM, "chunk bounds: %s", cudaGetErrorString(e)));
+		chunk_bounds_kernel<<<1, 32, 0, ctx->stream>>>(refs->off, refs->n / 2, 2, reads->off, task_cluster, task_read, cs, K,
+		                                               chk.a_decreases ? 0 : 1, d_bnd);
+		cudaError_t e = cudaMemcpyAsync(ctx->h_out.p, d_bnd, bnd.size() * sizeof(long long), cudaMemcpyDeviceToHost, ctx->stream);
+		if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+		dfree(ctx, d_bnd);
+		if (e != cudaSuccess) return fail(set_err(ctx, DFB_ERR_CUDA, "chunk bounds: %s", cudaGetErrorString(e)));
+		memcpy(bnd.data(), ctx->h_out.p, bnd.size() * sizeof(long long));
+		holder->stats.d2h_bytes += (int64_t)(bnd.size() * sizeof(long long));
+	}
+	else if (K)
+	{
+		const long long one[8] = {0, refs->n / 2, 0, reads->n, 0, chk.tab[0].off_n, 0, chk.tab[1].off_n};
+		memcpy(bnd.data(), one, sizeof(one));
+	}
+	struct View
+	{
+		dfb_seq_table a, b;
+		int64_t range[4];
+	};
+	std::vector<View> views((size_t)K);
+	for (int k = 0; k < K; k++)
+	{
+		const long long* o = bnd.data() + 8 * k;
+		View& v = views[(size_t)k];
+		v.a = dfb_seq_table{refs->bytes, refs->off + 2 * o[0], 2 * (o[1] - o[0])};
+		v.b = dfb_seq_table{reads->bytes, reads->off + o[2], o[3] - o[2]};
+		v.range[0] = o[4];
+		v.range[1] = o[5];
+		v.range[2] = o[6];
+		v.range[3] = o[7];
+	}
+	// sort key widths of the overflow events: rows <= longest read, columns <= longest window
+	OvKey key;
+	key.rb = bit_width(chk.tab[1].max_len + 1);
+	key.cb = bit_width(chk.tab[0].max_len + 1);
+	key.sub_passes = (1 + key.rb + key.cb + 7) / 8;
+	const bool device_build = any_fast_class(false, params);
+	std::vector<dfb_plan*> staged((size_t)K, nullptr), plans((size_t)K, nullptr);
+	auto enqueue = [&](int k) -> int {
+		const View& v = views[(size_t)k];
+		const int64_t a = t0[(size_t)k];
+		return device_build_enqueue(ctx, false, params, &v.a, &v.b, task_cluster + a, task_read + a, task_min_score + a, t0[(size_t)k + 1] - a,
+		                            (int32_t)bnd[8 * (size_t)k], (int32_t)bnd[8 * (size_t)k + 2], k, &staged[(size_t)k], v.range);
+	};
+	unsigned long long* d_base = nullptr; // the batch's row and column totals so far
+	int64_t rows_cap = 0, cols_cap = 0, rows_bound = 0, cols_bound = 0;
+	if (cudaError_t e = dalloc(ctx, (void**)&d_base, 2 * sizeof(unsigned long long))) return fail(set_err(ctx, DFB_ERR_NOMEM, "%s", cudaGetErrorString(e)));
+	if (cudaError_t e = cudaMemsetAsync(d_base, 0, 2 * sizeof(unsigned long long), ctx->stream)) rc = set_err(ctx, DFB_ERR_CUDA, "%s", cudaGetErrorString(e));
+	auto collect = [&](int k) -> int {
+		dfb_plan* pl = plans[(size_t)k];
+		cudaStream_t cs = ctx->copy_stream;
+		CK(ctx, wait_event(pl->done_ev));
+		CK(ctx, cudaStreamWaitEvent(cs, pl->done_ev, 0));
+		int h_ctrl[kNumClasses * 4];
+		unsigned long long n_ov = 0, asm_totals[2] = {0, 0};
+		if (int frc = fetch_counters(pl, cs, h_ctrl, &n_ov, asm_totals)) return frc;
+		if (int brc = bounds_check_status(ctx)) return brc;
+		holder->stats.d2h_bytes += (int64_t)(sizeof(n_ov) + sizeof(h_ctrl) + (pl->d_asm_sums ? sizeof(asm_totals) : 0));
+		for (int c = 0; c < kNumClasses; c++)
+			if (pl->cls[c].n_jobs) holder->stats.probe_jobs += (int64_t)h_ctrl[4 * c + 1] + h_ctrl[4 * c + 3];
+		const int64_t a = t0[(size_t)k], nk = t0[(size_t)k + 1] - a;
+		CK(ctx, cudaMemcpyAsync(out_best + a, pl->d_out, (size_t)nk * sizeof(int32_t), cudaMemcpyDeviceToDevice, ctx->stream));
+		rows_bound += (int64_t)asm_totals[0] + (int64_t)(n_ov / 2 + 1);
+		cols_bound += (int64_t)asm_totals[1] + (int64_t)n_ov;
+		int grc = grow_device(ctx, holder->d_res_rows, rows_cap, rows_bound);
+		if (!grc) grc = grow_device(ctx, holder->d_res_cols, cols_cap, cols_bound);
+		if (grc) return grc;
+		const int64_t task_bits = bit_width((unsigned long long)std::max<int64_t>(nk - 1, 0));
+		const int passes = key.sub_passes + (int)((task_bits + 7) / 8);
+		int arc = assemble_chunk_device(pl, n_ov, (long long)asm_totals[0], (long long)asm_totals[1], (int32_t)a, reads->off, task_read, key,
+		                                passes, d_base, holder->d_res_rows, holder->d_res_cols);
+		holder->stats.cells += pl->stats.cells;
+		holder->stats.fast_jobs += pl->stats.fast_jobs;
+		holder->stats.generic_jobs += pl->stats.generic_jobs;
+		holder->stats.kernel_launches += pl->stats.kernel_launches;
+		holder->stats.h2d_bytes += pl->stats.h2d_bytes;
+		holder->stats.d2h_bytes += pl->stats.d2h_bytes;
+		holder->stats.raw_bytes += pl->stats.raw_bytes;
+		holder->stats.packed_bytes += pl->stats.packed_bytes;
+		release_device(pl);
+		return arc;
+	};
+	Trace tr;
+	if (!rc && device_build && K)
+	{
+		rc = enqueue(0);
+		if (!rc) rc = device_build_kernels(staged[0]);
+	}
+	int64_t host_d2h = 0;
+	for (int k = 0; k < K && !rc; k++)
+	{
+		if (device_build && k + 1 < K && (rc = enqueue(k + 1))) break;
+		dfb_plan* pk = staged[(size_t)k];
+		staged[(size_t)k] = nullptr;
+		rc = DFB_BUILD_ON_HOST;
+		if (pk && (rc = device_build_finish(pk)))
+		{
+			dfb_plan_destroy(pk);
+			pk = nullptr;
+		}
+		if (rc == DFB_BUILD_ON_HOST)
+		{
+			const View& v = views[(size_t)k];
+			const int64_t a = t0[(size_t)k];
+			rc = plan_create_from_device(ctx, false, params, &v.a, &v.b, task_cluster + a, task_read + a, task_min_score + a, t0[(size_t)k + 1] - a,
+			                             (int32_t)bnd[8 * (size_t)k], (int32_t)bnd[8 * (size_t)k + 2], k, ctx->upload_stream, &host_d2h, &pk);
+		}
+		if (rc) break;
+		plans[(size_t)k] = pk;
+		// the next chunk's build kernels ride behind this chunk's first sweep; the previous chunk is assembled behind this one
+		dfb_plan* next = (k + 1 < K) ? staged[(size_t)k + 1] : nullptr;
+		const std::function<int()> hook = [&]() -> int { return next ? device_build_kernels(next) : DFB_OK; };
+		rc = plan_run_impl(pk, &hook);
+		if (!rc && k > 0) rc = collect(k - 1);
+	}
+	if (!rc && K) rc = collect(K - 1);
+	tr.lap("split device: chunks queued");
+	for (dfb_plan* sp : staged)
+		if (sp)
+		{
+			cudaStreamSynchronize(sp->up);
+			dfb_plan_destroy(sp);
+		}
+	unsigned long long totals[2] = {0, 0};
+	if (!rc)
+	{
+		cudaError_t e = cudaMemcpyAsync(ctx->h_out.p, d_base, sizeof(totals), cudaMemcpyDeviceToHost, ctx->stream);
+		if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+		if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->copy_stream);
+		if (e != cudaSuccess) rc = set_err(ctx, DFB_ERR_CUDA, "split device batch failed: %s", cudaGetErrorString(e));
+		else memcpy(totals, ctx->h_out.p, sizeof(totals));
+		holder->stats.d2h_bytes += (int64_t)sizeof(totals) + host_d2h;
+	}
+	if (!rc) rc = bounds_check_status(ctx);
+	for (dfb_plan* pk : plans)
+		if (pk) dfb_plan_destroy(pk);
+	dfree(ctx, d_base);
+	tr.lap("split device: done");
+	if (rc) return fail(rc);
+	holder->d_res_n_rows = (int64_t)totals[0];
+	holder->d_res_n_cols = (int64_t)totals[1];
+	holder->stats.events = (int64_t)totals[1];
+	holder->ran = holder->fetched = true;
+	if (n_rows) *n_rows = holder->d_res_n_rows;
+	if (n_cols) *n_cols = holder->d_res_n_cols;
+	ctx->last_split = holder;
+	return DFB_OK;
+}
+
+extern "C" int dfb_split_result_copy_device(dfb_ctx* ctx, dfb_split_row* rows, int32_t* cols)
+{
+	if (!ctx) return DFB_ERR_ARG;
+	const dfb_plan* h = ctx->last_split;
+	if (!h || !h->device_result) return set_err(ctx, DFB_ERR_STATE, "no device-resident split result on this context");
+	if ((h->d_res_n_rows && !rows) || (h->d_res_n_cols && !cols)) return set_err(ctx, DFB_ERR_ARG, "dfb_split_result_copy_device: null argument");
+	CK(ctx, cudaSetDevice(ctx->device));
+	if (!is_ctx_device_memory(ctx, rows)) return set_err(ctx, DFB_ERR_ARG, "rows is not device memory of device %d", ctx->device);
+	if (!is_ctx_device_memory(ctx, cols)) return set_err(ctx, DFB_ERR_ARG, "cols is not device memory of device %d", ctx->device);
+	if (h->d_res_n_rows)
+		CK(ctx, cudaMemcpyAsync(rows, h->d_res_rows, (size_t)h->d_res_n_rows * sizeof(dfb_split_row), cudaMemcpyDeviceToDevice, ctx->stream));
+	if (h->d_res_n_cols)
+		CK(ctx, cudaMemcpyAsync(cols, h->d_res_cols, (size_t)h->d_res_n_cols * sizeof(int32_t), cudaMemcpyDeviceToDevice, ctx->stream));
+	CK(ctx, cudaStreamSynchronize(ctx->stream));
+	return DFB_OK;
+}
+
+extern "C" int dfb_simple_align_device(dfb_ctx* ctx, const dfb_simple_params* params, const dfb_device_seq_table* refs,
+                                       const dfb_device_seq_table* seqs, const int32_t* task_ref, const int32_t* task_seq, int64_t n_tasks,
+                                       int32_t* out_score)
+{
+	return guarded(ctx, [&] { return dfb_simple_align_device_body(ctx, params, refs, seqs, task_ref, task_seq, n_tasks, out_score); });
+}
+
+extern "C" int dfb_split_align_device(dfb_ctx* ctx, const dfb_split_params* params, const dfb_device_seq_table* refs,
+                                      const dfb_device_seq_table* reads, const int32_t* task_cluster, const int32_t* task_read,
+                                      const int32_t* task_min_score, int64_t n_tasks, int32_t* out_best, int64_t* n_rows, int64_t* n_cols)
+{
+	return guarded(ctx, [&] {
+		return dfb_split_align_device_body(ctx, params, refs, reads, task_cluster, task_read, task_min_score, n_tasks, out_best, n_rows, n_cols);
+	});
 }
 
 #include "dfb_trace.cuh"

@@ -274,4 +274,245 @@ __global__ void __launch_bounds__(DFB_ASM_BLOCK) asm_write_kernel(AsmParams p)
 		});
 	}
 }
+
+// ---- overflow list assembled on the device (the device-resident entry points) ----------------------------------
+// The same rows the host makes of the overflow list (emit_task_rows in dfb_api.cu), in the same order:
+//   1. an LSD radix sort of the events, 8 bits per pass, stable: first over the (matrix, row, column) key, then over
+//      the task -- ov_hist_kernel + a scan of the digit-major histogram + ov_scatter_kernel per pass.  Any number of
+//      events per task and per batch; the passes needed follow from the longest read, window and the chunk's tasks.
+//   2. groups = runs of equal (task, matrix, row): ov_head_kernel flags their first events, a scan numbers them.
+//   3. ov_match_kernel pairs every matrix-1 group (row a) with the matrix-2 group of its task at row L - a (binary
+//      search over the sorted groups); a matched pair is one dfb_split_row with n1 + n2 columns.  Two scans number the
+//      rows and place their columns.
+//   4. ov_rows_kernel / ov_cols_kernel write the rows and the columns (one thread per event: a row of 10^5 tied
+//      columns is spread over the grid).
+//   5. ov_place_kernel merges these rows with the region-assembled rows of the chunk by task (the two never share a
+//      task) into the batch's row array, behind the chunks before it; columns: the region part first, then this part.
+#define DFB_OV_BLOCK 256
+
+struct OvKey
+{
+	int sub_passes; // passes over the (matrix, row, column) key; the task's passes follow
+	int rb, cb;     // bits of a row and of a column
+};
+
+__device__ __forceinline__ unsigned ov_digit(const Event& e, int pass, const OvKey& k)
+{
+	if (pass < k.sub_passes)
+	{
+		const unsigned long long row = (unsigned)e.half_row & 0x3fffffffu, half = (unsigned)e.half_row >> 30;
+		const unsigned long long sub = (half << (k.rb + k.cb)) | (row << k.cb) | (unsigned long long)(unsigned)e.col;
+		return (unsigned)(sub >> (8 * pass)) & 0xffu;
+	}
+	return ((unsigned)e.task >> (8 * (pass - k.sub_passes))) & 0xffu;
+}
+
+// block b's count of digit d at hist[d * n_blocks + b]: the exclusive scan of that order is every element's first slot
+__global__ void __launch_bounds__(DFB_OV_BLOCK) ov_hist_kernel(const Event* __restrict__ in, long long n, int pass, OvKey key,
+                                                               unsigned long long* hist, long long n_blocks)
+{
+	__shared__ unsigned int s[256];
+	s[threadIdx.x] = 0;
+	__syncthreads();
+	const long long i = (long long)blockIdx.x * DFB_OV_BLOCK + threadIdx.x;
+	if (i < n) atomicAdd(&s[ov_digit(in[i], pass, key)], 1u);
+	__syncthreads();
+	hist[(size_t)threadIdx.x * n_blocks + blockIdx.x] = s[threadIdx.x];
+}
+
+__global__ void __launch_bounds__(DFB_OV_BLOCK) ov_scatter_kernel(const Event* __restrict__ in, Event* __restrict__ out, long long n, int pass,
+                                                                  OvKey key, const unsigned long long* __restrict__ hist, long long n_blocks)
+{
+	__shared__ unsigned int s_wc[DFB_OV_BLOCK / 32][257]; // [warp][digit]: elements of the digit in the warp
+	for (int k = threadIdx.x; k < (DFB_OV_BLOCK / 32) * 257; k += DFB_OV_BLOCK) (&s_wc[0][0])[k] = 0;
+	__syncthreads();
+	const long long i = (long long)blockIdx.x * DFB_OV_BLOCK + threadIdx.x;
+	Event e;
+	unsigned d = 256; // (past the end: a digit of its own)
+	if (i < n)
+	{
+		e = in[i];
+		d = ov_digit(e, pass, key);
+	}
+	const unsigned peers = __match_any_sync(0xffffffffu, d);
+	const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+	if (lane == __ffs(peers) - 1) s_wc[warp][d] = (unsigned)__popc(peers);
+	__syncthreads();
+	if (i < n)
+	{
+		unsigned long long at = hist[(size_t)d * n_blocks + blockIdx.x] + (unsigned)__popc(peers & ((1u << lane) - 1u));
+		for (int w = 0; w < warp; w++) at += s_wc[w][d];
+		out[at] = e;
+	}
+}
+
+__device__ __forceinline__ unsigned long long ov_group_key(const Event& e)
+{
+	return ((unsigned long long)(unsigned)e.task << 32) | (unsigned)e.half_row;
+}
+
+struct OvAsmParams
+{
+	const Event* ev;            // sorted
+	long long n;                // events
+	unsigned long long* head;   // [n]: 1 at the first event of a group -> scanned: groups before
+	unsigned long long* scal;   // [0] groups, [1] rows, [2] columns (scan totals)
+	long long* g_first;         // [n + 1] first event of every group, then n
+	int32_t* g_match;           // [n] matrix-2 group paired with a matrix-1 group, -1
+	int32_t* g_matched_by;      // [n] the reverse, -1
+	unsigned long long* g_rows; // [n] 1 for a paired matrix-1 group -> scanned: its row
+	unsigned long long* g_cols; // [n] n1 + n2 -> scanned: its first column
+	// read length of chunk task t: read_off[r + 1] - read_off[r], r = task_read[task_base + t]
+	const int64_t* read_off;
+	const int32_t* task_read;
+	long long task_base;
+	dfb_split_row* x_rows;      // the rows, in order; col_begin relative to the chunk's columns
+	long long asm_cols;         // columns of the region assembly of the chunk (in front of these)
+	int32_t* cols;              // the batch's column array
+	const unsigned long long* base; // [0] rows, [1] columns of the batch before this chunk
+};
+
+__device__ __forceinline__ bool ov_is_head(const Event* ev, long long i)
+{
+	return i == 0 || ov_group_key(ev[i]) != ov_group_key(ev[i - 1]);
+}
+
+__global__ void __launch_bounds__(DFB_OV_BLOCK) ov_head_kernel(OvAsmParams p)
+{
+	const long long i = (long long)blockIdx.x * DFB_OV_BLOCK + threadIdx.x;
+	if (i < p.n) p.head[i] = ov_is_head(p.ev, i) ? 1ull : 0ull;
+}
+
+__global__ void __launch_bounds__(DFB_OV_BLOCK) ov_group_kernel(OvAsmParams p)
+{
+	const long long i = (long long)blockIdx.x * DFB_OV_BLOCK + threadIdx.x;
+	if (i >= p.n) return;
+	if (ov_is_head(p.ev, i)) p.g_first[p.head[i]] = i;
+	if (i == 0) p.g_first[p.scal[0]] = p.n;
+}
+
+__global__ void __launch_bounds__(DFB_OV_BLOCK) ov_match_kernel(OvAsmParams p)
+{
+	const long long g = (long long)blockIdx.x * DFB_OV_BLOCK + threadIdx.x;
+	if (g >= p.n) return;
+	const long long n_groups = (long long)p.scal[0];
+	unsigned long long rows = 0, cols = 0;
+	int32_t match = -1;
+	if (g < n_groups)
+	{
+		const Event e = p.ev[p.g_first[g]];
+		if (((unsigned)e.half_row >> 30) == 0)
+		{
+			const long long r = p.task_read[p.task_base + e.task];
+			const long long want = (p.read_off[r + 1] - p.read_off[r]) - (long long)(e.half_row & 0x3fffffff);
+			if (want >= 0 && want <= 0x3fffffff)
+			{
+				const unsigned long long k = ((unsigned long long)(unsigned)e.task << 32) | (1u << 30) | (unsigned)want;
+				long long lo = g + 1, hi = n_groups; // (matrix 2 sorts behind matrix 1 in the task)
+				while (lo < hi)
+				{
+					const long long mid = (lo + hi) >> 1;
+					if (ov_group_key(p.ev[p.g_first[mid]]) < k) lo = mid + 1;
+					else hi = mid;
+				}
+				if (lo < n_groups && ov_group_key(p.ev[p.g_first[lo]]) == k)
+				{
+					match = (int32_t)lo;
+					p.g_matched_by[lo] = (int32_t)g;
+					rows = 1;
+					cols = (unsigned long long)(p.g_first[g + 1] - p.g_first[g] + p.g_first[lo + 1] - p.g_first[lo]);
+				}
+			}
+		}
+	}
+	p.g_match[g] = match;
+	p.g_rows[g] = rows;
+	p.g_cols[g] = cols;
+}
+
+__global__ void __launch_bounds__(DFB_OV_BLOCK) ov_rows_kernel(OvAsmParams p)
+{
+	const long long g = (long long)blockIdx.x * DFB_OV_BLOCK + threadIdx.x;
+	if (g >= p.n || g >= (long long)p.scal[0]) return;
+	const int32_t j = p.g_match[g];
+	if (j < 0) return;
+	const Event e1 = p.ev[p.g_first[g]], e2 = p.ev[p.g_first[j]];
+	dfb_split_row row;
+	row.task = e1.task;
+	row.read_split = e1.half_row & 0x3fffffff;
+	row.score1 = e1.score;
+	row.score2 = e2.score;
+	row.col_begin = p.asm_cols + (long long)p.g_cols[g];
+	row.n1 = (int32_t)(p.g_first[g + 1] - p.g_first[g]);
+	row.n2 = (int32_t)(p.g_first[j + 1] - p.g_first[j]);
+	p.x_rows[p.g_rows[g]] = row;
+}
+
+__global__ void __launch_bounds__(DFB_OV_BLOCK) ov_cols_kernel(OvAsmParams p)
+{
+	const long long i = (long long)blockIdx.x * DFB_OV_BLOCK + threadIdx.x;
+	if (i >= p.n) return;
+	const long long g = (long long)p.head[i] + (ov_is_head(p.ev, i) ? 1 : 0) - 1;
+	long long at;
+	if (p.g_match[g] >= 0) at = (long long)p.g_cols[g] + (i - p.g_first[g]);
+	else if (p.g_matched_by[g] >= 0)
+	{
+		const long long g1 = p.g_matched_by[g];
+		at = (long long)p.g_cols[g1] + (p.g_first[g1 + 1] - p.g_first[g1]) + (i - p.g_first[g]);
+	}
+	else return;
+	p.cols[(long long)p.base[1] + p.asm_cols + at] = p.ev[i].col;
+}
+
+// items [0, n_asm): region rows; [n_asm, n_asm + n_x_bound): overflow rows (as many as scal[1]); then the region columns
+__global__ void __launch_bounds__(DFB_OV_BLOCK) ov_place_kernel(const dfb_split_row* __restrict__ asm_rows, long long n_asm,
+                                                                const int32_t* __restrict__ asm_cols, long long n_asm_cols,
+                                                                const dfb_split_row* __restrict__ x_rows, long long n_x_bound,
+                                                                const unsigned long long* __restrict__ scal, int32_t task_shift,
+                                                                const unsigned long long* __restrict__ base, dfb_split_row* out_rows,
+                                                                int32_t* out_cols)
+{
+	const long long i = (long long)blockIdx.x * DFB_OV_BLOCK + threadIdx.x;
+	const long long n_x = scal ? (long long)scal[1] : 0;
+	auto below = [](const dfb_split_row* r, long long n, int32_t task) { // rows with a smaller task
+		long long lo = 0, hi = n;
+		while (lo < hi)
+		{
+			const long long mid = (lo + hi) >> 1;
+			if (r[mid].task < task) lo = mid + 1;
+			else hi = mid;
+		}
+		return lo;
+	};
+	dfb_split_row row;
+	long long at;
+	if (i < n_asm)
+	{
+		row = asm_rows[i];
+		at = i + below(x_rows, n_x, row.task);
+	}
+	else if (i < n_asm + n_x_bound)
+	{
+		const long long q = i - n_asm;
+		if (q >= n_x) return;
+		row = x_rows[q];
+		at = q + below(asm_rows, n_asm, row.task);
+	}
+	else
+	{
+		const long long c = i - n_asm - n_x_bound;
+		if (c < n_asm_cols) out_cols[(long long)base[1] + c] = asm_cols[c];
+		return;
+	}
+	row.task += task_shift;
+	row.col_begin += (long long)base[1];
+	out_rows[(long long)base[0] + at] = row;
+}
+
+// the batch's totals behind the chunk
+__global__ void ov_advance_kernel(unsigned long long* base, long long n_asm, long long n_asm_cols, const unsigned long long* scal)
+{
+	base[0] += (unsigned long long)n_asm + (scal ? scal[1] : 0ull);
+	base[1] += (unsigned long long)n_asm_cols + (scal ? scal[2] : 0ull);
+}
 }  // namespace dfb

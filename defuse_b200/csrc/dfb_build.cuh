@@ -353,4 +353,139 @@ __global__ void __launch_bounds__(DFB_BUILD_BLOCK) simple_scatter_kernel(SplitBu
 	else jp->out1 = (int32_t)t;
 }
 
+// ---- argument checks of the device-resident entry points ------------------------------------------------------
+// What check_table and the host builder's task pass find, computed where the caller's arrays live; only this record
+// goes to the host, which words the same messages from it.
+struct TableCheck
+{
+	unsigned long long first_bad; // 2k: offsets decrease at k; 2k + 1: sequence k too long (~0: none)
+	unsigned long long max_len;
+	long long off0, off_n;
+};
+
+struct DeviceCheck
+{
+	TableCheck tab[2];            // table A (references / windows), table B (sequences / reads)
+	unsigned long long bad_task;  // lowest task with an index out of range (~0: none)
+	int a_decreases, b_decreases; // the task arrays decrease somewhere
+};
+
+__global__ void device_check_init_kernel(DeviceCheck* c)
+{
+	c->tab[0].first_bad = c->tab[1].first_bad = ~0ull;
+	c->tab[0].max_len = c->tab[1].max_len = 0;
+	c->bad_task = ~0ull;
+	c->a_decreases = c->b_decreases = 0;
+}
+
+__global__ void __launch_bounds__(DFB_BUILD_BLOCK) table_check_kernel(const int64_t* __restrict__ off, long long n, TableCheck* out)
+{
+	const long long k0 = (long long)blockIdx.x * DFB_BUILD_BLOCK + threadIdx.x, stride = (long long)gridDim.x * DFB_BUILD_BLOCK;
+	if (k0 == 0)
+	{
+		out->off0 = off[0];
+		out->off_n = off[n];
+	}
+	unsigned long long mx = 0;
+	for (long long k = k0; k < n; k += stride)
+	{
+		const long long len = off[k + 1] - off[k];
+		if (len < 0) atomicMin(&out->first_bad, 2ull * (unsigned long long)k);
+		else if (len > 0x7fffff00LL) atomicMin(&out->first_bad, 2ull * (unsigned long long)k + 1);
+		else mx = max(mx, (unsigned long long)len);
+	}
+	for (int o = 16; o > 0; o >>= 1) mx = max(mx, __shfl_down_sync(0xffffffffu, mx, o));
+	if ((threadIdx.x & 31) == 0 && mx) atomicMax(&out->max_len, mx);
+}
+
+// a_lim / b_lim: entries task_a / task_b may name (split: clusters, reads; simple: references, sequences)
+__global__ void __launch_bounds__(DFB_BUILD_BLOCK) task_check_kernel(const int32_t* __restrict__ ta, const int32_t* __restrict__ tb, long long n,
+                                                                      long long a_lim, long long b_lim, DeviceCheck* out)
+{
+	const long long t0 = (long long)blockIdx.x * DFB_BUILD_BLOCK + threadIdx.x, stride = (long long)gridDim.x * DFB_BUILD_BLOCK;
+	int a_dec = 0, b_dec = 0;
+	for (long long t = t0; t < n; t += stride)
+	{
+		const int32_t a = ta[t], b = tb[t];
+		if (a < 0 || a >= a_lim || b < 0 || b >= b_lim) atomicMin(&out->bad_task, (unsigned long long)t);
+		if (t > 0)
+		{
+			a_dec |= a < ta[t - 1];
+			b_dec |= b < tb[t - 1];
+		}
+	}
+	if (__any_sync(0xffffffffu, a_dec) && (threadIdx.x & 31) == 0) out->a_decreases = 1;
+	if (__any_sync(0xffffffffu, b_dec) && (threadIdx.x & 31) == 0) out->b_decreases = 1;
+}
+
+// Where the chunks of a device-resident batch sit in the tables: for chunk k over tasks [t0[k], t0[k+1]),
+// b_lo = task_b[t0[k]], b_hi = task_b[t0[k+1] - 1] + 1 and, with a_monotone, the same for task_a (else a covers the
+// whole table); then the byte offsets of those views.  out[k]: a_lo, a_hi, b_lo, b_hi, off_a[per a_lo],
+// off_a[per a_hi], off_b[b_lo], off_b[b_hi].
+#define DFB_MAX_CHUNKS 8
+struct ChunkStarts
+{
+	long long t[DFB_MAX_CHUNKS + 1];
+};
+
+__global__ void chunk_bounds_kernel(const int64_t* __restrict__ off_a, long long n_a_items, int per, const int64_t* __restrict__ off_b,
+                                    const int32_t* __restrict__ ta, const int32_t* __restrict__ tb, ChunkStarts t0, int K, int a_monotone,
+                                    long long* out)
+{
+	const int k = threadIdx.x;
+	if (k >= K) return;
+	const long long lo = t0.t[k], hi = t0.t[k + 1];
+	long long a_lo = 0, a_hi = n_a_items;
+	if (a_monotone)
+	{
+		a_lo = ta[lo];
+		a_hi = (long long)ta[hi - 1] + 1;
+	}
+	const long long b_lo = tb[lo], b_hi = (long long)tb[hi - 1] + 1;
+	long long* o = out + 8 * k;
+	o[0] = a_lo;
+	o[1] = a_hi;
+	o[2] = b_lo;
+	o[3] = b_hi;
+	o[4] = off_a[per * a_lo];
+	o[5] = off_a[per * a_hi];
+	o[6] = off_b[b_lo];
+	o[7] = off_b[b_hi];
+}
+
+// ---- exclusive scan of a u64 array in place (the desc_count / desc_scan / desc_write pattern) -------------------
+__global__ void __launch_bounds__(DFB_BUILD_BLOCK) u64_scan_sums_kernel(const unsigned long long* __restrict__ v, long long n,
+                                                                         unsigned long long* block_sums)
+{
+	const long long i0 = ((long long)blockIdx.x * DFB_BUILD_BLOCK + threadIdx.x) * DFB_BUILD_ITEMS;
+	unsigned long long sum = 0;
+#pragma unroll
+	for (int k = 0; k < DFB_BUILD_ITEMS; k++)
+		if (i0 + k < n) sum += v[i0 + k];
+	unsigned long long all = 0;
+	block_exclusive_scan(sum, &all);
+	if (threadIdx.x == 0) block_sums[blockIdx.x] = all;
+}
+
+__global__ void __launch_bounds__(DFB_BUILD_BLOCK) u64_scan_write_kernel(unsigned long long* v, long long n,
+                                                                          const unsigned long long* __restrict__ block_sums)
+{
+	const long long i0 = ((long long)blockIdx.x * DFB_BUILD_BLOCK + threadIdx.x) * DFB_BUILD_ITEMS;
+	unsigned long long x[DFB_BUILD_ITEMS], sum = 0;
+#pragma unroll
+	for (int k = 0; k < DFB_BUILD_ITEMS; k++)
+	{
+		x[k] = i0 + k < n ? v[i0 + k] : 0ull;
+		sum += x[k];
+	}
+	unsigned long long at = block_sums[blockIdx.x] + block_exclusive_scan(sum, nullptr);
+#pragma unroll
+	for (int k = 0; k < DFB_BUILD_ITEMS; k++)
+		if (i0 + k < n)
+		{
+			v[i0 + k] = at;
+			at += x[k];
+		}
+}
+
 }  // namespace dfb

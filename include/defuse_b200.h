@@ -151,7 +151,8 @@ DFB_API void dfb_ctx_destroy(dfb_ctx* ctx);
  * on this thread.  Never NULL. */
 DFB_API const char* dfb_last_error(const dfb_ctx* ctx);
 /* Run on a caller-provided cudaStream_t (e.g. torch's current stream) instead of the
- * context's own; pass NULL to go back. */
+ * context's own; pass NULL to go back.  (NULL does not name the legacy default stream here: the context's own stream
+ * does not wait for it.  Pass cudaStreamLegacy, (void*)1, to run behind work on the legacy default stream.) */
 DFB_API int dfb_ctx_set_stream(dfb_ctx* ctx, void* cuda_stream);
 DFB_API int dfb_ctx_device_info(const dfb_ctx* ctx, dfb_device_info* info);
 
@@ -187,6 +188,46 @@ DFB_API int dfb_split_result_view(const dfb_ctx* ctx, const dfb_split_row** rows
  * what the call itself moved -- a batch cut into chunks uploads every window once, a resident plan's statistics
  * (dfb_plan_get_stats) do not describe it.  Timings are 0. */
 DFB_API int dfb_split_result_stats(const dfb_ctx* ctx, dfb_plan_stats* stats);
+
+/* ---- device-resident forms: batches already in GPU memory, results left there ----------------- */
+
+/* A table of byte strings in device memory (e.g. torch tensors): the CSR form of dfb_seq_table with `bytes` and `off`
+ * on the GPU.  `n` and `n_bytes` are host values; n_bytes is the size of the `bytes` allocation, and off[n] may not
+ * exceed it. */
+typedef struct dfb_device_seq_table
+{
+	const uint8_t* bytes; /* device memory */
+	const int64_t* off;   /* device memory, n + 1 entries, off[0] == 0, non-decreasing */
+	int64_t n;            /* host value */
+	int64_t n_bytes;      /* host value: size of the `bytes` allocation */
+} dfb_device_seq_table;
+
+/* The device-resident forms of dfb_simple_align_batch and dfb_split_align_batch.  Every array -- both tables, the task
+ * arrays and the outputs -- is device memory of the context's device; host memory (pinned or pageable), managed memory
+ * and memory of another device are refused with DFB_ERR_ARG before any work is queued.  The work is ordered behind what
+ * was queued on the context's stream (dfb_ctx_set_stream) before the call, and the call returns once the outputs are
+ * written.  Results are those of the host forms on the same data, byte for byte and in the same order; malformed
+ * tables and task indices fail with the same status and message (plus "off[n] exceeds n_bytes"), except that an index
+ * out of range is always reported at the lowest bad task of the batch (the host form cuts a large batch with
+ * non-decreasing reads into chunks first and may name a chunk's first task).  Sequence bytes,
+ * offsets, task arrays and results stay on the GPU: what crosses PCIe is fixed-size counters (the argument-check record,
+ * class counts, overflow and row/column totals; dfb_split_result_stats counts them), except for chunks holding tasks
+ * only the s32 kernels take (scoring triples or lengths outside the s16x2 range), whose offsets and task arrays -- never
+ * their bytes -- are read back to build their job lists on the host. */
+DFB_API int dfb_simple_align_device(dfb_ctx* ctx, const dfb_simple_params* params,
+                                    const dfb_device_seq_table* refs, const dfb_device_seq_table* seqs,
+                                    const int32_t* d_task_ref, const int32_t* d_task_seq, int64_t n_tasks,
+                                    int32_t* d_out_score);
+/* out_best as for dfb_split_align_batch; *n_rows / *n_cols receive the result's size.  The rows and columns stay in
+ * device memory owned by the context until the next split call on it: copy them with dfb_split_result_copy_device.
+ * (dfb_split_result_size / _copy / _view refuse a device-resident result with DFB_ERR_STATE.) */
+DFB_API int dfb_split_align_device(dfb_ctx* ctx, const dfb_split_params* params,
+                                   const dfb_device_seq_table* refs, const dfb_device_seq_table* reads,
+                                   const int32_t* d_task_cluster, const int32_t* d_task_read,
+                                   const int32_t* d_task_min_score, int64_t n_tasks,
+                                   int32_t* d_out_best, int64_t* n_rows, int64_t* n_cols);
+/* Copies the last dfb_split_align_device result into device buffers of n_rows / n_cols entries. */
+DFB_API int dfb_split_result_copy_device(dfb_ctx* ctx, dfb_split_row* d_rows, int32_t* d_cols);
 
 /* ---- backtrace of chosen split alignments (GetAlignments(..., backtrace=true)) ------------- */
 
