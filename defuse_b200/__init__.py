@@ -72,6 +72,11 @@ SPLIT_ROW_DTYPE = np.dtype([("task", "<i4"), ("read_split", "<i4"), ("score1", "
                             ("col_begin", "<i8"), ("n1", "<i4"), ("n2", "<i4")])
 assert SPLIT_ROW_DTYPE.itemsize == 32
 
+# dfb_split_record: what SplitAlignmentTask::Align keeps per distinct refSplit (DeviceSplitResult.records())
+SPLIT_RECORD_DTYPE = np.dtype([("task", "<i4"), ("ref_split1", "<i4"), ("ref_split2", "<i4"), ("read_split1", "<i4"),
+                               ("read_split2", "<i4"), ("score", "<i4")])
+assert SPLIT_RECORD_DTYPE.itemsize == 24
+
 _lib = None
 
 
@@ -125,6 +130,8 @@ def load_library():
         "dfb_split_align_device": ([vp, P(_SplitParams), P(_DeviceSeqTable), P(_DeviceSeqTable), vp, vp, vp, i64, vp, P(i64), P(i64)],
                                    ctypes.c_int),
         "dfb_split_result_copy_device": ([vp, vp, vp], ctypes.c_int),
+        "dfb_split_records_device": ([vp, P(_DeviceSeqTable), P(_DeviceSeqTable), vp, vp, i64, vp, i64, vp, i64, P(i64)], ctypes.c_int),
+        "dfb_split_records_copy_device": ([vp, vp], ctypes.c_int),
         "dfb_split_backtrace_batch": ([vp, P(_SplitParams), P(_SeqTable), P(_SeqTable), vp, vp, vp, vp, vp, i64, vp, vp, i64,
                                        P(i64)], ctypes.c_int),
     }
@@ -144,6 +151,7 @@ ABI_SYMBOLS = (
     "dfb_simple_plan_fetch", "dfb_split_plan_fetch", "dfb_split_plan_copy", "dfb_plan_get_stats", "dfb_plan_destroy",
     "dfb_microbench_issue_rate", "dfb_split_backtrace_batch", "dfb_ctx_memory_info",
     "dfb_split_result_stats", "dfb_simple_align_device", "dfb_split_align_device", "dfb_split_result_copy_device",
+    "dfb_split_records_device", "dfb_split_records_copy_device",
 )
 
 
@@ -424,13 +432,23 @@ class SplitResult:
 
 class DeviceSplitResult:
     """Result of SplitReadAligner.align_device, in GPU memory: `best` (int32, per task), `rows` (the 32-byte
-    dfb_split_row records as an (n, 8) int32 tensor; the field accessors below read it) and `cols` (int32 column pool)."""
+    dfb_split_row records as an (n, 8) int32 tensor; the field accessors below read it) and `cols` (int32 column pool).
+    It keeps the context, the tables and the task tensors of the batch it was computed from."""
 
-    def __init__(self, best, rows, cols, lens):
+    def __init__(self, best, rows, cols, ctx, refs, reads, task_cluster, task_read):
         self.best = best
         self.rows = rows
         self.cols = cols
-        self._lens = lens
+        self.ctx = ctx
+        self.refs = refs
+        self.reads = reads
+        self.task_cluster = task_cluster
+        self.task_read = task_read
+
+    def _lens(self):
+        tc, tr = self.task_cluster.cpu().numpy(), self.task_read.cpu().numpy()
+        return SplitReadAligner._lens(SeqTable(np.zeros(0, np.uint8), self.refs.off.cpu().numpy()),
+                                      SeqTable(np.zeros(0, np.uint8), self.reads.off.cpu().numpy()), tc, tr)
 
     # fields of the records (SPLIT_ROW_DTYPE): task, read_split, score1, score2, col_begin (int64), n1, n2
     @property
@@ -468,6 +486,30 @@ class DeviceSplitResult:
         rows = np.ascontiguousarray(self.rows.cpu().numpy()).view(SPLIT_ROW_DTYPE).reshape(-1)
         lens = self._lens()
         return SplitResult(self.best.cpu().numpy(), rows, self.cols.cpu().numpy(), lambda: lens)
+
+    def records(self):
+        """The records SplitAlignmentTask::Align keeps for every task (tools/SplitAlignment.cpp:381-400), expanded and
+        de-duplicated on the GPU through dfb_split_records_device: an (n, 6) int32 CUDA tensor with the columns of
+        SPLIT_RECORD_DTYPE (task, ref_split1, ref_split2, read_split1, read_split2, score), in task order and, within
+        a task, in GetAlignments' order -- np.concatenate of SplitResult.records(t) with the task prepended.  Runs on
+        torch's current stream.  The read and window lengths come from the batch's tables and task tensors: they must
+        not have been reused since the align_device call."""
+        import torch
+        ctx, lib = self.ctx, self.ctx._lib
+        _check_tensor("cols", self.cols, torch.int32, self.rows.device)
+        if self.rows.dtype != torch.int32 or self.rows.dim() != 2 or self.rows.shape[1] != 8 or not self.rows.is_contiguous():
+            raise ValueError("rows must be a contiguous (n, 8) int32 tensor of dfb_split_row records")
+        rt, st = self.refs.c_struct(), self.reads.c_struct()
+        n = ctypes.c_int64()
+
+        def run():
+            ctx._check(lib.dfb_split_records_device(ctx._h, ctypes.byref(rt), ctypes.byref(st), _dptr(self.task_cluster),
+                                                    _dptr(self.task_read), self.task_cluster.numel(), _dptr(self.rows),
+                                                    self.rows.shape[0], _dptr(self.cols), self.cols.numel(), ctypes.byref(n)))
+            out = torch.empty((n.value, 6), dtype=torch.int32, device=self.rows.device)
+            ctx._check(lib.dfb_split_records_copy_device(ctx._h, _dptr(out)))
+            return out
+        return ctx._on_torch_stream(run)
 
 
 def _view_arrays(rows_p, n_rows, cols_p, n_cols, copy):
@@ -645,12 +687,7 @@ class SplitReadAligner:
             return rows, cols
 
         rows, cols = self.ctx._on_torch_stream(run)
-
-        def lens():
-            tc, tr = task_cluster.cpu().numpy(), task_read.cpu().numpy()
-            return self._lens(SeqTable(np.zeros(0, np.uint8), refs.off.cpu().numpy()),
-                              SeqTable(np.zeros(0, np.uint8), reads.off.cpu().numpy()), tc, tr)
-        return DeviceSplitResult(out[:n], rows, cols, lens)
+        return DeviceSplitResult(out[:n], rows, cols, self.ctx, refs, reads, task_cluster, task_read)
 
     def backtrace_batch(self, refs, reads, task_cluster, task_read, ref_split1, ref_split2, read_split):
         """matches1 / matches2 of chosen alignments (GetAlignments(..., backtrace=True), tools/SplitReadAligner.cpp:

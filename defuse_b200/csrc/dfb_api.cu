@@ -226,6 +226,10 @@ struct dfb_ctx
 	HostPool* pool = nullptr;       // plan building (and everything else on the caller's thread)
 	HostPool* pool_fetch = nullptr; // result assembly when it runs on the pipelining helper thread
 	dfb_plan* last_split = nullptr; // result holder of dfb_split_align_batch
+	// records of the last dfb_split_records_device call (device memory of the stream-ordered pool)
+	dfb_split_record* d_records = nullptr;
+	int64_t n_records = 0;
+	bool has_records = false;
 	int host_threads = 1;
 	// recycled host memory of the result assembly (kept mapped between batches)
 	HostArr<dfb_split_row> spare_rows;
@@ -433,6 +437,7 @@ extern "C" void dfb_ctx_destroy(dfb_ctx* ctx)
 	if (!ctx) return;
 	cudaSetDevice(ctx->device);
 	if (ctx->last_split) dfb_plan_destroy(ctx->last_split);
+	if (ctx->d_records) cudaFreeAsync(ctx->d_records, ctx->stream);
 	cudaStreamSynchronize(ctx->stream);
 	for (auto& b : ctx->h_in) b.release();
 	ctx->h_ring.release();
@@ -2954,6 +2959,44 @@ static bool is_ctx_device_memory(const dfb_ctx* ctx, const void* p)
 	return a.type == cudaMemoryTypeDevice && a.device == ctx->device;
 }
 
+// the kernels of check_device_args: the record is initialised, then both tables and the task arrays are checked
+static void enqueue_device_checks(dfb_ctx* ctx, bool simple, const dfb_device_seq_table* A, const dfb_device_seq_table* B,
+                                  const int32_t* ta, const int32_t* tb, int64_t n_tasks, DeviceCheck* d_chk)
+{
+	const dfb_device_seq_table* tabs[2] = {A, B};
+	const int max_grid = ctx->prop.multiProcessorCount * 8;
+	auto grid = [&](int64_t n) { return (unsigned)std::max<int64_t>(1, std::min<int64_t>((n + DFB_BUILD_BLOCK - 1) / DFB_BUILD_BLOCK, max_grid)); };
+	device_check_init_kernel<<<1, 1, 0, ctx->stream>>>(d_chk);
+	for (int k = 0; k < 2; k++) table_check_kernel<<<grid(tabs[k]->n), DFB_BUILD_BLOCK, 0, ctx->stream>>>(tabs[k]->off, tabs[k]->n, &d_chk->tab[k]);
+	if (n_tasks)
+		task_check_kernel<<<grid(n_tasks), DFB_BUILD_BLOCK, 0, ctx->stream>>>(ta, tb, n_tasks, simple ? A->n : A->n / 2, B->n, d_chk);
+}
+
+// the status and message of a check record read back from the device
+static int device_check_status(dfb_ctx* ctx, bool simple, const dfb_device_seq_table* A, const dfb_device_seq_table* B, int64_t n_tasks,
+                               const DeviceCheck& chk)
+{
+	const char* names[2] = {"refs", simple ? "seqs" : "reads"};
+	const dfb_device_seq_table* tabs[2] = {A, B};
+	for (int k = 0; k < 2; k++)
+	{
+		const TableCheck& c = chk.tab[k];
+		if (tabs[k]->n > 0 && !tabs[k]->bytes && c.off_n > 0) return set_err(ctx, DFB_ERR_ARG, "%s: null table", names[k]);
+		if (c.off0 != 0) return set_err(ctx, DFB_ERR_ARG, "%s: off[0] must be 0", names[k]);
+		if (c.first_bad != ~0ull)
+		{
+			if (c.first_bad & 1) return set_err(ctx, DFB_ERR_ARG, "%s: sequence %lld too long", names[k], (long long)(c.first_bad >> 1));
+			return set_err(ctx, DFB_ERR_ARG, "%s: offsets decrease at %lld", names[k], (long long)(c.first_bad >> 1));
+		}
+		if (c.off_n > tabs[k]->n_bytes)
+			return set_err(ctx, DFB_ERR_ARG, "%s: off[n] = %lld exceeds n_bytes = %lld", names[k], (long long)c.off_n, (long long)tabs[k]->n_bytes);
+	}
+	if (!simple && (A->n & 1)) return set_err(ctx, DFB_ERR_ARG, "refs must hold two windows per cluster (n is odd)");
+	if (n_tasks > 0x7fffff00LL) return set_err(ctx, DFB_ERR_ARG, "too many tasks in one batch");
+	if (chk.bad_task != ~0ull) return set_err(ctx, DFB_ERR_ARG, "task %lld: table index out of range", (long long)chk.bad_task);
+	return DFB_OK;
+}
+
 // The argument checks of the host form (check_simple_args / check_split_args, and the builders' task index check) with
 // the same statuses and messages, run on the device; plus off[n] <= n_bytes.  *chk receives the record.
 static int check_device_args(dfb_ctx* ctx, bool simple, const void* params, const dfb_device_seq_table* A, const dfb_device_seq_table* B,
@@ -2977,34 +3020,13 @@ static int check_device_args(dfb_ctx* ctx, bool simple, const void* params, cons
 	CK(ctx, dalloc(ctx, (void**)&d_chk, sizeof(DeviceCheck)));
 	CK(ctx, ctx->h_out.ensure(sizeof(DeviceCheck)));
 	DeviceCheck* h_chk = (DeviceCheck*)ctx->h_out.p;
-	const int max_grid = ctx->prop.multiProcessorCount * 8;
-	auto grid = [&](int64_t n) { return (unsigned)std::max<int64_t>(1, std::min<int64_t>((n + DFB_BUILD_BLOCK - 1) / DFB_BUILD_BLOCK, max_grid)); };
-	device_check_init_kernel<<<1, 1, 0, ctx->stream>>>(d_chk);
-	for (int k = 0; k < 2; k++) table_check_kernel<<<grid(tabs[k]->n), DFB_BUILD_BLOCK, 0, ctx->stream>>>(tabs[k]->off, tabs[k]->n, &d_chk->tab[k]);
-	if (n_tasks)
-		task_check_kernel<<<grid(n_tasks), DFB_BUILD_BLOCK, 0, ctx->stream>>>(ta, tb, n_tasks, simple ? A->n : A->n / 2, B->n, d_chk);
+	enqueue_device_checks(ctx, simple, A, B, ta, tb, n_tasks, d_chk);
 	CK(ctx, cudaGetLastError());
 	CK(ctx, cudaMemcpyAsync(h_chk, d_chk, sizeof(DeviceCheck), cudaMemcpyDeviceToHost, ctx->stream));
 	cudaFreeAsync(d_chk, ctx->stream);
 	CK(ctx, cudaStreamSynchronize(ctx->stream));
 	*chk = *h_chk;
-	for (int k = 0; k < 2; k++)
-	{
-		const TableCheck& c = chk->tab[k];
-		if (tabs[k]->n > 0 && !tabs[k]->bytes && c.off_n > 0) return set_err(ctx, DFB_ERR_ARG, "%s: null table", names[k]);
-		if (c.off0 != 0) return set_err(ctx, DFB_ERR_ARG, "%s: off[0] must be 0", names[k]);
-		if (c.first_bad != ~0ull)
-		{
-			if (c.first_bad & 1) return set_err(ctx, DFB_ERR_ARG, "%s: sequence %lld too long", names[k], (long long)(c.first_bad >> 1));
-			return set_err(ctx, DFB_ERR_ARG, "%s: offsets decrease at %lld", names[k], (long long)(c.first_bad >> 1));
-		}
-		if (c.off_n > tabs[k]->n_bytes)
-			return set_err(ctx, DFB_ERR_ARG, "%s: off[n] = %lld exceeds n_bytes = %lld", names[k], (long long)c.off_n, (long long)tabs[k]->n_bytes);
-	}
-	if (!simple && (A->n & 1)) return set_err(ctx, DFB_ERR_ARG, "refs must hold two windows per cluster (n is odd)");
-	if (n_tasks > 0x7fffff00LL) return set_err(ctx, DFB_ERR_ARG, "too many tasks in one batch");
-	if (chk->bad_task != ~0ull) return set_err(ctx, DFB_ERR_ARG, "task %lld: table index out of range", (long long)chk->bad_task);
-	return DFB_OK;
+	return device_check_status(ctx, simple, A, B, n_tasks, *chk);
 }
 
 // Work on the upload and copy streams is ordered behind what the caller queued on the context's stream before the call
@@ -3468,3 +3490,4 @@ extern "C" int dfb_split_align_device(dfb_ctx* ctx, const dfb_split_params* para
 }
 
 #include "dfb_trace.cuh"
+#include "dfb_records.cuh"

@@ -229,6 +229,40 @@ DFB_API int dfb_split_align_device(dfb_ctx* ctx, const dfb_split_params* params,
 /* Copies the last dfb_split_align_device result into device buffers of n_rows / n_cols entries. */
 DFB_API int dfb_split_result_copy_device(dfb_ctx* ctx, dfb_split_row* d_rows, int32_t* d_cols);
 
+/* One record SplitAlignmentTask::Align keeps (tools/SplitAlignment.cpp:381-400): the first alignment of a task with
+ * a given refSplit, scored min(score1, score2).  This is what dosplitalign writes per task. */
+typedef struct dfb_split_record
+{
+	int32_t task;
+	int32_t ref_split1;  /* refSplit.first  = i1 */
+	int32_t ref_split2;  /* refSplit.second = len(reference2) - i2 - 1 */
+	int32_t read_split1; /* readSplit.first  = read_split */
+	int32_t read_split2; /* readSplit.second = len(read) - read_split */
+	int32_t score;       /* min(score1, score2) */
+} dfb_split_record;
+
+/* The records of a device-resident split result, expanded and de-duplicated on the GPU.  rows / cols are a result in
+ * the form dfb_split_result_copy_device writes (any device buffers holding one: the call keeps no state of the last
+ * split call), refs / reads / d_task_cluster / d_task_read the batch it was computed from; len(read) and
+ * len(reference2) are read from them.  Order, which is the order GetAlignments emits (tools/SplitReadAligner.cpp:
+ * 272-297) and dosplitalign keeps: tasks ascending; within a task, rows in the order given, then i1 ascending, then
+ * i2 ascending; of the alignments with the same (i1, i2) only the first in this order is kept.  Rows with n1 == 0 or
+ * n2 == 0 and tasks without rows give nothing.  Every array is device memory of the context's device (else
+ * DFB_ERR_ARG before any work is queued).  The argument checks run on the GPU: those of dfb_split_align_device on the
+ * tables and task arrays (same statuses and messages), and on the rows -- task in [0, n_tasks) and non-decreasing,
+ * col_begin >= 0, n1, n2 >= 0, col_begin + n1 + n2 <= n_cols, 0 <= read_split <= len(read), every column in
+ * [0, len(window)] on its side and strictly ascending within its list -- which also catch tables that do not belong to
+ * the rows.  The work is ordered behind the context's stream and the call returns once the records are written; what
+ * crosses PCIe is the check record and the totals.  *n_records receives the number of records, which stay in device
+ * memory owned by the context until the next dfb_split_records_device call on it (or dfb_ctx_destroy). */
+DFB_API int dfb_split_records_device(dfb_ctx* ctx, const dfb_device_seq_table* refs, const dfb_device_seq_table* reads,
+                                     const int32_t* d_task_cluster, const int32_t* d_task_read, int64_t n_tasks,
+                                     const dfb_split_row* d_rows, int64_t n_rows, const int32_t* d_cols, int64_t n_cols,
+                                     int64_t* n_records);
+/* Copies the records of the last successful dfb_split_records_device call into a device buffer of n_records entries;
+ * DFB_ERR_STATE when there are none. */
+DFB_API int dfb_split_records_copy_device(dfb_ctx* ctx, dfb_split_record* d_records);
+
 /* ---- backtrace of chosen split alignments (GetAlignments(..., backtrace=true)) ------------- */
 
 /* The matches1 / matches2 lists of SplitReadAlignment (tools/SplitReadAligner.h:21-30) for alignments the caller
