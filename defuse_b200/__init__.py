@@ -134,6 +134,9 @@ def load_library():
         "dfb_split_records_copy_device": ([vp, vp], ctypes.c_int),
         "dfb_split_backtrace_batch": ([vp, P(_SplitParams), P(_SeqTable), P(_SeqTable), vp, vp, vp, vp, vp, i64, vp, vp, i64,
                                        P(i64)], ctypes.c_int),
+        "dfb_split_backtrace_device": ([vp, P(_SplitParams), P(_DeviceSeqTable), P(_DeviceSeqTable), vp, vp, i64, vp, i64, P(i64)],
+                                       ctypes.c_int),
+        "dfb_split_backtrace_copy_device": ([vp, vp, vp], ctypes.c_int),
     }
     for name, (args, res) in sig.items():
         fn = getattr(lib, name)
@@ -151,7 +154,7 @@ ABI_SYMBOLS = (
     "dfb_simple_plan_fetch", "dfb_split_plan_fetch", "dfb_split_plan_copy", "dfb_plan_get_stats", "dfb_plan_destroy",
     "dfb_microbench_issue_rate", "dfb_split_backtrace_batch", "dfb_ctx_memory_info",
     "dfb_split_result_stats", "dfb_simple_align_device", "dfb_split_align_device", "dfb_split_result_copy_device",
-    "dfb_split_records_device", "dfb_split_records_copy_device",
+    "dfb_split_records_device", "dfb_split_records_copy_device", "dfb_split_backtrace_device", "dfb_split_backtrace_copy_device",
 )
 
 
@@ -433,9 +436,10 @@ class SplitResult:
 class DeviceSplitResult:
     """Result of SplitReadAligner.align_device, in GPU memory: `best` (int32, per task), `rows` (the 32-byte
     dfb_split_row records as an (n, 8) int32 tensor; the field accessors below read it) and `cols` (int32 column pool).
-    It keeps the context, the tables and the task tensors of the batch it was computed from."""
+    It keeps the context, the tables and the task tensors of the batch it was computed from, and the aligner's scoring
+    (`params`), which backtrace() uses."""
 
-    def __init__(self, best, rows, cols, ctx, refs, reads, task_cluster, task_read):
+    def __init__(self, best, rows, cols, ctx, refs, reads, task_cluster, task_read, params=None):
         self.best = best
         self.rows = rows
         self.cols = cols
@@ -444,6 +448,7 @@ class DeviceSplitResult:
         self.reads = reads
         self.task_cluster = task_cluster
         self.task_read = task_read
+        self.params = params
 
     def _lens(self):
         tc, tr = self.task_cluster.cpu().numpy(), self.task_read.cpu().numpy()
@@ -509,6 +514,44 @@ class DeviceSplitResult:
             out = torch.empty((n.value, 6), dtype=torch.int32, device=self.rows.device)
             ctx._check(lib.dfb_split_records_copy_device(ctx._h, _dptr(out)))
             return out
+        return ctx._on_torch_stream(run)
+
+    def backtrace(self, records):
+        """matches1 / matches2 of chosen alignments (GetAlignments(..., backtrace=True)) through
+        dfb_split_backtrace_device, with the scoring of the align_device call: the device twin of
+        SplitReadAligner.backtrace_batch.  `records` is an (n, 6) int32 CUDA tensor of SPLIT_RECORD_DTYPE rows -- the
+        output of records() or any rows of it, in any order; record k names the alignment of task records[k, 0] with
+        refSplit (records[k, 1], records[k, 2]) and readSplit records[k, 3:5].  Returns (match_off, pairs): an int64
+        CUDA tensor of 2n + 1 entries and an (n_pairs, 2) int32 CUDA tensor of (refPos, readPos) rows, with
+        pairs[match_off[2k]:match_off[2k+1]] = matches1 of record k and pairs[match_off[2k+1]:match_off[2k+2]] its
+        matches2.  Runs on torch's current stream.  The tables and task tensors must not have been reused since the
+        align_device call."""
+        import torch
+        if not isinstance(records, torch.Tensor):
+            raise TypeError("records must be a torch.Tensor, got %s" % type(records).__name__)
+        if records.dtype != torch.int32:
+            raise TypeError("records must be torch.int32, got %s" % records.dtype)
+        if not records.is_cuda:
+            raise ValueError("records must be a CUDA tensor, got one on %s" % records.device)
+        if records.device != self.rows.device:
+            raise ValueError("records is on %s, the result on %s" % (records.device, self.rows.device))
+        if records.dim() != 2 or records.shape[1] != 6 or not records.is_contiguous():
+            raise ValueError("records must be a contiguous (n, 6) int32 tensor of dfb_split_record rows")
+        if self.params is None:
+            raise ValueError("this result carries no scoring: it was not made by SplitReadAligner.align_device")
+        ctx, lib = self.ctx, self.ctx._lib
+        rt, st = self.refs.c_struct(), self.reads.c_struct()
+        n = records.shape[0]
+        total = ctypes.c_int64()
+
+        def run():
+            ctx._check(lib.dfb_split_backtrace_device(ctx._h, ctypes.byref(self.params), ctypes.byref(rt), ctypes.byref(st),
+                                                      _dptr(self.task_cluster), _dptr(self.task_read), self.task_cluster.numel(),
+                                                      _dptr(records), n, ctypes.byref(total)))
+            off = torch.empty(2 * n + 1, dtype=torch.int64, device=records.device)
+            pairs = torch.empty((total.value, 2), dtype=torch.int32, device=records.device)
+            ctx._check(lib.dfb_split_backtrace_copy_device(ctx._h, _dptr(off), _dptr(pairs)))
+            return off, pairs
         return ctx._on_torch_stream(run)
 
 
@@ -687,7 +730,7 @@ class SplitReadAligner:
             return rows, cols
 
         rows, cols = self.ctx._on_torch_stream(run)
-        return DeviceSplitResult(out[:n], rows, cols, self.ctx, refs, reads, task_cluster, task_read)
+        return DeviceSplitResult(out[:n], rows, cols, self.ctx, refs, reads, task_cluster, task_read, self.params)
 
     def backtrace_batch(self, refs, reads, task_cluster, task_read, ref_split1, ref_split2, read_split):
         """matches1 / matches2 of chosen alignments (GetAlignments(..., backtrace=True), tools/SplitReadAligner.cpp:

@@ -230,6 +230,12 @@ struct dfb_ctx
 	dfb_split_record* d_records = nullptr;
 	int64_t n_records = 0;
 	bool has_records = false;
+	// match lists of the last dfb_split_backtrace_device call: 2 n + 1 offsets and the (refPos, readPos) pairs, one
+	// block per wave of the call, in order
+	int64_t* d_bt_off = nullptr;
+	std::vector<std::pair<int2*, int64_t>> bt_chunks;
+	int64_t n_bt_records = 0, n_bt_pairs = 0;
+	bool has_bt = false;
 	int host_threads = 1;
 	// recycled host memory of the result assembly (kept mapped between batches)
 	HostArr<dfb_split_row> spare_rows;
@@ -438,6 +444,8 @@ extern "C" void dfb_ctx_destroy(dfb_ctx* ctx)
 	cudaSetDevice(ctx->device);
 	if (ctx->last_split) dfb_plan_destroy(ctx->last_split);
 	if (ctx->d_records) cudaFreeAsync(ctx->d_records, ctx->stream);
+	if (ctx->d_bt_off) cudaFreeAsync(ctx->d_bt_off, ctx->stream);
+	for (auto& c : ctx->bt_chunks) cudaFreeAsync(c.first, ctx->stream);
 	cudaStreamSynchronize(ctx->stream);
 	for (auto& b : ctx->h_in) b.release();
 	ctx->h_ring.release();

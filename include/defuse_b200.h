@@ -286,6 +286,28 @@ DFB_API int dfb_split_backtrace_batch(dfb_ctx* ctx, const dfb_split_params* para
                           const int32_t* task_read_split, int64_t n_tasks,
                           int64_t* match_off, int32_t* matches, int64_t matches_cap, int64_t* n_pairs);
 
+/* The device-resident form of dfb_split_backtrace_batch, for records of a device-resident split result.  Record k
+ * names one alignment of task t = d_records[k].task: reads[d_task_read[t]] against cluster d_task_cluster[t], with
+ * refSplit (ref_split1, ref_split2) and readSplit.first = read_split1; the start cells are those of
+ * dfb_split_backtrace_batch, and score is not read.  The records may be any rows of a dfb_split_records_device output
+ * or records built by hand, in any order and with repeats.  The output has the layout of dfb_split_backtrace_batch --
+ * 2 * n_records + 1 int64 offsets, interleaved int32 (refPos, readPos) pairs, both lists ascending -- and is byte-equal
+ * to it called per record with (task_cluster[t], task_read[t], ref_split1, ref_split2, read_split1); it is exact-size
+ * and *n_pairs receives the total.  Every array is device memory of the context's device (else DFB_ERR_ARG before any
+ * work is queued).  The argument checks run on the GPU: those of dfb_split_align_device on the tables and task arrays
+ * (same statuses and messages), and per record -- task in [0, n_tasks), both start cells inside their matrices,
+ * read_split2 == len(read) - read_split1 (which also catches tables that do not belong to the records) -- reported at
+ * the lowest bad record.  The work is ordered behind the context's stream and the call returns once the output is
+ * written; what crosses PCIe is the check record and the totals.  The output stays in device memory owned by the
+ * context until the next dfb_split_backtrace_device call on it (or dfb_ctx_destroy). */
+DFB_API int dfb_split_backtrace_device(dfb_ctx* ctx, const dfb_split_params* params,
+                                       const dfb_device_seq_table* refs, const dfb_device_seq_table* reads,
+                                       const int32_t* d_task_cluster, const int32_t* d_task_read, int64_t n_tasks,
+                                       const dfb_split_record* d_records, int64_t n_records, int64_t* n_pairs);
+/* Copies the output of the last successful dfb_split_backtrace_device call into device buffers of 2 * n_records + 1
+ * offsets and 2 * n_pairs int32; DFB_ERR_STATE when there is none. */
+DFB_API int dfb_split_backtrace_copy_device(dfb_ctx* ctx, int64_t* d_match_off, int32_t* d_matches);
+
 /* ---- staged form: the same work with the batch resident in HBM -------------------------- */
 
 /* Copies the tables to the device, packs them (2-bit codes + exception plane) and builds
