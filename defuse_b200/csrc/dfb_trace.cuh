@@ -1,306 +1,14 @@
 // Backtrace of chosen split alignments: SplitReadAligner::GetAlignments(..., backtrace=true)
 // (tools/SplitReadAligner.cpp:56-69 pointer rule, :124-143 BackTracePath, :145-154 ReverseMatches, :287-292).
 //
-// Included at the end of dfb_api.cu (it needs dfb_ctx).  The workload is small by construction -- splitseq
-// re-aligns only the reads that support one predicted break (tools/splitseq.cpp:100-125) -- so this path is
-// built for exactness over every parameter set (s32 arithmetic, raw byte equality, any length), not for TCUPS:
-//
-//   trace_fill_kernel   one warp per matrix (a task has two: read x ref1, rev(read) x rev(ref2)).  Lane l owns
-//                       read row j = tile + l + 1 and sweeps the reference as a skewed wavefront, exactly the
-//                       geometry of the s32 DP kernel; what is new is the pointer of every cell, 2 bits, packed
-//                       16 columns per word by the lane that owns the row:
-//                         0 diagonal, 1 (i-1,j), 2 (i,j-1); later writers win, so 2 > 1 > 0 (:56-69)
-//   trace_walk_kernel   one thread per matrix walks the pointers from the start cell until j == 0 and records
-//                       the diagonal steps in walk order (descending positions).
-// The host reverses matrix 1's list and maps matrix 2's coordinates back to the unreversed sequences (whose
-// double reversal is the walk order itself).
-#pragma once
-
-namespace dfb
-{
-struct TraceJob
-{
-	long long ref_off;  // first byte of the reference in the raw pool
-	long long read_off; // first byte of the read in the raw pool
-	int R, L;
-	int reversed;       // 1: both sequences are consumed back to front (matrix 2)
-	int start_i, start_j;
-	long long bits_off;    // words; (L+1) rows of W = (R+16)/16 words
-	long long scratch_off; // ints; R+1 row-boundary values
-	long long match_off;   // pairs; capacity L
-};
-
-__device__ __forceinline__ int trace_ref_byte(const unsigned char* raw, const TraceJob& jb, int i) // i = 1..R
-{
-	return raw[jb.ref_off + (jb.reversed ? jb.R - i : i - 1)];
-}
-__device__ __forceinline__ int trace_read_byte(const unsigned char* raw, const TraceJob& jb, int j) // j = 1..L
-{
-	return raw[jb.read_off + (jb.reversed ? jb.L - j : j - 1)];
-}
-
-__global__ void __launch_bounds__(128) trace_fill_kernel(const unsigned char* __restrict__ raw, const TraceJob* __restrict__ jobs,
-                                                         int n_jobs, int match, int mismatch, int gap, int end_gaps,
-                                                         unsigned* __restrict__ bits, int* __restrict__ scratch)
-{
-	const int lane = threadIdx.x & 31;
-	const int warps = (gridDim.x * blockDim.x) >> 5;
-	for (int job = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; job < n_jobs; job += warps)
-	{
-		const TraceJob jb = jobs[job];
-		const int R = jb.R, L = jb.L;
-		const int W = (R + 16) >> 4;
-		unsigned* const my_bits = bits + jb.bits_off;
-		int* const edge = scratch + jb.scratch_off;
-		const int row0 = end_gaps ? 0 : gap; // H(0,j) = j * row0 (:44-48)
-		for (int tile = 0; tile < L; tile += 32)
-		{
-			const int j = tile + lane + 1;
-			const bool live = j <= L;
-			const int rc = live ? trace_read_byte(raw, jb, j) : -1;
-			int own = j * row0;        // H(i-1, j), starts at column 0
-			int diag = (j - 1) * row0; // H(i-1, j-1)
-			int cur = 0;               // H(i, j) just computed: what the lane below sees as H(i, j-1)
-			unsigned word = 0;
-			unsigned* const row_bits = my_bits + (long long)j * W;
-			const bool last_lane = lane == 31 && tile + 32 < L;
-			for (int s = 1; s <= R + 31; s++)
-			{
-				const int i = s - lane;
-				int above = __shfl_up_sync(0xffffffffu, cur, 1);
-				if (live && i >= 1 && i <= R)
-				{
-					if (lane == 0) above = tile == 0 ? 0 : edge[i]; // H(i, tile): row 0 is all zero (:40-43)
-					const int m = diag + (trace_ref_byte(raw, jb, i) == rc ? match : mismatch);
-					const int gr = own + gap;   // from (i-1, j)
-					const int gd = above + gap; // from (i, j-1)
-					const int mx = max(m, max(gr, gd));
-					const unsigned dir = gd == mx ? 2u : (gr == mx ? 1u : 0u);
-					word |= dir << (2 * (i & 15));
-					if ((i & 15) == 15 || i == R)
-					{
-						row_bits[i >> 4] = word;
-						word = 0;
-					}
-					diag = above;
-					own = mx;
-					cur = mx;
-					if (last_lane) edge[i] = mx;
-				}
-			}
-			__syncwarp();
-		}
-	}
-}
-
-__global__ void trace_walk_kernel(const TraceJob* __restrict__ jobs, int n_jobs, const unsigned* __restrict__ bits,
-                                  int2* __restrict__ matches, int* __restrict__ n_matches)
-{
-	const int job = blockIdx.x * blockDim.x + threadIdx.x;
-	if (job >= n_jobs) return;
-	const TraceJob jb = jobs[job];
-	const int W = (jb.R + 16) >> 4;
-	const unsigned* const my_bits = bits + jb.bits_off;
-	int2* out = matches + jb.match_off;
-	int i = jb.start_i, j = jb.start_j, n = 0;
-	while (j > 0)
-	{
-		// row i == 0 points along the read (:46-47)
-		const unsigned dir = i == 0 ? 2u : (my_bits[(long long)j * W + (i >> 4)] >> (2 * (i & 15))) & 3u;
-		if (dir == 0)
-		{
-			out[n++] = make_int2(i - 1, j - 1); // (refPos, readPos) of a diagonal step (:133-139)
-			i--;
-			j--;
-		}
-		else if (dir == 1)
-			i--;
-		else
-			j--;
-	}
-	n_matches[job] = n;
-}
-}  // namespace dfb
-
-// ------------------------------------------------------------------------------------------
-// host entry
-// ------------------------------------------------------------------------------------------
-
-extern "C" int dfb_split_backtrace_batch(dfb_ctx* ctx, const dfb_split_params* params, const dfb_seq_table* refs,
-                                         const dfb_seq_table* reads, const int32_t* task_cluster, const int32_t* task_read,
-                                         const int32_t* task_ref_split1, const int32_t* task_ref_split2,
-                                         const int32_t* task_read_split, int64_t n_tasks, int64_t* match_off,
-                                         int32_t* matches, int64_t matches_cap, int64_t* n_pairs_out)
-{
-	if (!ctx) return DFB_ERR_ARG;
-	if (!params || n_tasks < 0 || !match_off || !n_pairs_out ||
-	    (n_tasks > 0 && (!task_cluster || !task_read || !task_ref_split1 || !task_ref_split2 || !task_read_split)))
-		return set_err(ctx, DFB_ERR_ARG, "dfb_split_backtrace_batch: null argument");
-	int rc = check_table(ctx, refs, "refs");
-	if (rc) return rc;
-	rc = check_table(ctx, reads, "reads");
-	if (rc) return rc;
-	if (refs->n % 2) return set_err(ctx, DFB_ERR_ARG, "refs must hold two windows per cluster");
-	CK(ctx, cudaSetDevice(ctx->device));
-
-	// validate and size: the start cells of task t are (i1, a) in matrix 1 and (R2 - refSplit2 - 1, L - a) in matrix 2
-	match_off[0] = 0;
-	for (int64_t t = 0; t < n_tasks; t++)
-	{
-		const int64_t c = task_cluster[t], r = task_read[t];
-		if (c < 0 || 2 * c + 1 >= refs->n || r < 0 || r >= reads->n)
-			return set_err(ctx, DFB_ERR_ARG, "task %lld: index out of range", (long long)t);
-		const int64_t R1 = refs->off[2 * c + 1] - refs->off[2 * c], R2 = refs->off[2 * c + 2] - refs->off[2 * c + 1];
-		const int64_t L = reads->off[r + 1] - reads->off[r];
-		const int64_t a = task_read_split[t], i1 = task_ref_split1[t], i2 = R2 - (int64_t)task_ref_split2[t] - 1;
-		if (a < 0 || a > L || i1 < 0 || i1 > R1 || i2 < 0 || i2 > R2)
-			return set_err(ctx, DFB_ERR_ARG, "task %lld: start cell outside the matrices", (long long)t);
-		match_off[2 * t + 1] = match_off[2 * t] + a;       // a diagonal step consumes one read base
-		match_off[2 * t + 2] = match_off[2 * t + 1] + (L - a);
-	}
-	// (match_off holds capacities for now; it is compacted to the real counts below)
-	const int64_t cap_pairs = match_off[2 * n_tasks];
-	std::vector<int64_t> cap_off(match_off, match_off + 2 * n_tasks + 1);
-
-	// chunks bounded by pointer-matrix memory
-	const size_t kMaxBitsWords = (size_t)1 << 28; // 1 GiB of pointer words per chunk
-	std::vector<TraceJob> jobs;
-	std::vector<int2> h_pairs;
-	std::vector<int> h_cnt;
-	std::vector<int64_t> counts((size_t)(2 * n_tasks), 0);
-	std::vector<int2> all_pairs((size_t)cap_pairs);
-	const int64_t raw_ref = refs->off[refs->n], raw_read = reads->off[reads->n];
-	unsigned char* d_raw = nullptr;
-	cudaStream_t st = ctx->stream;
-	CK(ctx, cudaMallocAsync((void**)&d_raw, (size_t)(raw_ref + raw_read + 16), st));
-	auto fail = [&](int code) {
-		cudaStreamSynchronize(st);
-		cudaFreeAsync(d_raw, st);
-		return code;
-	};
-	cudaError_t e = cudaSuccess;
-	if (raw_ref) e = cudaMemcpyAsync(d_raw, refs->bytes, (size_t)raw_ref, cudaMemcpyHostToDevice, st);
-	if (e == cudaSuccess && raw_read) e = cudaMemcpyAsync(d_raw + raw_ref, reads->bytes, (size_t)raw_read, cudaMemcpyHostToDevice, st);
-	if (e != cudaSuccess) return fail(set_err(ctx, DFB_ERR_CUDA, "upload failed: %s", cudaGetErrorString(e)));
-
-	for (int64_t first = 0; first < n_tasks;)
-	{
-		jobs.clear();
-		size_t words = 0, scratch = 0, pairs = 0;
-		int64_t last = first;
-		for (; last < n_tasks; last++)
-		{
-			const int64_t c = task_cluster[last], r = task_read[last];
-			const int64_t R1 = refs->off[2 * c + 1] - refs->off[2 * c], R2 = refs->off[2 * c + 2] - refs->off[2 * c + 1];
-			const int64_t L = reads->off[r + 1] - reads->off[r];
-			const size_t w1 = (size_t)(L + 1) * (size_t)((R1 + 16) >> 4), w2 = (size_t)(L + 1) * (size_t)((R2 + 16) >> 4);
-			if (!jobs.empty() && words + w1 + w2 > kMaxBitsWords) break;
-			const int a = task_read_split[last];
-			TraceJob j1{refs->off[2 * c], raw_ref + reads->off[r], (int)R1, (int)L, 0, task_ref_split1[last], a,
-			            (long long)words, (long long)scratch, (long long)pairs};
-			words += w1;
-			scratch += (size_t)R1 + 1;
-			pairs += (size_t)a;
-			TraceJob j2{refs->off[2 * c + 1], raw_ref + reads->off[r], (int)R2, (int)L, 1,
-			            (int)(R2 - task_ref_split2[last] - 1), (int)(L - a), (long long)words, (long long)scratch, (long long)pairs};
-			words += w2;
-			scratch += (size_t)R2 + 1;
-			pairs += (size_t)(L - a);
-			jobs.push_back(j1);
-			jobs.push_back(j2);
-		}
-		const int n_jobs = (int)jobs.size();
-		TraceJob* d_jobs = nullptr;
-		unsigned* d_bits = nullptr;
-		int* d_scratch = nullptr;
-		int2* d_pairs = nullptr;
-		int* d_cnt = nullptr;
-		if ((e = cudaMallocAsync((void**)&d_jobs, sizeof(TraceJob) * (size_t)n_jobs, st)) != cudaSuccess ||
-		    (e = cudaMallocAsync((void**)&d_bits, sizeof(unsigned) * (words + 1), st)) != cudaSuccess ||
-		    (e = cudaMallocAsync((void**)&d_scratch, sizeof(int) * (scratch + 1), st)) != cudaSuccess ||
-		    (e = cudaMallocAsync((void**)&d_pairs, sizeof(int2) * (pairs + 1), st)) != cudaSuccess ||
-		    (e = cudaMallocAsync((void**)&d_cnt, sizeof(int) * (size_t)n_jobs, st)) != cudaSuccess)
-		{
-			// (blocks already taken go back to the pool with the stream)
-			if (d_jobs) cudaFreeAsync(d_jobs, st);
-			if (d_bits) cudaFreeAsync(d_bits, st);
-			if (d_scratch) cudaFreeAsync(d_scratch, st);
-			if (d_pairs) cudaFreeAsync(d_pairs, st);
-			return fail(set_err(ctx, DFB_ERR_NOMEM, "device allocation failed: %s", cudaGetErrorString(e)));
-		}
-		h_pairs.resize(pairs + 1);
-		h_cnt.resize((size_t)n_jobs);
-		e = cudaMemcpyAsync(d_jobs, jobs.data(), sizeof(TraceJob) * (size_t)n_jobs, cudaMemcpyHostToDevice, st);
-		if (e == cudaSuccess)
-		{
-			const int warps_per_block = 4;
-			const int grid = std::max(1, std::min((n_jobs + warps_per_block - 1) / warps_per_block, ctx->prop.multiProcessorCount * 8));
-			trace_fill_kernel<<<grid, 32 * warps_per_block, 0, st>>>(d_raw, d_jobs, n_jobs, params->match, params->mismatch,
-			                                                         params->gap, params->end_gaps, d_bits, d_scratch);
-			trace_walk_kernel<<<(n_jobs + 63) / 64, 64, 0, st>>>(d_jobs, n_jobs, d_bits, d_pairs, d_cnt);
-			e = cudaGetLastError();
-		}
-		if (e == cudaSuccess) e = cudaMemcpyAsync(h_pairs.data(), d_pairs, sizeof(int2) * pairs, cudaMemcpyDeviceToHost, st);
-		if (e == cudaSuccess) e = cudaMemcpyAsync(h_cnt.data(), d_cnt, sizeof(int) * (size_t)n_jobs, cudaMemcpyDeviceToHost, st);
-		if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-		cudaFreeAsync(d_jobs, st);
-		cudaFreeAsync(d_bits, st);
-		cudaFreeAsync(d_scratch, st);
-		cudaFreeAsync(d_pairs, st);
-		cudaFreeAsync(d_cnt, st);
-		if (e != cudaSuccess) return fail(set_err(ctx, DFB_ERR_CUDA, "backtrace kernels failed: %s", cudaGetErrorString(e)));
-		for (int k = 0; k < n_jobs; k++)
-		{
-			const int64_t t = first + k / 2;
-			const int half = k & 1;
-			const TraceJob& jb = jobs[(size_t)k];
-			const int n = h_cnt[(size_t)k];
-			counts[(size_t)(2 * t + half)] = n;
-			int2* dst = all_pairs.data() + cap_off[(size_t)(2 * t + half)];
-			const int2* src = h_pairs.data() + jb.match_off;
-			if (!half)
-				for (int q = 0; q < n; q++) dst[q] = src[n - 1 - q]; // BackTracePath's reverse (:142)
-			else
-				for (int q = 0; q < n; q++) dst[q] = make_int2(jb.R - src[q].x - 1, jb.L - src[q].y - 1); // ReverseMatches (:145-154)
-		}
-		first = last;
-	}
-	cudaFreeAsync(d_raw, st);
-
-	// compact: real counts instead of capacities
-	int64_t total = 0;
-	for (int64_t k = 0; k < 2 * n_tasks; k++)
-	{
-		match_off[k] = total;
-		total += counts[(size_t)k];
-	}
-	match_off[2 * n_tasks] = total;
-	*n_pairs_out = total;
-	if (matches)
-	{
-		if (matches_cap < total) return set_err(ctx, DFB_ERR_ARG, "matches buffer holds %lld pairs, %lld needed", (long long)matches_cap, (long long)total);
-		for (int64_t k = 0; k < 2 * n_tasks; k++)
-		{
-			const int2* src = all_pairs.data() + cap_off[(size_t)k];
-			int32_t* dst = matches + 2 * match_off[k];
-			for (int64_t q = 0; q < counts[(size_t)k]; q++)
-			{
-				dst[2 * q] = src[q].x;
-				dst[2 * q + 1] = src[q].y;
-			}
-		}
-	}
-	return DFB_OK;
-}
-
-// ------------------------------------------------------------------------------------------
-// device-resident form: dfb_split_backtrace_device
-// ------------------------------------------------------------------------------------------
+// Included at the end of dfb_api.cu (it needs dfb_ctx).  Exact over every parameter set (s32 arithmetic, raw byte
+// equality, any length).  One path serves both entry points: dfb_split_backtrace_device takes records in device memory,
+// dfb_split_backtrace_batch checks its host arrays, uploads them with one record per alignment and copies the result back.
 //
 // Record k names one alignment of task t = records[k].task: start cell (ref_split1, read_split1) in matrix 1 and
-// (len(ref2) - ref_split2 - 1, len(read) - read_split1) in matrix 2.  Cell (i, j) depends only on cells up and to the
-// left, so the pointers every record of a group of same-task records needs are those of the bounding box of its start
-// cells -- rows 0..max j, columns 0..max i of each matrix -- filled with trace_fill_kernel's arithmetic and pointer rule.
+// (len(ref2) - ref_split2 - 1, len(read) - read_split1) in matrix 2 (matrix 2 is rev(read) x rev(ref2)).  Cell (i, j)
+// depends only on cells up and to the left, so the pointers every record of a group of same-task records needs are those
+// of the bounding box of its start cells -- rows 0..max j, columns 0..max i of each matrix.
 //
 //   bt_records_kernel   per record: argument checks, piece heads, capacity len(read)
 //   bt_pieces_kernel    per record: the first record of each piece
@@ -312,6 +20,8 @@ extern "C" int dfb_split_backtrace_batch(dfb_ctx* ctx, const dfb_split_params* p
 //
 // A piece is a run of consecutive records of one task, also cut where k is a multiple of the run cap, so that one
 // heavy task (poly-A: 467 k records) spreads over many blocks; each piece fills its boxes once.
+#pragma once
+
 #define DFB_BT_THREADS 128
 #define DFB_BT_RUN_CAP 256                      // records per piece at most (DESIGN.md 4.5b: the measurement)
 #define DFB_BT_SMEM_BYTES (96 << 10)            // pieces whose boxes fit take the shared-memory kernel
@@ -469,8 +179,10 @@ __global__ void __launch_bounds__(DFB_BUILD_BLOCK) bt_box_kernel(const dfb_split
 	}
 }
 
-// H over rows 1..J (read) and columns 1..I (reference) of one matrix, by one warp: trace_fill_kernel's wavefront, s32
-// arithmetic and pointer rule on the top-left corner of the matrix; the pointer of (i, j) goes to bits[(j - 1) W + i / 16]
+// H over rows 1..J (read) and columns 1..I (reference) of one matrix -- its top-left corner -- by one warp: lane l owns read
+// row j = tile + l + 1 and sweeps the reference as a skewed wavefront (the geometry of the s32 DP kernel), in s32.  The
+// pointer of (i, j), 2 bits packed 16 columns per word, goes to bits[(j - 1) W + i / 16]: 0 diagonal, 1 (i-1,j),
+// 2 (i,j-1); later writers win, so 2 > 1 > 0 (:56-69)
 __device__ __forceinline__ void bt_fill(const unsigned char* __restrict__ ref, const unsigned char* __restrict__ read, int R, int L,
                                         bool reversed, int I, int J, unsigned* bits, int* edge, int match, int mismatch, int gap, int row0)
 {
@@ -602,30 +314,20 @@ __global__ void __launch_bounds__(DFB_BUILD_BLOCK) bt_compact_kernel(BtWalk p, l
 }
 }  // namespace dfb
 
-static int dfb_split_backtrace_device_body(dfb_ctx* ctx, const dfb_split_params* params, const dfb_device_seq_table* refs,
-                                           const dfb_device_seq_table* reads, const int32_t* task_cluster, const int32_t* task_read,
-                                           int64_t n_tasks, const dfb_split_record* records, int64_t n_records, int64_t* n_pairs)
+static void bt_free(dfb_ctx* ctx, BtResult& r)
+{
+	dfree(ctx, r.d_off);
+	for (auto& c : r.chunks) dfree(ctx, c.first);
+	r = BtResult();
+}
+
+// The work of both entry points, on arguments whose pointers and sizes the caller has checked; *res receives the result
+// (and is left as it was on failure).  The checks of the tables, task arrays and records run here, on the device.
+static int bt_run(dfb_ctx* ctx, const dfb_split_params* params, const dfb_device_seq_table* refs, const dfb_device_seq_table* reads,
+                  const int32_t* task_cluster, const int32_t* task_read, int64_t n_tasks, const dfb_split_record* records,
+                  int64_t n_records, BtResult* res)
 {
 	using namespace dfb;
-	if (!ctx) return DFB_ERR_ARG;
-	ctx->has_bt = false;
-	ctx->n_bt_records = ctx->n_bt_pairs = 0;
-	dfree(ctx, ctx->d_bt_off);
-	for (auto& c : ctx->bt_chunks) dfree(ctx, c.first);
-	ctx->bt_chunks.clear();
-	if (!params || !n_pairs || n_tasks < 0 || n_records < 0 || (n_tasks > 0 && (!task_cluster || !task_read)) || (n_records > 0 && !records))
-		return set_err(ctx, DFB_ERR_ARG, "dfb_split_backtrace_device: null argument");
-	const char* names[2] = {"refs", "reads"};
-	const dfb_device_seq_table* tabs[2] = {refs, reads};
-	for (int k = 0; k < 2; k++)
-		if (!tabs[k] || !tabs[k]->off || tabs[k]->n < 0 || tabs[k]->n_bytes < 0) return set_err(ctx, DFB_ERR_ARG, "%s: null table", names[k]);
-	CK(ctx, cudaSetDevice(ctx->device));
-	const void* ptrs[7] = {refs->bytes, refs->off, reads->bytes, reads->off, task_cluster, task_read, records};
-	const char* what[7] = {"refs->bytes", "refs->off", "reads->bytes", "reads->off", "task_cluster", "task_read", "records"};
-	for (int k = 0; k < 7; k++)
-		if (!is_ctx_device_memory(ctx, ptrs[k]))
-			return set_err(ctx, DFB_ERR_ARG, "%s is not device memory of device %d", what[k], ctx->device);
-	if (n_tasks > 0x7fffff00LL) return set_err(ctx, DFB_ERR_ARG, "too many tasks in one batch");
 	int run_cap = DFB_BT_RUN_CAP;
 	if (const char* e = getenv("DFB_BT_RUN_CAP")) // (measurement: DESIGN.md 4.5b)
 		if (atoi(e) > 0) run_cap = atoi(e);
@@ -780,14 +482,12 @@ static int dfb_split_backtrace_device_body(dfb_ctx* ctx, const dfb_split_params*
 	if (e == cudaSuccess) e = cudaStreamSynchronize(s);
 	if (e != cudaSuccess) return fail(set_err(ctx, DFB_ERR_CUDA, "backtrace: %s", cudaGetErrorString(e)));
 	if (int rc = bounds_check_status(ctx)) return fail(rc);
-	ctx->d_bt_off = (int64_t*)cnt;
+	res->d_off = (int64_t*)cnt;
 	cnt = nullptr;
-	ctx->bt_chunks.swap(chunks);
+	res->chunks.swap(chunks);
 	cleanup();
-	ctx->n_bt_records = n;
-	ctx->n_bt_pairs = total;
-	ctx->has_bt = true;
-	*n_pairs = (int64_t)total;
+	res->n_records = n;
+	res->n_pairs = total;
 	return DFB_OK;
 }
 
@@ -795,8 +495,25 @@ extern "C" int dfb_split_backtrace_device(dfb_ctx* ctx, const dfb_split_params* 
                                           const dfb_device_seq_table* reads, const int32_t* task_cluster, const int32_t* task_read,
                                           int64_t n_tasks, const dfb_split_record* records, int64_t n_records, int64_t* n_pairs)
 {
-	return guarded(ctx, [&] {
-		return dfb_split_backtrace_device_body(ctx, params, refs, reads, task_cluster, task_read, n_tasks, records, n_records, n_pairs);
+	return guarded(ctx, [&]() -> int {
+		if (!ctx) return DFB_ERR_ARG;
+		bt_free(ctx, ctx->bt);
+		if (!params || !n_pairs || n_tasks < 0 || n_records < 0 || (n_tasks > 0 && (!task_cluster || !task_read)) || (n_records > 0 && !records))
+			return set_err(ctx, DFB_ERR_ARG, "dfb_split_backtrace_device: null argument");
+		const char* names[2] = {"refs", "reads"};
+		const dfb_device_seq_table* tabs[2] = {refs, reads};
+		for (int k = 0; k < 2; k++)
+			if (!tabs[k] || !tabs[k]->off || tabs[k]->n < 0 || tabs[k]->n_bytes < 0) return set_err(ctx, DFB_ERR_ARG, "%s: null table", names[k]);
+		CK(ctx, cudaSetDevice(ctx->device));
+		const void* ptrs[7] = {refs->bytes, refs->off, reads->bytes, reads->off, task_cluster, task_read, records};
+		const char* what[7] = {"refs->bytes", "refs->off", "reads->bytes", "reads->off", "task_cluster", "task_read", "records"};
+		for (int k = 0; k < 7; k++)
+			if (!is_ctx_device_memory(ctx, ptrs[k]))
+				return set_err(ctx, DFB_ERR_ARG, "%s is not device memory of device %d", what[k], ctx->device);
+		if (n_tasks > 0x7fffff00LL) return set_err(ctx, DFB_ERR_ARG, "too many tasks in one batch");
+		if (int rc = bt_run(ctx, params, refs, reads, task_cluster, task_read, n_tasks, records, n_records, &ctx->bt)) return rc;
+		*n_pairs = ctx->bt.n_pairs;
+		return DFB_OK;
 	});
 }
 
@@ -804,19 +521,115 @@ extern "C" int dfb_split_backtrace_copy_device(dfb_ctx* ctx, int64_t* match_off,
 {
 	return guarded(ctx, [&]() -> int {
 		if (!ctx) return DFB_ERR_ARG;
-		if (!ctx->has_bt) return set_err(ctx, DFB_ERR_STATE, "no backtrace on this context: call dfb_split_backtrace_device first");
-		if (!match_off || (ctx->n_bt_pairs && !matches)) return set_err(ctx, DFB_ERR_ARG, "dfb_split_backtrace_copy_device: null argument");
+		const BtResult& bt = ctx->bt;
+		if (!bt.d_off) return set_err(ctx, DFB_ERR_STATE, "no backtrace on this context: call dfb_split_backtrace_device first");
+		if (!match_off || (bt.n_pairs && !matches)) return set_err(ctx, DFB_ERR_ARG, "dfb_split_backtrace_copy_device: null argument");
 		CK(ctx, cudaSetDevice(ctx->device));
 		if (!is_ctx_device_memory(ctx, match_off)) return set_err(ctx, DFB_ERR_ARG, "match_off is not device memory of device %d", ctx->device);
 		if (!is_ctx_device_memory(ctx, matches)) return set_err(ctx, DFB_ERR_ARG, "matches is not device memory of device %d", ctx->device);
-		CK(ctx, cudaMemcpyAsync(match_off, ctx->d_bt_off, (size_t)(2 * ctx->n_bt_records + 1) * 8, cudaMemcpyDeviceToDevice, ctx->stream));
+		CK(ctx, cudaMemcpyAsync(match_off, bt.d_off, (size_t)(2 * bt.n_records + 1) * 8, cudaMemcpyDeviceToDevice, ctx->stream));
 		int64_t at = 0;
-		for (const auto& c : ctx->bt_chunks)
+		for (const auto& c : bt.chunks)
 		{
 			CK(ctx, cudaMemcpyAsync(matches + 2 * at, c.first, (size_t)c.second * sizeof(int2), cudaMemcpyDeviceToDevice, ctx->stream));
 			at += c.second;
 		}
 		CK(ctx, cudaStreamSynchronize(ctx->stream));
 		return DFB_OK;
+	});
+}
+
+// The host form: the arguments are checked on the host, the tables, task arrays and one record per alignment are
+// uploaded, and the result of bt_run comes back to the caller's arrays.  Nothing stays allocated, and the context's
+// dfb_split_backtrace_device result is not touched.
+extern "C" int dfb_split_backtrace_batch(dfb_ctx* ctx, const dfb_split_params* params, const dfb_seq_table* refs,
+                                         const dfb_seq_table* reads, const int32_t* task_cluster, const int32_t* task_read,
+                                         const int32_t* task_ref_split1, const int32_t* task_ref_split2,
+                                         const int32_t* task_read_split, int64_t n_tasks, int64_t* match_off,
+                                         int32_t* matches, int64_t matches_cap, int64_t* n_pairs_out)
+{
+	return guarded(ctx, [&]() -> int {
+		if (!ctx) return DFB_ERR_ARG;
+		if (!params || n_tasks < 0 || !match_off || !n_pairs_out ||
+		    (n_tasks > 0 && (!task_cluster || !task_read || !task_ref_split1 || !task_ref_split2 || !task_read_split)))
+			return set_err(ctx, DFB_ERR_ARG, "dfb_split_backtrace_batch: null argument");
+		int rc = check_table(ctx, refs, "refs");
+		if (rc) return rc;
+		rc = check_table(ctx, reads, "reads");
+		if (rc) return rc;
+		if (refs->n % 2) return set_err(ctx, DFB_ERR_ARG, "refs must hold two windows per cluster");
+		if (n_tasks > 0x7fffff00LL) return set_err(ctx, DFB_ERR_ARG, "too many tasks in one batch");
+		CK(ctx, cudaSetDevice(ctx->device));
+
+		// the start cells of task t are (i1, a) in matrix 1 and (R2 - refSplit2 - 1, L - a) in matrix 2
+		std::vector<dfb_split_record> rec((size_t)n_tasks);
+		for (int64_t t = 0; t < n_tasks; t++)
+		{
+			const int64_t c = task_cluster[t], r = task_read[t];
+			if (c < 0 || 2 * c + 1 >= refs->n || r < 0 || r >= reads->n)
+				return set_err(ctx, DFB_ERR_ARG, "task %lld: index out of range", (long long)t);
+			const int64_t R1 = refs->off[2 * c + 1] - refs->off[2 * c], R2 = refs->off[2 * c + 2] - refs->off[2 * c + 1];
+			const int64_t L = reads->off[r + 1] - reads->off[r];
+			const int64_t a = task_read_split[t], i1 = task_ref_split1[t], i2 = R2 - (int64_t)task_ref_split2[t] - 1;
+			if (a < 0 || a > L || i1 < 0 || i1 > R1 || i2 < 0 || i2 > R2)
+				return set_err(ctx, DFB_ERR_ARG, "task %lld: start cell outside the matrices", (long long)t);
+			rec[(size_t)t] = dfb_split_record{(int32_t)t, task_ref_split1[t], task_ref_split2[t], (int32_t)a, (int32_t)(L - a), 0};
+		}
+
+		cudaStream_t s = ctx->stream;
+		uint8_t* d_bytes[2] = {nullptr, nullptr};
+		int64_t* d_off[2] = {nullptr, nullptr};
+		int32_t *d_tc = nullptr, *d_tr = nullptr;
+		dfb_split_record* d_rec = nullptr;
+		BtResult res;
+		auto done = [&](int code) {
+			for (int k = 0; k < 2; k++)
+			{
+				dfree(ctx, d_bytes[k]);
+				dfree(ctx, d_off[k]);
+			}
+			dfree(ctx, d_tc);
+			dfree(ctx, d_tr);
+			dfree(ctx, d_rec);
+			bt_free(ctx, res);
+			cudaStreamSynchronize(s);
+			return code;
+		};
+		cudaError_t e = cudaSuccess;
+		auto upload = [&](void** d, const void* h, size_t bytes) {
+			if (e == cudaSuccess) e = dalloc(ctx, d, bytes);
+			if (e == cudaSuccess && bytes) e = cudaMemcpyAsync(*d, h, bytes, cudaMemcpyHostToDevice, s);
+		};
+		const dfb_seq_table* tabs[2] = {refs, reads};
+		dfb_device_seq_table dt[2];
+		for (int k = 0; k < 2; k++)
+		{
+			const int64_t nb = tabs[k]->off[tabs[k]->n];
+			upload((void**)&d_bytes[k], tabs[k]->bytes, (size_t)nb);
+			upload((void**)&d_off[k], tabs[k]->off, (size_t)(tabs[k]->n + 1) * 8);
+			dt[k] = dfb_device_seq_table{d_bytes[k], d_off[k], tabs[k]->n, nb};
+		}
+		upload((void**)&d_tc, task_cluster, (size_t)n_tasks * 4);
+		upload((void**)&d_tr, task_read, (size_t)n_tasks * 4);
+		upload((void**)&d_rec, rec.data(), (size_t)n_tasks * sizeof(dfb_split_record));
+		if (e != cudaSuccess)
+			return done(set_err(ctx, e == cudaErrorMemoryAllocation ? DFB_ERR_NOMEM : DFB_ERR_CUDA, "backtrace upload: %s", cudaGetErrorString(e)));
+
+		if ((rc = bt_run(ctx, params, &dt[0], &dt[1], d_tc, d_tr, n_tasks, d_rec, n_tasks, &res))) return done(rc);
+		const bool fits = !matches || matches_cap >= res.n_pairs;
+		e = cudaMemcpyAsync(match_off, res.d_off, (size_t)(2 * n_tasks + 1) * 8, cudaMemcpyDeviceToHost, s);
+		int64_t at = 0;
+		for (const auto& c : res.chunks)
+		{
+			if (e != cudaSuccess || !matches || !fits) break;
+			e = cudaMemcpyAsync(matches + 2 * at, c.first, (size_t)c.second * sizeof(int2), cudaMemcpyDeviceToHost, s);
+			at += c.second;
+		}
+		if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+		if (e != cudaSuccess) return done(set_err(ctx, DFB_ERR_CUDA, "backtrace copy: %s", cudaGetErrorString(e)));
+		*n_pairs_out = res.n_pairs;
+		if (!fits)
+			return done(set_err(ctx, DFB_ERR_ARG, "matches buffer holds %lld pairs, %lld needed", (long long)matches_cap, (long long)res.n_pairs));
+		return done(DFB_OK);
 	});
 }

@@ -277,8 +277,13 @@ DFB_API int dfb_split_records_copy_device(dfb_ctx* ctx, dfb_split_record* d_reco
  *   match_off : 2*n_tasks + 1 entries; pairs [match_off[2t], match_off[2t+1]) are matches1 of task t,
  *               [match_off[2t+1], match_off[2t+2]) its matches2
  *   matches   : interleaved (refPos, readPos); at most sum(len(read)) pairs are produced, so a buffer of
- *               2 * sum(len(read)) int32 always suffices (matches_cap counts pairs); NULL only sizes
- *   n_pairs   : total number of pairs */
+ *               2 * sum(len(read)) int32 always suffices (matches_cap counts pairs); NULL only sizes; a matches_cap
+ *               below the total is DFB_ERR_ARG, with match_off and n_pairs written and matches untouched
+ *   n_pairs   : total number of pairs
+ * The arguments are checked on the host; the tables, task arrays and one dfb_split_record per alignment are then
+ * uploaded and the kernels of dfb_split_backtrace_device run on them.  Nothing stays allocated after the call, and the
+ * context's dfb_split_backtrace_device result is left as it was.  At most 0x7fffff00 alignments per call (records
+ * carry an int32 task index); more is DFB_ERR_ARG "too many tasks in one batch". */
 DFB_API int dfb_split_backtrace_batch(dfb_ctx* ctx, const dfb_split_params* params,
                           const dfb_seq_table* refs, const dfb_seq_table* reads,
                           const int32_t* task_cluster, const int32_t* task_read,

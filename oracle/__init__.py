@@ -11,6 +11,7 @@ Two implementations of the same per-task interface:
 import ctypes
 import os
 import subprocess
+from concurrent.futures import ThreadPoolExecutor
 
 import numpy as np
 
@@ -71,6 +72,9 @@ def _lib(impl):
         lib.dpo_split_align_batch.restype = ctypes.c_int64
         lib.dpo_split_backtrace.argtypes = ([_c_u8p, ctypes.c_int] * 3 + [ctypes.c_int] * 7 + [_c_i32p] * 4)
         lib.dpo_split_backtrace.restype = None
+        lib.dpo_split_backtrace_batch.argtypes = ([ctypes.c_int] * 4 + [_c_u8p, _c_i64p, _c_u8p, _c_i64p] + [_c_i32p] * 5 +
+                                                  [ctypes.c_int64] * 2 + [_c_i64p, _c_i32p])
+        lib.dpo_split_backtrace_batch.restype = ctypes.c_int64
     elif impl == "ref":
         if not os.path.exists(REF_LIB):
             raise FileNotFoundError("oracle/_ref/libref_aligners.so not built (run `make -C oracle ref` where /root/reference exists)")
@@ -303,3 +307,39 @@ def split_align_batch(ref_bytes, ref_off, read_bytes, read_off, task_cluster, ta
         if total <= cap:
             return cnt, out[:total].copy()
         cap = int(total)
+
+
+def split_backtrace_batch(refs, reads, task_cluster, task_read, ref_split1, ref_split2, read_split, params=(2, -1, -2, False),
+                          threads=None):
+    """split_backtrace for every alignment of a batch, in the layout of dfb_split_backtrace_batch (port).  refs / reads
+    are CSR tables (`.data` bytes, `.off` n+1 offsets; cluster c owns windows 2c and 2c+1); alignment t is
+    reads[task_read[t]] against cluster task_cluster[t] with refSplit (ref_split1[t], ref_split2[t]) and readSplit.first
+    read_split[t]; params starts with (match, mismatch, gap, end_gaps).  Returns (match_off[2n+1] int64, pairs[(total,2)]
+    int32).  The alignments are spread over threads (ctypes releases the GIL)."""
+    m, x, g, eg = params[:4]
+    lib = _lib("port")
+    rb, sb = _u8(refs.data), _u8(reads.data)
+    ro = np.ascontiguousarray(refs.off, dtype=np.int64)
+    so = np.ascontiguousarray(reads.off, dtype=np.int64)
+    arrs = [np.ascontiguousarray(a, dtype=np.int32) for a in (task_cluster, task_read, ref_split1, ref_split2, read_split)]
+    n = len(arrs[0])
+    assert all(len(a) == n for a in arrs)
+    off = np.zeros(2 * n + 1, dtype=np.int64)
+    threads = threads or min(32, os.cpu_count() or 1)
+    bounds = np.linspace(0, n, min(threads, max(n, 1)) + 1).astype(np.int64)
+    lengths = (so[1:] - so[:-1])[arrs[1]] if n else np.zeros(0, np.int64)
+
+    def run(k):
+        t0, t1 = int(bounds[k]), int(bounds[k + 1])
+        pairs = np.zeros((max(int(lengths[t0:t1].sum()), 1), 2), dtype=np.int32)
+        got = lib.dpo_split_backtrace_batch(m, x, g, int(eg), _p(rb, _c_u8p), _p(ro, _c_i64p), _p(sb, _c_u8p), _p(so, _c_i64p),
+                                            *[_p(a, _c_i32p) for a in arrs], t0, t1, _p(off, _c_i64p), _p(pairs, _c_i32p))
+        return pairs[:got]
+
+    with ThreadPoolExecutor(len(bounds) - 1) as ex:
+        parts = list(ex.map(run, range(len(bounds) - 1)))
+    base = 0
+    for k, part in enumerate(parts):   # ranges count from their own start
+        off[2 * bounds[k] + 1:2 * bounds[k + 1] + 1] += base
+        base += len(part)
+    return off, np.concatenate(parts)

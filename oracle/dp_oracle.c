@@ -404,3 +404,34 @@ DPO_API void dpo_split_backtrace(const uint8_t* read, int L, const uint8_t* ref1
 	free(ref2r);
 	free(readr);
 }
+
+/* dpo_split_backtrace over alignments [t0, t1) of a batch, in the layout of dfb_split_backtrace_batch: alignment t
+ * of reads[task_read[t]] against cluster task_cluster[t] (windows 2c and 2c+1).  match_off[2t+1] and match_off[2t+2]
+ * receive the ends of its matches1 and matches2, counted from pairs of the range, which holds 2 * sum(len(read)) ints;
+ * match_off[2 * t0] is left to the caller.  Returns the number of pairs written. */
+DPO_API int64_t dpo_split_backtrace_batch(int match, int mismatch, int gap, int end_gaps,
+                                          const uint8_t* ref_bytes, const int64_t* ref_off,
+                                          const uint8_t* read_bytes, const int64_t* read_off,
+                                          const int32_t* task_cluster, const int32_t* task_read,
+                                          const int32_t* ref_split1, const int32_t* ref_split2,
+                                          const int32_t* read_split, int64_t t0, int64_t t1,
+                                          int64_t* match_off, int32_t* pairs)
+{
+	int64_t total = 0;
+	for (int64_t t = t0; t < t1; t++)
+	{
+		int c = task_cluster[t], r = task_read[t];
+		int L = (int)(read_off[r + 1] - read_off[r]);
+		int32_t* m2 = (int32_t*)malloc(sizeof(int32_t) * 2 * ((size_t)L + 1));
+		int32_t n1 = 0, n2 = 0;
+		dpo_split_backtrace(read_bytes + read_off[r], L, ref_bytes + ref_off[2 * c], (int)(ref_off[2 * c + 1] - ref_off[2 * c]),
+		                    ref_bytes + ref_off[2 * c + 1], (int)(ref_off[2 * c + 2] - ref_off[2 * c + 1]), match, mismatch,
+		                    gap, end_gaps, ref_split1[t], ref_split2[t], read_split[t], pairs + 2 * total, &n1, m2, &n2);
+		memcpy(pairs + 2 * (total + n1), m2, sizeof(int32_t) * 2 * (size_t)n2);
+		free(m2);
+		match_off[2 * t + 1] = total + n1;
+		match_off[2 * t + 2] = total + n1 + n2;
+		total += n1 + n2;
+	}
+	return total;
+}

@@ -1,5 +1,5 @@
 """DeviceSplitResult.backtrace() (dfb_split_backtrace_device) per workload: records, runs (consecutive records of one
-task), pieces, filled box cells against the full-matrix cells the host form fills, pairs out, the time of the backtrace
+task), pieces, filled box cells against the cells of both full matrices, pairs out, the time of the backtrace
 call next to align_device and records() of the same batch, peak pool memory of the backtrace call, a sweep of the run
 cap, and what a caller had before it -- to_host() plus SplitReadAligner.backtrace_batch on host arrays -- timed once.
 

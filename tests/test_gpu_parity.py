@@ -432,16 +432,10 @@ def test_pipelined_one_call_path(oracle_mod, gpu_ctx, monkeypatch):
 # backtrace: GetAlignments(..., backtrace=true) -- dfb_split_backtrace_batch against the oracle
 # ---------------------------------------------------------------------------------------------
 
-def _check_backtrace(oracle, ctx, refs, reads, task_cluster, task_read, min_score, params=(2, -1, -2, False, 8), per_task=4):
-    import defuse_b200 as d
+def _backtrace_vs_oracle(oracle, al, refs, reads, tc, trd, s1, s2, a):
+    """backtrace_batch of the alignments against the oracle's backtrace of each"""
     rt, st = _tables(refs, reads)
-    m, x, g, eg, ms = params
-    al = d.SplitReadAligner(m, x, g, eg, ms, ctx=ctx)
-    res = al.align_batch(rt, st, task_cluster, task_read, min_score)
-    tc, trd, s1, s2, a = [], [], [], [], []
-    for t in range(len(task_cluster)):
-        for row in res.alignments(t)[:per_task]:
-            tc.append(task_cluster[t]); trd.append(task_read[t]); s1.append(row[0]); s2.append(row[1]); a.append(row[2])
+    m, x, g, eg = al.params.match, al.params.mismatch, al.params.gap, bool(al.params.end_gaps)
     off, pairs = al.backtrace_batch(rt, st, tc, trd, s1, s2, a)
     assert off[0] == 0 and off[-1] == len(pairs) and (np.diff(off) >= 0).all()
     for k in range(len(tc)):
@@ -449,6 +443,19 @@ def _check_backtrace(oracle, ctx, refs, reads, task_cluster, task_read, min_scor
         g1, g2 = pairs[off[2 * k]:off[2 * k + 1]], pairs[off[2 * k + 1]:off[2 * k + 2]]
         assert g1.shape == w1.shape and (g1 == w1).all(), "alignment %d matches1: got\n%s\nwant\n%s" % (k, g1[:6], w1[:6])
         assert g2.shape == w2.shape and (g2 == w2).all(), "alignment %d matches2: got\n%s\nwant\n%s" % (k, g2[:6], w2[:6])
+    return off, pairs
+
+
+def _check_backtrace(oracle, ctx, refs, reads, task_cluster, task_read, min_score, params=(2, -1, -2, False, 8), per_task=4):
+    import defuse_b200 as d
+    rt, st = _tables(refs, reads)
+    al = d.SplitReadAligner(*params, ctx=ctx)
+    res = al.align_batch(rt, st, task_cluster, task_read, min_score)
+    tc, trd, s1, s2, a = [], [], [], [], []
+    for t in range(len(task_cluster)):
+        for row in res.alignments(t)[:per_task]:
+            tc.append(task_cluster[t]); trd.append(task_read[t]); s1.append(row[0]); s2.append(row[1]); a.append(row[2])
+    _backtrace_vs_oracle(oracle, al, refs, reads, tc, trd, s1, s2, a)
     return len(tc)
 
 
@@ -483,6 +490,102 @@ def test_backtrace_long_reads_and_ties(oracle_mod, gpu_ctx):
             tc.append(c); trd.append(len(reads)); reads.append(read)
     ms = np.array([int(1.2 * len(reads[r])) for r in trd], np.int32)
     assert _check_backtrace(oracle_mod, gpu_ctx, refs, reads, np.array(tc, np.int32), np.array(trd, np.int32), ms, per_task=6) > 10
+
+
+@pytest.mark.parametrize("end_gaps", [False, True])
+def test_backtrace_edge_start_cells(oracle_mod, gpu_ctx, end_gaps):
+    """start cells on the corners and edges of both matrices -- i1 in {0, R1}, i2 in {0, R2}, a in {0, L} -- and inner
+    points, whether or not an alignment exists there; the last task's read is empty"""
+    import defuse_b200 as d
+    rng = np.random.default_rng(44)
+    refs, reads, tc, trd = util.split_batch(rng, 3, 2, 100, 280, 420)
+    reads.append(b"")
+    tc, trd = np.append(tc, 1).astype(np.int32), np.append(trd, len(reads) - 1).astype(np.int32)
+    k_tc, k_trd, s1, s2, a = [], [], [], [], []
+    for t in range(len(tc)):
+        R1, R2, L = len(refs[2 * tc[t]]), len(refs[2 * tc[t] + 1]), len(reads[trd[t]])
+        for i1 in (0, R1 // 2, R1):
+            for rs2 in (-1, R2 // 3, R2 - 1):      # i2 = R2, ..., 0
+                for split in sorted({0, min(1, L), L // 2, L}):
+                    k_tc.append(tc[t]); k_trd.append(trd[t]); s1.append(i1); s2.append(rs2); a.append(split)
+    al = d.SplitReadAligner(2, -1, -2, end_gaps, 8, ctx=gpu_ctx)
+    off, pairs = _backtrace_vs_oracle(oracle_mod, al, refs, reads, k_tc, k_trd, s1, s2, a)
+    assert len(pairs) > 0
+
+
+def test_backtrace_reads_longer_than_1024(oracle_mod, gpu_ctx):
+    """reads over 1024 bases against 1300-1500-base windows: boxes too large for shared memory (the global arena)"""
+    import defuse_b200 as d
+    rng = np.random.default_rng(25)
+    refs, reads, tc, trd = util.split_batch(rng, 2, 2, (1030, 1200), 1300, 1500)
+    ms = np.array([d.split_min_score(len(reads[r])) for r in trd], np.int32)
+    assert _check_backtrace(oracle_mod, gpu_ctx, refs, reads, tc, trd, ms, per_task=3) > 0
+
+
+def test_backtrace_size_only_and_short_buffer(gpu_ctx):
+    """matches = NULL sizes the output; a matches_cap below the total is refused after match_off and n_pairs are
+    written, and matches is left as it was"""
+    import ctypes
+    import defuse_b200 as d
+    rng = np.random.default_rng(46)
+    refs, reads, tc, trd = util.split_batch(rng, 4, 3, 100, 280, 420)
+    rt, st = _tables(refs, reads)
+    s1 = np.array([len(refs[2 * c]) // 2 for c in tc], np.int32)
+    s2 = np.array([len(refs[2 * c + 1]) // 2 for c in tc], np.int32)
+    a = np.array([len(reads[r]) // 2 for r in trd], np.int32)
+    al = d.SplitReadAligner(ctx=gpu_ctx)
+    want_off, want = al.backtrace_batch(rt, st, tc, trd, s1, s2, a)
+    assert len(want) > 1
+    lib, n = gpu_ctx._lib, len(tc)
+    rts, sts = rt.c_struct(), st.c_struct()
+    arrays = [np.ascontiguousarray(x, np.int32) for x in (tc, trd, s1, s2, a)]
+
+    def call(matches, cap):
+        off, total = np.full(2 * n + 1, -1, np.int64), ctypes.c_int64(-1)
+        rc = lib.dfb_split_backtrace_batch(gpu_ctx._h, ctypes.byref(al.params), ctypes.byref(rts), ctypes.byref(sts),
+                                           *[x.ctypes.data for x in arrays], n, off.ctypes.data, matches, cap, ctypes.byref(total))
+        return rc, off, total.value
+
+    rc, off, total = call(None, 0)
+    assert rc == 0 and off.tobytes() == want_off.tobytes() and total == len(want)
+    short = np.full((len(want) - 1, 2), -7, np.int32)
+    rc, off, total = call(short.ctypes.data, len(want) - 1)
+    assert rc == 2
+    assert b"matches buffer holds %d pairs, %d needed" % (len(want) - 1, len(want)) in lib.dfb_last_error(gpu_ctx._h)
+    assert off.tobytes() == want_off.tobytes() and total == len(want)
+    assert (short == -7).all()
+
+
+def test_device_backtrace_survives_a_host_backtrace(gpu_ctx):
+    """a dfb_split_backtrace_device result stays on the context across a dfb_split_backtrace_batch call and is still
+    what dfb_split_backtrace_copy_device copies out"""
+    import ctypes
+    import torch
+    import defuse_b200 as d
+    rng = np.random.default_rng(47)
+    refs, reads, tc, trd = util.split_batch(rng, 10, 5, 100, 280, 420)
+    rt, st = _tables(refs, reads)
+    ms = np.array([d.split_min_score(len(reads[r])) for r in trd], np.int32)
+    al = d.SplitReadAligner(ctx=gpu_ctx)
+    dev = [torch.from_numpy(x).cuda() for x in (tc, trd, ms)]
+    res = al.align_device(d.DeviceSeqTable.from_host(rt, "cuda:0"), d.DeviceSeqTable.from_host(st, "cuda:0"), *dev)
+    rec = res.records()
+    r = rec.cpu().numpy()
+    assert len(r) > 10
+    want_off, want = al.backtrace_batch(rt, st, tc[r[:, 0]], trd[r[:, 0]], r[:, 1], r[:, 2], r[:, 3])
+    lib, n = gpu_ctx._lib, ctypes.c_int64()
+    rts, sts = res.refs.c_struct(), res.reads.c_struct()
+    assert lib.dfb_split_backtrace_device(gpu_ctx._h, ctypes.byref(res.params), ctypes.byref(rts), ctypes.byref(sts),
+                                          res.task_cluster.data_ptr(), res.task_read.data_ptr(), res.task_cluster.numel(),
+                                          rec.data_ptr(), rec.shape[0], ctypes.byref(n)) == 0
+    assert n.value == len(want)
+    other_off, _ = al.backtrace_batch(rt, st, tc[r[::3, 0]], trd[r[::3, 0]], r[::3, 1], r[::3, 2], r[::3, 3])
+    assert len(other_off) != len(want_off)
+    off = torch.empty(2 * len(r) + 1, dtype=torch.int64, device="cuda:0")
+    pairs = torch.empty((n.value, 2), dtype=torch.int32, device="cuda:0")
+    assert lib.dfb_split_backtrace_copy_device(gpu_ctx._h, off.data_ptr(), pairs.data_ptr()) == 0
+    assert off.cpu().numpy().tobytes() == want_off.tobytes()
+    assert pairs.cpu().numpy().tobytes() == want.tobytes()
 
 
 def test_backtrace_argument_errors(gpu_ctx):
