@@ -188,13 +188,6 @@ static void parallel_for(HostPool* pool, int T, F fn)
 	for (auto& x : th) x.join();
 }
 
-struct AsmChunk
-{
-	HostArr<dfb_split_row> rows;
-	HostArr<int32_t> cols;
-	size_t n_rows = 0, n_cols = 0;
-};
-
 // Match lists of a backtrace in device memory of the stream-ordered pool: 2 n + 1 offsets and the (refPos, readPos)
 // pairs, one exact-size block per wave of the call, in order
 struct BtResult
@@ -244,10 +237,6 @@ struct dfb_ctx
 	// recycled host memory of the result assembly (kept mapped between batches)
 	HostArr<dfb_split_row> spare_rows;
 	HostArr<int32_t> spare_cols;
-	std::vector<AsmChunk> asm_chunks;
-	HostArr<int32_t> slot_of;
-	HostArr<dfb_split_row> chunk_rows[kStageSlots]; // per-chunk results of a pipelined batch, before the merge
-	HostArr<int32_t> chunk_cols[kStageSlots];
 };
 
 static thread_local std::string g_create_err;
@@ -465,10 +454,6 @@ extern "C" void dfb_ctx_destroy(dfb_ctx* ctx)
 	delete ctx->pool_fetch;
 	ctx->spare_rows.release();
 	ctx->spare_cols.release();
-	ctx->slot_of.release();
-	for (auto& c : ctx->asm_chunks) { c.rows.release(); c.cols.release(); }
-	for (auto& c : ctx->chunk_rows) c.release();
-	for (auto& c : ctx->chunk_cols) c.release();
 	if (ctx->own_stream) cudaStreamDestroy(ctx->own_stream);
 	delete ctx;
 }
@@ -698,7 +683,6 @@ struct dfb_plan
 	cudaEvent_t done_ev = nullptr; // recorded behind the last kernel of dfb_plan_run
 	cudaStream_t up = nullptr;     // stream of the upload + pack work (the compute stream unless pipelined)
 	cudaEvent_t packed_ev = nullptr; // recorded behind the pack kernels when `up` is not the compute stream
-	int result_slot = -1;          // chunk of a pipelined batch: which recycled result arrays of the ctx to use
 	dfb_plan_stats stats{};
 };
 
@@ -807,16 +791,8 @@ extern "C" void dfb_plan_destroy(dfb_plan* plan)
 		if (plan->ctx->last_split == plan) plan->ctx->last_split = nullptr;
 		release_device(plan);
 		// hand the result arrays back for the next batch
-		if (plan->result_slot >= 0)
-		{
-			plan->rows.swap(plan->ctx->chunk_rows[plan->result_slot]);
-			plan->cols.swap(plan->ctx->chunk_cols[plan->result_slot]);
-		}
-		else
-		{
-			if (plan->rows.cap > plan->ctx->spare_rows.cap) plan->rows.swap(plan->ctx->spare_rows);
-			if (plan->cols.cap > plan->ctx->spare_cols.cap) plan->cols.swap(plan->ctx->spare_cols);
-		}
+		if (plan->rows.cap > plan->ctx->spare_rows.cap) plan->rows.swap(plan->ctx->spare_rows);
+		if (plan->cols.cap > plan->ctx->spare_cols.cap) plan->cols.swap(plan->ctx->spare_cols);
 	}
 	if (plan->pending.ready) cudaEventDestroy(plan->pending.ready);
 	if (plan->pending.uploaded) cudaEventDestroy(plan->pending.uploaded);
@@ -2496,62 +2472,44 @@ static bool device_build_chosen(dfb_ctx* ctx, bool simple, const dfb_split_param
 	return device;
 }
 
-// A batch of either aligner (tables and tasks as for plan_create_host) cut into the chunks that start at t0, whose
-// table-B indices do not decrease.  A chunk sees a view of table B (its own entries) and, when the batch's table-A
-// indices do not decrease either (`a_monotone`), a view of table A too -- else the whole table.  Device-built chunks
-// (three beats per chunk): the uploads of chunk k+1 are queued on the upload stream while chunk k is finished --
-// allocations, packing and job scatter once its class counts are back -- and launched; the job-build kernels of chunk
-// k+1 ride on the compute stream between chunk k's two sweeps, so their counts are on the host before chunk k's probe
-// sweep ends and the GPU never waits for this thread.  The plans land in `plans`; chunk_queued(k) runs once chunk k is
-// on the GPU (a non-zero return stops the batch), batch_done(rc) once no more is queued: it waits for what is in flight
-// and returns the batch's result.  The plans are destroyed on return.
-static int pipeline_run(dfb_ctx* ctx, bool simple, const dfb_split_params* params, const dfb_seq_table* A, const dfb_seq_table* B,
-                        const int32_t* task_a, const int32_t* task_b, const int32_t* task_min_score, bool a_monotone,
-                        const std::vector<int64_t>& t0, std::vector<dfb_plan*>& plans, const std::function<int(int)>& chunk_queued,
-                        const std::function<int(int)>& batch_done)
+// A chunk of a pipelined batch: its views of the two tables, the caller's numbers of their first entries and, for
+// device-resident tables, the byte ranges [a0, a1), [b0, b1) the views cover (null: host tables)
+struct ChunkView
+{
+	dfb_seq_table a, b;
+	int32_t a_lo = 0, b_lo = 0;
+	const int64_t* range = nullptr;
+};
+
+// A batch of either aligner (tasks as for plan_create_host) cut into the chunks that start at t0.  view_of(k) gives chunk
+// k's table views, host_plan(k) builds chunk k on the host.  Device-built chunks (`device_build`; three beats per chunk):
+// the uploads of chunk k+1 are queued on the upload stream while chunk k is finished -- allocations, packing and job
+// scatter once its class counts are back -- and launched; the job-build kernels of chunk k+1 ride on the compute stream
+// between chunk k's two sweeps, so their counts are on the host before chunk k's probe sweep ends and the GPU never waits
+// for this thread.  A chunk the device build hands back (DFB_BUILD_ON_HOST) is built by host_plan.  The plans land in
+// `plans`; chunk_queued(k) runs once chunk k is on the GPU (a non-zero return stops the batch), batch_done(rc) once no
+// more is queued: it waits for what is in flight and returns the batch's result.  The plans are destroyed on return.
+static int pipeline_run(dfb_ctx* ctx, bool simple, const dfb_split_params* params, const int32_t* task_a, const int32_t* task_b,
+                        const int32_t* task_min_score, const std::vector<int64_t>& t0, bool device_build,
+                        const std::function<int(int, ChunkView&)>& view_of,
+                        const std::function<int(int, const ChunkView&, dfb_plan**)>& host_plan, std::vector<dfb_plan*>& plans,
+                        const std::function<int(int)>& chunk_queued, const std::function<int(int)>& batch_done)
 {
 	const int K = (int)t0.size() - 1;
-	const int64_t per = simple ? 1 : 2; // table-A entries per task index (split: the two windows of a cluster)
-	struct View
-	{
-		dfb_seq_table a, b;
-		int32_t a_lo = 0, b_lo = 0;
-	};
-	auto chunk_of = [&](int k, View& v) -> int {
-		const int64_t t_lo = t0[(size_t)k], t_hi = t0[(size_t)k + 1];
-		if (t_hi <= t_lo) return set_err(ctx, DFB_ERR_STATE, "empty chunk in a pipelined batch");
-		const int64_t b_lo = task_b[t_lo], b_hi = (int64_t)task_b[t_hi - 1] + 1;
-		if (b_lo < 0 || b_hi > B->n) return set_err(ctx, DFB_ERR_ARG, "task %lld: table index out of range", (long long)t_lo);
-		int64_t a_lo = 0, a_hi = A->n / per;
-		if (a_monotone)
-		{
-			a_lo = task_a[t_lo];
-			a_hi = (int64_t)task_a[t_hi - 1] + 1;
-			if (a_lo < 0 || per * a_hi > A->n)
-				return set_err(ctx, DFB_ERR_ARG, "task %lld: table index out of range", (long long)(simple || a_lo < 0 ? t_lo : t_hi - 1));
-		}
-		v.a = dfb_seq_table{A->bytes, A->off + per * a_lo, per * (a_hi - a_lo)};
-		v.b = dfb_seq_table{B->bytes, B->off + b_lo, b_hi - b_lo};
-		v.a_lo = (int32_t)a_lo;
-		v.b_lo = (int32_t)b_lo;
-		return DFB_OK;
-	};
-	auto min_score_of = [&](int64_t t) -> const int32_t* { return simple ? nullptr : task_min_score + t; };
 	std::vector<dfb_plan*> staged((size_t)K, nullptr);
 	auto upload = [&](int k) -> int {
-		View v;
+		ChunkView v;
 		const int64_t a = t0[(size_t)k];
-		int rc = chunk_of(k, v);
-		return rc ? rc : device_build_enqueue(ctx, simple, params, &v.a, &v.b, task_a + a, task_b + a, min_score_of(a), t0[(size_t)k + 1] - a,
-		                                      v.a_lo, v.b_lo, k, &staged[(size_t)k]);
+		int rc = view_of(k, v);
+		return rc ? rc : device_build_enqueue(ctx, simple, params, &v.a, &v.b, task_a + a, task_b + a, simple ? nullptr : task_min_score + a,
+		                                      t0[(size_t)k + 1] - a, v.a_lo, v.b_lo, k, &staged[(size_t)k], v.range);
 	};
-	const bool device_build = device_build_chosen(ctx, simple, params);
 	// DFB_TRACE: the device's side of the batch -- when every chunk's uploads, first sweep and (split) probe sweep +
 	// assembly ended, measured from an event recorded on the (idle) compute stream now
 	cudaEvent_t trace_base = nullptr;
 	if (trace_on() && cudaEventCreate(&trace_base) == cudaSuccess) cudaEventRecord(trace_base, ctx->stream);
 	int rc = DFB_OK;
-	if (device_build)
+	if (device_build && K)
 	{
 		rc = upload(0);
 		if (!rc) rc = device_build_kernels(staged[0]); // (the GPU is idle: straight away)
@@ -2569,15 +2527,11 @@ static int pipeline_run(dfb_ctx* ctx, bool simple, const dfb_split_params* param
 		}
 		if (rc == DFB_BUILD_ON_HOST)
 		{
-			View v;
-			const int64_t a = t0[(size_t)k];
-			if (!(rc = chunk_of(k, v)))
-				rc = plan_create_host(ctx, simple, params, &v.a, &v.b, task_a + a, task_b + a, min_score_of(a), t0[(size_t)k + 1] - a, v.a_lo,
-				                      v.b_lo, k, (k & 1) ? ctx->upload_stream2 : ctx->upload_stream, &pk);
+			ChunkView v;
+			if (!(rc = view_of(k, v))) rc = host_plan(k, v, &pk);
 		}
 		if (rc) break;
 		plans[(size_t)k] = pk;
-		if (!simple) pk->result_slot = k;
 		if (trace_base) pk->timing = true;
 		// the next chunk's build kernels ride behind this chunk's first sweep on the compute stream
 		dfb_plan* next = (k + 1 < K) ? staged[(size_t)k + 1] : nullptr;
@@ -2617,6 +2571,43 @@ static int pipeline_run(dfb_ctx* ctx, bool simple, const dfb_split_params* param
 	return rc;
 }
 
+// pipeline_run over host tables, whose table-B indices do not decrease.  A chunk sees a view of table B (its own entries)
+// and, when the batch's table-A indices do not decrease either (`a_monotone`), a view of table A too -- else the whole
+// table.  Chunks the device does not build are built by plan_create_host.
+static int pipeline_run_host(dfb_ctx* ctx, bool simple, const dfb_split_params* params, const dfb_seq_table* A, const dfb_seq_table* B,
+                             const int32_t* task_a, const int32_t* task_b, const int32_t* task_min_score, bool a_monotone,
+                             const std::vector<int64_t>& t0, std::vector<dfb_plan*>& plans, const std::function<int(int)>& chunk_queued,
+                             const std::function<int(int)>& batch_done)
+{
+	const int64_t per = simple ? 1 : 2; // table-A entries per task index (split: the two windows of a cluster)
+	auto view_of = [&](int k, ChunkView& v) -> int {
+		const int64_t t_lo = t0[(size_t)k], t_hi = t0[(size_t)k + 1];
+		if (t_hi <= t_lo) return set_err(ctx, DFB_ERR_STATE, "empty chunk in a pipelined batch");
+		const int64_t b_lo = task_b[t_lo], b_hi = (int64_t)task_b[t_hi - 1] + 1;
+		if (b_lo < 0 || b_hi > B->n) return set_err(ctx, DFB_ERR_ARG, "task %lld: table index out of range", (long long)t_lo);
+		int64_t a_lo = 0, a_hi = A->n / per;
+		if (a_monotone)
+		{
+			a_lo = task_a[t_lo];
+			a_hi = (int64_t)task_a[t_hi - 1] + 1;
+			if (a_lo < 0 || per * a_hi > A->n)
+				return set_err(ctx, DFB_ERR_ARG, "task %lld: table index out of range", (long long)(simple || a_lo < 0 ? t_lo : t_hi - 1));
+		}
+		v.a = dfb_seq_table{A->bytes, A->off + per * a_lo, per * (a_hi - a_lo)};
+		v.b = dfb_seq_table{B->bytes, B->off + b_lo, b_hi - b_lo};
+		v.a_lo = (int32_t)a_lo;
+		v.b_lo = (int32_t)b_lo;
+		return DFB_OK;
+	};
+	auto host_plan = [&](int k, const ChunkView& v, dfb_plan** out) -> int {
+		const int64_t a = t0[(size_t)k];
+		return plan_create_host(ctx, simple, params, &v.a, &v.b, task_a + a, task_b + a, simple ? nullptr : task_min_score + a,
+		                        t0[(size_t)k + 1] - a, v.a_lo, v.b_lo, k, (k & 1) ? ctx->upload_stream2 : ctx->upload_stream, out);
+	};
+	return pipeline_run(ctx, simple, params, task_a, task_b, task_min_score, t0, device_build_chosen(ctx, simple, params), view_of, host_plan,
+	                    plans, chunk_queued, batch_done);
+}
+
 // Large batches whose task_seq is non-decreasing go through pipeline_run: chunk k+1 is uploaded and packed underneath
 // chunk k's sweep, the scores of chunk k-1 go back on the copy stream meanwhile.  A chunk takes a view of the sequences it
 // names; of the references too when task_ref is non-decreasing as well (matealign: one window per task), else the whole
@@ -2651,7 +2642,7 @@ static int simple_align_pipelined(dfb_ctx* ctx, const dfb_split_params* params, 
 		trp.lap("simple pipelined: done");
 		return rc;
 	};
-	return pipeline_run(ctx, true, params, refs, seqs, task_ref, task_seq, nullptr, refs_monotone, t0, plans, copy_scores, wait_all);
+	return pipeline_run_host(ctx, true, params, refs, seqs, task_ref, task_seq, nullptr, refs_monotone, t0, plans, copy_scores, wait_all);
 }
 
 static int dfb_simple_align_batch_body(dfb_ctx* ctx, const dfb_simple_params* params, const dfb_seq_table* refs,
@@ -2820,8 +2811,8 @@ static int split_align_pipelined(dfb_ctx* ctx, const dfb_split_params* params, c
 		}
 		return rc;
 	};
-	const int rc = pipeline_run(ctx, false, params, refs, reads, task_cluster, task_read, task_min_score, clusters_monotone, t0, plans,
-	                            hand_to_lane2, join_lane2);
+	const int rc = pipeline_run_host(ctx, false, params, refs, reads, task_cluster, task_read, task_min_score, clusters_monotone, t0, plans,
+	                                 hand_to_lane2, join_lane2);
 	trp.lap("pipelined: chunks destroyed");
 	if (rc)
 	{
@@ -3307,11 +3298,12 @@ static int dfb_split_align_device_body(dfb_ctx* ctx, const dfb_split_params* par
 	};
 	// the host form's chunks (split_chunk_starts), so that the column pool comes out the same
 	const bool chunked = n_tasks >= pipeline_min_tasks() && !chk.b_decreases;
-	const std::vector<int64_t> t0 = chunked ? split_chunk_starts(n_tasks) : std::vector<int64_t>{0, n_tasks};
-	const int K = n_tasks ? (int)t0.size() - 1 : 0;
+	std::vector<int64_t> t0 = chunked ? split_chunk_starts(n_tasks) : std::vector<int64_t>{0, n_tasks};
+	if (!n_tasks) t0.resize(1); // (no chunk)
+	const int K = (int)t0.size() - 1;
 	static_assert(dfb_ctx::kStageSlots <= DFB_MAX_CHUNKS, "ChunkStarts too small");
 	// chunk views: a_lo, a_hi, b_lo, b_hi and their byte offsets
-	std::vector<long long> bnd((size_t)std::max(K, 1) * 8, 0);
+	std::vector<int64_t> bnd((size_t)std::max(K, 1) * 8, 0);
 	if (chunked)
 	{
 		ChunkStarts cs;
@@ -3330,39 +3322,31 @@ static int dfb_split_align_device_body(dfb_ctx* ctx, const dfb_split_params* par
 	}
 	else if (K)
 	{
-		const long long one[8] = {0, refs->n / 2, 0, reads->n, 0, chk.tab[0].off_n, 0, chk.tab[1].off_n};
+		const int64_t one[8] = {0, refs->n / 2, 0, reads->n, 0, (int64_t)chk.tab[0].off_n, 0, (int64_t)chk.tab[1].off_n};
 		memcpy(bnd.data(), one, sizeof(one));
 	}
-	struct View
-	{
-		dfb_seq_table a, b;
-		int64_t range[4];
-	};
-	std::vector<View> views((size_t)K);
-	for (int k = 0; k < K; k++)
-	{
-		const long long* o = bnd.data() + 8 * k;
-		View& v = views[(size_t)k];
+	// chunk k's views: entries o[0] .. o[1] of the clusters and o[2] .. o[3] of the reads, bytes o[4] .. o[5] and o[6] .. o[7]
+	auto view_of = [&](int k, ChunkView& v) -> int {
+		const int64_t* o = bnd.data() + 8 * (size_t)k;
 		v.a = dfb_seq_table{refs->bytes, refs->off + 2 * o[0], 2 * (o[1] - o[0])};
 		v.b = dfb_seq_table{reads->bytes, reads->off + o[2], o[3] - o[2]};
-		v.range[0] = o[4];
-		v.range[1] = o[5];
-		v.range[2] = o[6];
-		v.range[3] = o[7];
-	}
+		v.a_lo = (int32_t)o[0];
+		v.b_lo = (int32_t)o[2];
+		v.range = o + 4;
+		return DFB_OK;
+	};
+	int64_t host_d2h = 0;
+	auto host_plan = [&](int k, const ChunkView& v, dfb_plan** out) -> int {
+		const int64_t a = t0[(size_t)k];
+		return plan_create_from_device(ctx, false, params, &v.a, &v.b, task_cluster + a, task_read + a, task_min_score + a, t0[(size_t)k + 1] - a,
+		                               v.a_lo, v.b_lo, k, ctx->upload_stream, &host_d2h, out);
+	};
 	// sort key widths of the overflow events: rows <= longest read, columns <= longest window
 	OvKey key;
 	key.rb = bit_width(chk.tab[1].max_len + 1);
 	key.cb = bit_width(chk.tab[0].max_len + 1);
 	key.sub_passes = (1 + key.rb + key.cb + 7) / 8;
-	const bool device_build = any_fast_class(false, params);
-	std::vector<dfb_plan*> staged((size_t)K, nullptr), plans((size_t)K, nullptr);
-	auto enqueue = [&](int k) -> int {
-		const View& v = views[(size_t)k];
-		const int64_t a = t0[(size_t)k];
-		return device_build_enqueue(ctx, false, params, &v.a, &v.b, task_cluster + a, task_read + a, task_min_score + a, t0[(size_t)k + 1] - a,
-		                            (int32_t)bnd[8 * (size_t)k], (int32_t)bnd[8 * (size_t)k + 2], k, &staged[(size_t)k], v.range);
-	};
+	std::vector<dfb_plan*> plans((size_t)K, nullptr);
 	unsigned long long* d_base = nullptr; // the batch's row and column totals so far
 	int64_t rows_cap = 0, cols_cap = 0, rows_bound = 0, cols_bound = 0;
 	if (cudaError_t e = dalloc(ctx, (void**)&d_base, 2 * sizeof(unsigned long long))) return fail(set_err(ctx, DFB_ERR_NOMEM, "%s", cudaGetErrorString(e)));
@@ -3401,60 +3385,27 @@ static int dfb_split_align_device_body(dfb_ctx* ctx, const dfb_split_params* par
 		release_device(pl);
 		return arc;
 	};
-	Trace tr;
-	if (!rc && device_build && K)
-	{
-		rc = enqueue(0);
-		if (!rc) rc = device_build_kernels(staged[0]);
-	}
-	int64_t host_d2h = 0;
-	for (int k = 0; k < K && !rc; k++)
-	{
-		if (device_build && k + 1 < K && (rc = enqueue(k + 1))) break;
-		dfb_plan* pk = staged[(size_t)k];
-		staged[(size_t)k] = nullptr;
-		rc = DFB_BUILD_ON_HOST;
-		if (pk && (rc = device_build_finish(pk)))
-		{
-			dfb_plan_destroy(pk);
-			pk = nullptr;
-		}
-		if (rc == DFB_BUILD_ON_HOST)
-		{
-			const View& v = views[(size_t)k];
-			const int64_t a = t0[(size_t)k];
-			rc = plan_create_from_device(ctx, false, params, &v.a, &v.b, task_cluster + a, task_read + a, task_min_score + a, t0[(size_t)k + 1] - a,
-			                             (int32_t)bnd[8 * (size_t)k], (int32_t)bnd[8 * (size_t)k + 2], k, ctx->upload_stream, &host_d2h, &pk);
-		}
-		if (rc) break;
-		plans[(size_t)k] = pk;
-		// the next chunk's build kernels ride behind this chunk's first sweep; the previous chunk is assembled behind this one
-		dfb_plan* next = (k + 1 < K) ? staged[(size_t)k + 1] : nullptr;
-		const std::function<int()> hook = [&]() -> int { return next ? device_build_kernels(next) : DFB_OK; };
-		rc = plan_run_impl(pk, &hook);
-		if (!rc && k > 0) rc = collect(k - 1);
-	}
-	if (!rc && K) rc = collect(K - 1);
-	tr.lap("split device: chunks queued");
-	for (dfb_plan* sp : staged)
-		if (sp)
-		{
-			cudaStreamSynchronize(sp->up);
-			dfb_plan_destroy(sp);
-		}
+	// chunk k-1 is collected once chunk k is queued: its assembly runs behind chunk k's sweeps
+	auto queued = [&](int k) -> int { return k ? collect(k - 1) : DFB_OK; };
 	unsigned long long totals[2] = {0, 0};
+	auto done = [&](int brc) -> int {
+		if (!brc && K) brc = collect(K - 1);
+		if (!brc)
+		{
+			cudaError_t e = cudaMemcpyAsync(ctx->h_out.p, d_base, sizeof(totals), cudaMemcpyDeviceToHost, ctx->stream);
+			if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+			if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->copy_stream);
+			if (e != cudaSuccess) brc = set_err(ctx, DFB_ERR_CUDA, "split device batch failed: %s", cudaGetErrorString(e));
+			else memcpy(totals, ctx->h_out.p, sizeof(totals));
+			holder->stats.d2h_bytes += (int64_t)sizeof(totals) + host_d2h;
+		}
+		if (!brc) brc = bounds_check_status(ctx);
+		return brc;
+	};
+	Trace tr;
 	if (!rc)
-	{
-		cudaError_t e = cudaMemcpyAsync(ctx->h_out.p, d_base, sizeof(totals), cudaMemcpyDeviceToHost, ctx->stream);
-		if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-		if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->copy_stream);
-		if (e != cudaSuccess) rc = set_err(ctx, DFB_ERR_CUDA, "split device batch failed: %s", cudaGetErrorString(e));
-		else memcpy(totals, ctx->h_out.p, sizeof(totals));
-		holder->stats.d2h_bytes += (int64_t)sizeof(totals) + host_d2h;
-	}
-	if (!rc) rc = bounds_check_status(ctx);
-	for (dfb_plan* pk : plans)
-		if (pk) dfb_plan_destroy(pk);
+		rc = pipeline_run(ctx, false, params, task_cluster, task_read, task_min_score, t0, any_fast_class(false, params), view_of, host_plan,
+		                  plans, queued, done);
 	dfree(ctx, d_base);
 	tr.lap("split device: done");
 	if (rc) return fail(rc);

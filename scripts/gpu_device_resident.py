@@ -6,9 +6,25 @@ PCIe bytes, peak pool memory; plus bench.py's e2e of a parent build (DFB_PARENT_
 Writes profiles/<tag>_device_resident.json.  Shapes: the bench split shape (20 000 clusters x 100 reads), the
 localalign shape (BASELINE config 2: 1 M 100-bp reads, 10 k references of 2001 bp), the matealign shape (config 4:
 150-bp reads, one 1001-bp window per task) and the stress shape (synth.STRESS, 4 000 clusters x 50).  The arms
-alternate inside every shape after one warm-up call each; both results are compared byte for byte."""
+alternate inside every shape after one warm-up call each; both results are compared byte for byte.
+
+    python scripts/gpu_device_resident.py --tag r06 --host-ab --parent-lib build/parent/libdefuse_b200.so [--rounds 3]
+
+Writes profiles/<tag>_host_form_ab.json instead: the host one-call form (SplitReadAligner.align_batch, pinned arrays) of
+the parent build against this build, one process per build in alternating order per round.  A process reads the card's
+name, power limit and SM clock, warms every workload up with one call and times `calls` calls of each with a host clock
+(the call ends in a synchronise); it hashes best, rows and columns, which must be equal across both builds, and reads
+the peak pool memory.  Workloads: the bench e2e batch (2 M tasks) with DFB_HOST_BUILD=1 and with DFB_DEVICE_BUILD=1,
+the 200 k-task bench shape, STRESS, the poly-A batch of tests/test_device_resident.py (one call form and pipelined) and
+a 20 k-task batch below DFB_PIPELINE_MIN_TASKS; the device-resident form (align_device + to_host) on the bench e2e batch,
+which shares the chunk loop and the collection; then the dosplitalign tool, each build's binary beside its library: one
+warm-up run and six timed ones of the whole process, whose wall clock includes CUDA start-up (1-4 s on these boxes,
+DESIGN.md section 7), so that leg only shows a difference larger than the start-up's spread."""
 import argparse
+import hashlib
 import json
+import shutil
+import tempfile
 import os
 import subprocess
 import sys
@@ -114,6 +130,124 @@ def bench_ab(parent_lib, runs):
     return out
 
 
+TOOL_DATASET = dict(seed=62, n_clusters=2000, pairs_per_cluster=50)
+
+
+def host_workloads():
+    """(name, workload, env, calls)"""
+    import synth
+    e2e = synth.split_workload(3, 20000, 100)
+    yield "e2e_2M_host_build", e2e, {"DFB_HOST_BUILD": "1"}, 5
+    yield "e2e_2M_device_build", e2e, {"DFB_DEVICE_BUILD": "1"}, 5
+    yield "bench_200k", synth.split_workload(9, 2000, 100), {}, 10
+    yield "stress", synth.split_workload(5, 4000, 50, **synth.STRESS), {}, 10
+    poly = {"ref_bytes": np.frombuffer(b"A" * 1400, np.uint8), "ref_off": np.array([0, 700, 1400], np.int64),
+            "read_bytes": np.frombuffer(b"A" * 200 * 24, np.uint8), "read_off": np.arange(25, dtype=np.int64) * 200,
+            "task_cluster": np.zeros(24, np.int32), "task_read": np.arange(24, dtype=np.int32), "min_score": np.full(24, 360, np.int32)}
+    yield "poly_a", poly, {}, 5
+    yield "poly_a_pipelined", poly, {"DFB_PIPELINE_MIN_TASKS": "16"}, 5
+    yield "small_20k", synth.split_workload(4, 200, 100), {}, 20
+    yield "device_form_e2e_2M", e2e, {}, 5
+
+
+def host_worker(arm, data):
+    import defuse_b200 as d
+    ctx = d.default_context(0)
+    out = {"arm": arm, "lib": os.path.relpath(d.LIB_PATH, ROOT), "card": card(), "workloads": {}}
+    for name, w, env, calls in host_workloads():
+        h, keep = {}, []
+        for k, v in w.items():
+            h[k], t = pinned(np.ascontiguousarray(v))
+            keep.append(t)
+        refs, reads = d.SeqTable(h["ref_bytes"], h["ref_off"]), d.SeqTable(h["read_bytes"], h["read_off"])
+        al = d.SplitReadAligner(ctx=ctx)
+        os.environ.update(env)
+        call = lambda: al.align_batch(refs, reads, h["task_cluster"], h["task_read"], h["min_score"])
+        if name.startswith("device_form"):
+            import torch
+            drefs, dreads = d.DeviceSeqTable.from_host(refs, "cuda:0"), d.DeviceSeqTable.from_host(reads, "cuda:0")
+            dt = [torch.from_numpy(h[k]).cuda() for k in ("task_cluster", "task_read", "min_score")]
+
+            def call():
+                r = al.align_device(drefs, dreads, *dt)
+                torch.cuda.synchronize()
+                return r
+        r = call()  # warm-up
+        ctx.memory_info(reset=True)
+        ms = []
+        for _ in range(calls):
+            t0 = time.perf_counter()
+            r = call()
+            ms.append((time.perf_counter() - t0) * 1e3)
+        for k in env:
+            del os.environ[k]
+        st = ctx.split_result_stats()
+        if name.startswith("device_form"):
+            r = r.to_host()
+        out["workloads"][name] = {
+            "n_tasks": int(len(h["task_read"])), "rows": int(len(r.rows)), "cols": int(len(r.cols)), "ms": ms,
+            "median_ms": float(np.median(ms)), "min_ms": float(min(ms)), "max_ms": float(max(ms)),
+            "pool_used_high_bytes": int(ctx.memory_info()[2]), "d2h_bytes": int(st["d2h_bytes"]), "h2d_bytes": int(st["h2d_bytes"]),
+            "output_sha256": hashlib.sha256(r.best.tobytes() + r.rows.tobytes() + r.cols.tobytes()).hexdigest()}
+    common = json.load(open(os.path.join(data, "args.json")))
+    ms, digest = [], None
+    for run in range(7):  # (the first is the warm-up)
+        outp = os.path.join(data, "out_%s.alignments" % arm)
+        t0 = time.perf_counter()
+        subprocess.run([os.path.join(data, "tools", arm, "bin", "dosplitalign")] + common + ["-a", outp], check=True, capture_output=True)
+        if run:
+            ms.append((time.perf_counter() - t0) * 1e3)
+        digest = hashlib.sha256(open(outp, "rb").read()).hexdigest()
+    out["workloads"]["dosplitalign_tool"] = {"ms": ms, "median_ms": float(np.median(ms)), "min_ms": float(min(ms)), "max_ms": float(max(ms)),
+                                             "output_sha256": digest}
+    out["card_after"] = card()
+    print(json.dumps(out))
+
+
+def host_ab(parent_lib, rounds, out_path):
+    from synth import files
+    this_lib = os.path.join(ROOT, "defuse_b200", "libdefuse_b200.so")
+    bin_dir = os.path.join(ROOT, "defuse_b200", "bin")
+    runs = {"parent": [], "this": []}
+    with tempfile.TemporaryDirectory() as data:
+        json.dump(files.make_split_dataset(data, **TOOL_DATASET), open(os.path.join(data, "args.json"), "w"))
+        for arm, lib in (("parent", parent_lib), ("this", this_lib)):
+            os.makedirs(os.path.join(data, "tools", arm, "bin"))
+            shutil.copy(os.path.join(bin_dir, "dosplitalign"), os.path.join(data, "tools", arm, "bin", "dosplitalign"))
+            shutil.copy(lib, os.path.join(data, "tools", arm, "libdefuse_b200.so"))
+        for r in range(rounds):
+            for arm in (("parent", "this") if r % 2 == 0 else ("this", "parent")):
+                env = dict(os.environ)
+                env.pop("DFB_LIB_PATH", None)
+                if arm == "parent":
+                    env["DFB_LIB_PATH"] = parent_lib
+                p = subprocess.run([sys.executable, os.path.abspath(__file__), "--tag", "worker", "--host-worker", arm, "--data", data],
+                                   capture_output=True, text=True, env=env, cwd=ROOT)
+                if p.returncode:
+                    sys.exit("%s worker failed:\n%s" % (arm, p.stderr[-4000:]))
+                runs[arm].append(json.loads(p.stdout.strip().splitlines()[-1]))
+                print("round", r, arm, json.dumps({k: v["median_ms"] for k, v in runs[arm][-1]["workloads"].items()}), flush=True)
+    summary = {}
+    for name in runs["this"][0]["workloads"]:
+        row = {}
+        for arm in ("parent", "this"):
+            ws = [x["workloads"][name] for x in runs[arm]]
+            med = [x["median_ms"] for x in ws]
+            row[arm] = {"median_ms_per_round": med, "median_ms": float(np.median(med)),
+                        "range_ms": [min(x["min_ms"] for x in ws), max(x["max_ms"] for x in ws)]}
+            for k in ("pool_used_high_bytes", "d2h_bytes", "h2d_bytes"):
+                if k in ws[0]:
+                    row[arm][k] = max(x[k] for x in ws)
+        row["outputs_equal"] = len({x["workloads"][name]["output_sha256"] for a in runs for x in runs[a]}) == 1
+        summary[name] = row
+    result = {"card": runs["this"][0]["card"], "card_after": runs["this"][-1]["card_after"], "rounds": rounds,
+              "tool_dataset": TOOL_DATASET, "summary": summary, "runs": runs}
+    with open(out_path, "w") as f:
+        json.dump(result, f, indent=1)
+    print(json.dumps({k: {a: v[a]["median_ms"] for a in ("parent", "this")} for k, v in summary.items()}, indent=1))
+    print("wrote", out_path)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--tag", required=True)
@@ -121,7 +255,16 @@ def main():
     ap.add_argument("--parent-lib", default=None)
     ap.add_argument("--bench-runs", type=int, default=3)
     ap.add_argument("--out-dir", default=os.path.join(ROOT, "profiles"))
+    ap.add_argument("--host-ab", action="store_true")
+    ap.add_argument("--rounds", type=int, default=3)
+    ap.add_argument("--host-worker", choices=("parent", "this"))
+    ap.add_argument("--data")
     args = ap.parse_args()
+    if args.host_worker:
+        return host_worker(args.host_worker, args.data)
+    if args.host_ab:
+        os.makedirs(args.out_dir, exist_ok=True)
+        return host_ab(os.path.abspath(args.parent_lib), args.rounds, os.path.join(args.out_dir, "%s_host_form_ab.json" % args.tag))
     import defuse_b200 as d
     import synth
     ctx = d.default_context(0)
