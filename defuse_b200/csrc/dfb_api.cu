@@ -511,8 +511,19 @@ extern "C" int dfb_ctx_memory_info(dfb_ctx* ctx, int reset, int64_t* reserved_no
 // kernel classes: (lanes per job pair, rows per lane); capacity G*S read rows
 // ------------------------------------------------------------------------------------------
 
+// Reads of 81-100 bases go to four-lane groups of 25 rows: exactly 100 rows (eight-lane groups of 13 sweep 104) and half
+// the wavefront skew (3 head and tail steps instead of 7), with the per-step fixed cost shared by 25 rows instead of 13.
+// -DDFB_NARROW_GROUPS=0 takes the class out (build-time knob for A/B runs; those reads then run at <8,13>).
+#ifndef DFB_NARROW_GROUPS
+#define DFB_NARROW_GROUPS 1
+#endif
+#if DFB_NARROW_GROUPS
+#define DFB_NARROW_CLASS(X) X(4, 25)
+#else
+#define DFB_NARROW_CLASS(X)
+#endif
 #define DFB_CLASSES(X) \
-	X(8, 4) X(8, 7) X(8, 10) X(8, 13) X(8, 16) X(8, 19) X(8, 22) X(8, 25) X(8, 32) \
+	X(8, 4) X(8, 7) X(8, 10) DFB_NARROW_CLASS(X) X(8, 13) X(8, 16) X(8, 19) X(8, 22) X(8, 25) X(8, 32) \
 	X(16, 20) X(16, 25) X(16, 32) X(32, 24) X(32, 32)
 
 struct ClassDef
@@ -1121,8 +1132,8 @@ static int alloc_work(dfb_plan* pl, JobPair* d_jobs_base, GenJob* d_gen_base, co
 			DALLOC(ctx, cw.d_slot_n, n * sizeof(int));
 			DALLOC(ctx, cw.d_slot_ev, n * DFB_SLOT_EVENTS * sizeof(uint2));
 			DALLOC(ctx, cw.d_slot_rng, n * sizeof(uint32_t));
-			// checkpoints every CK = 4G steps of the wavefront (R + G - 1 steps)
-			const int G = kClasses[c].G, CK = 4 * G;
+			// checkpoints every CK = ckpt_steps(G) steps of the wavefront (R + G - 1 steps)
+			const int G = kClasses[c].G, CK = ckpt_steps(G);
 			const size_t gs_bytes = n * (size_t)G * kClasses[c].S * sizeof(uint32_t);
 			cw.ckpt_blocks = (int)(((int64_t)cw.max_R + G - 2) / CK);
 			size_t ck_bytes = n * (size_t)cw.ckpt_blocks * (size_t)(kClasses[c].S + 2) * G * sizeof(uint32_t);

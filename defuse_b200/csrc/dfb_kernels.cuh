@@ -277,9 +277,14 @@ __device__ __noinline__ void emit_probe_event(const FastParams& p, int item, int
 	}
 }
 
-// Decodes one ring block (8G reference columns of both halves) from the raw pool words cp.async left in shared memory
-// into 32-bit {half 1, half 0} symbol pairs.  Lane g owns columns 8g .. 8g+7 of the block and stores them in an order
-// rotated by the lane, so that the 32 lanes of the warp hit 32 different banks.  cw0 / cw1: pool word of ring column 0
+// Steps of the wavefront per checkpoint block: the first sweep's row-maximum fold and checkpoint interval, the probe
+// sweep's resume granularity.  4G, but at least 32: a four-lane group would otherwise fold and checkpoint every 16
+// steps, twice the per-cell cost of both.  A reference ring block is two checkpoint blocks (CH = 2 CK columns).
+__host__ __device__ constexpr int ckpt_steps(int G) { return G >= 8 ? 4 * G : 32; }
+
+// Decodes one ring block (CH = 2 ckpt_steps(G) reference columns of both halves) from the raw pool words cp.async left in
+// shared memory into 32-bit {half 1, half 0} symbol pairs.  Lane g owns CPL = CH/G columns (8; 16 for G = 4) starting at
+// CPL*g and stores them in an order rotated by the lane, so that the 32 lanes of the warp hit 32 different banks.  cw0 / cw1: pool word of ring column 0
 // in either half's reference (negative in front of the reference: those columns are padding).  The last G-1 columns of the
 // ring are stored a second time in front of it (ring[-1] = ring[RING-1] ...): lane g of the first sweep reads column u-g
 // at ring_lane[u mod RING] with ring_lane = ring - g and a warp-uniform index that needs no mask (MIRROR; the probe sweep
@@ -291,42 +296,50 @@ __device__ __noinline__ void ring_decode_block(uint32_t* ring, const uint2* raw_
                                                unsigned long long pool_words)
 {
 	(void)pool_words;
-	constexpr int HG = G / 2, CH = 8 * G, RING = 2 * CH;
-	constexpr int RSH = (G == 8) ? 0 : (G == 16 ? 1 : 2); // bank = 8 * (g + q * G / 8) + rotation (mod 32): distinct over the warp
-	const uint2 w0 = raw_slot[g >> 1], w1 = raw_slot[HG + (g >> 1)];
-	const int wrel = blk * HG + (g >> 1);
+	constexpr int CH = 2 * ckpt_steps(G), RING = 2 * CH;
+	constexpr int WB = CH / 16;  // pool words of one half in a ring block
+	constexpr int CPL = CH / G;  // columns per lane
+	static_assert(CPL == 8 || CPL == 16, "a lane decodes half a pool word or a whole one");
+	// G >= 8 (rings RING + G = 8 mod 32 words apart): bank = 8 * (g + q * G / 8) + rotation (mod 32): distinct over the warp.
+	// G = 4 (rings 4 mod 32 apart, 16 columns per lane): bank = 4q + 16g + ((n + g) mod 16) + 4 (mod 32) is (n + g) mod 4,
+	// distinct over the four lanes of a group, and the eight groups shift it by 4q: each residue class once.
+	constexpr int RSH = (G <= 8) ? 0 : (G == 16 ? 1 : 2);
+	const int wl = (g * CPL) >> 4;   // the lane's pool word in the block
+	const int bit0 = (g * CPL) & 15; // and its first base in that word
+	const uint2 w0 = raw_slot[wl], w1 = raw_slot[WB + wl];
+	const int wrel = blk * WB + wl;
 	const int wi0 = cw0 + wrel, wi1 = cw1 + wrel;
-	const int bit0 = 8 * (g & 1);
-	// the lane's eight bases of either half: 2-bit codes, exception flags, and how many of them lie inside the reference
+	// the lane's CPL bases of either half: 2-bit codes, exception flags, and how many of them lie inside the reference
 	const uint32_t c0 = w0.x >> (2 * bit0), c1 = w1.x >> (2 * bit0);
-	const int nv0 = wi0 < 0 ? 0 : min(8, max(0, (int)R0 - (wi0 * 16 + bit0)));
-	const int nv1 = wi1 < 0 ? 0 : min(8, max(0, (int)R1 - (wi1 * 16 + bit0)));
+	const int nv0 = wi0 < 0 ? 0 : min(CPL, max(0, (int)R0 - (wi0 * 16 + bit0)));
+	const int nv1 = wi1 < 0 ? 0 : min(CPL, max(0, (int)R1 - (wi1 * 16 + bit0)));
 	const uint32_t m0 = (w0.y >> bit0) & ((1u << nv0) - 1u), m1 = (w1.y >> bit0) & ((1u << nv1) - 1u);
 	DFB_BC(nv0 == 0 || (unsigned long long)ref_w0 + (unsigned long long)wi0 < pool_words, 201);
 	DFB_BC(nv1 == 0 || (unsigned long long)ref_w1 + (unsigned long long)wi1 < pool_words, 202);
 	const int rot = g >> RSH;
-	// ring slot of the lane's first column: a multiple of 8, so + nn never wraps
-	const int base_idx = (int)(((uint32_t)blk * CH + 16u * (g >> 1) + bit0) & (RING - 1));
+	// ring slot of the lane's first column: a multiple of CPL, so + nn never wraps
+	const int base_idx = (int)(((uint32_t)blk * CH + (uint32_t)(CPL * g)) & (RING - 1));
 	uint32_t* dst = ring + base_idx;
 	const int mirror_from = MIRROR ? RING - G - base_idx : 8; // columns nn > mirror_from have a mirror slot (RING words below)
 	// Both halves of a column with one PRMT: the 2-bit codes of the two references sit in the two halves of cc; the
 	// selector {code0, 4, code1, 4} picks {"ACGT"[code0], 0, "ACGT"[code1], 0} out of ("ACGT", 0).
+	// (16 columns per lane do not fit one register that way: the two codes are gathered one by one)
 	const uint32_t cc = (c0 & 0xFFFFu) | (c1 << 16);
 #pragma unroll
-	for (int n = 0; n < 8; n++)
+	for (int n = 0; n < CPL; n++)
 	{
-		const int nn = (n + rot) & 7;
-		const uint32_t x = (cc >> (2 * nn)) & 0x00030003u;
+		const int nn = (n + rot) & (CPL - 1);
+		const uint32_t x = CPL == 8 ? (cc >> (2 * nn)) & 0x00030003u : ((c0 >> (2 * nn)) & 3u) | (((c1 >> (2 * nn)) & 3u) << 16);
 		const uint32_t word = prmt(0x54474341u, 0u, x | (x >> 8) | 0x4040u);
 		dst[nn] = word;
 		if (MIRROR && nn > mirror_from) dst[nn - RING] = word;
 	}
 	uint16_t* dst16 = reinterpret_cast<uint16_t*>(dst);
-	if (nv0 < 8 || nv1 < 8)
+	if (nv0 < CPL || nv1 < CPL)
 	{
 		// columns in front of a reference or at and past its end equal no read symbol (only the blocks at a reference's
 		// ends have any)
-		for (int nn = 0; nn < 8; nn++)
+		for (int nn = 0; nn < CPL; nn++)
 		{
 			const int mirror = (MIRROR && nn > mirror_from) ? nn - RING : nn; // (the same slot again when the column has no mirror)
 			if (nn >= nv0) dst16[2 * nn] = dst16[2 * mirror] = (uint16_t)DFB_REF_PAD;
@@ -336,7 +349,7 @@ __device__ __noinline__ void ring_decode_block(uint32_t* ring, const uint2* raw_
 	if (m0 | m1)
 	{
 		// exception plane (rare): the raw byte replaces the decoded code
-		for (int nn = 0; nn < 8; nn++)
+		for (int nn = 0; nn < CPL; nn++)
 		{
 			const int mirror = (MIRROR && nn > mirror_from) ? nn - RING : nn;
 			if ((m0 >> nn) & 1u) dst16[2 * nn] = dst16[2 * mirror] = __ldg(obytes + ((size_t)ref_w0 + (size_t)wi0) * 16 + bit0 + nn);
@@ -369,8 +382,10 @@ __device__ __noinline__ void emit_probe_hits(const FastParams& p, int item, int 
 	}
 }
 
-// registers per thread the mode needs (arrays of S) decide how many CTAs we ask ptxas to fit per SM
-template <int S, int MODE>
+// registers per thread the mode needs (arrays of S) decide how many CTAs we ask ptxas to fit per SM.  Four-lane groups
+// (25-row strips, granule masks in shared memory) fit 168 registers in either mode with no local-memory traffic in the
+// pair loop (at 128, ptxas spills hundreds of bytes in SPLIT mode): three CTAs.
+template <int G, int S, int MODE>
 struct FastOcc
 {
 	static constexpr int kArrays = (MODE == MODE_SPLIT) ? 5 : 2;
@@ -378,29 +393,34 @@ struct FastOcc
 #ifndef DFB_OCC_SMALL
 #define DFB_OCC_SMALL 4 // CTAs per SM asked of ptxas for the classes with short strips (build-time knob for A/B runs)
 #endif
-	static constexpr int kMinBlocks = kEst <= 128 ? DFB_OCC_SMALL : (kEst <= 168 ? 3 : (kEst <= 255 ? 2 : 1));
+	static constexpr int kMinBlocks =
+	    G == 4 ? 3 : (kEst <= 128 ? DFB_OCC_SMALL : (kEst <= 168 ? 3 : (kEst <= 255 ? 2 : 1)));
 };
 
 template <int G, int S, int MODE>
-__global__ void __launch_bounds__(128, FastOcc<S, MODE>::kMinBlocks) dp_fast_kernel(const __grid_constant__ FastParams p)
+__global__ void __launch_bounds__(128, FastOcc<G, S, MODE>::kMinBlocks) dp_fast_kernel(const __grid_constant__ FastParams p)
 {
 	constexpr int NG = 32 / G;      // job pairs per warp
-	constexpr int CH = 8 * G;       // reference ring: block of CH columns, two blocks resident
-	constexpr int CK = 4 * G;       // checkpoint interval (steps): probe windows are whole CK blocks
+	constexpr int CK = ckpt_steps(G); // checkpoint interval (steps): probe windows are whole CK blocks
+	constexpr int CH = 2 * CK;      // reference ring: block of CH columns, two blocks resident
 	constexpr int RING = 2 * CH;
 	// G words in front of every ring: the mirror of its last G-1 columns (ring_decode_block) -- and what puts the rings of a
 	// warp's groups, which read the same index in the same step, into different banks
 	constexpr int RING_STRIDE = RING + G;
 	constexpr int ROWS = G * S;
 	constexpr int RDW = (ROWS + 15) / 16;
-	constexpr int HG = G / 2;       // pool words of one half in a ring block
-	static_assert(G >= 8 && (G & (G - 1)) == 0 && G <= 32, "group size");
+	constexpr int WB = CH / 16;     // pool words of one half in a ring block
+	static_assert(G >= 4 && (G & (G - 1)) == 0 && G <= 32, "group size");
 	static_assert(S >= 1 && S <= 32, "strip height");
-	static_assert(CH == 2 * CK, "the ring is refilled at the top of every second checkpoint block");
+	static_assert(WB <= G && G - 1 <= CK, "one lane per cp.async chunk; a lane joins inside the first checkpoint block");
 
 	__shared__ uint32_t s_ring[4][NG][RING_STRIDE];
 	__shared__ uint32_t s_rows[4][NG][RDW * 16 + 1]; // (whole 16-base words: the read staging stores without a row test)
-	__shared__ __align__(16) uint2 s_raw[4][NG][2][2][HG]; // [slot][half][word]: raw pool words of the ring blocks in flight (cp.async)
+	__shared__ __align__(16) uint2 s_raw[4][NG][2][2][WB]; // [slot][half][word]: raw pool words of the ring blocks in flight (cp.async)
+	// SPLIT, four-lane groups: the granule masks of the lane's rows (read and written only at the fold and in the epilogue)
+	// live here rather than in 25 registers, which buys the third CTA per SM
+	constexpr bool INFO_SMEM = MODE == MODE_SPLIT && G == 4;
+	__shared__ uint32_t s_info[4][INFO_SMEM ? S : 1][32];
 
 	const int lane = threadIdx.x & 31;
 	const int warp = threadIdx.x >> 5;
@@ -493,13 +513,13 @@ __global__ void __launch_bounds__(128, FastOcc<S, MODE>::kMinBlocks) dp_fast_ker
 		// ---- reference ring: two blocks of CH columns resident as 32-bit {half 1, half 0} symbol pairs; the pool words
 		//      of the next block are copied into shared memory by cp.async while the wavefront crosses the current one ----
 		const uint32_t R0 = jp.R[0], R1 = jp.R[1];
-		uint2(*raw)[2][HG] = s_raw[warp][q];
-		// lanes 0 .. G/2-1 copy one 16-byte chunk (two pool words) each: G/4 chunks per half
+		uint2(*raw)[2][WB] = s_raw[warp][q];
+		// lanes 0 .. WB-1 copy one 16-byte chunk (two pool words) each: WB/2 chunks per half
 		auto issue_block = [&](int blk) {
-			if (g < HG)
+			if (g < WB)
 			{
-				const int h = g / (G / 4), c = g % (G / 4);
-				const uint32_t wi = (uint32_t)blk * HG + 2u * c;
+				const int h = g / (WB / 2), c = g % (WB / 2);
+				const uint32_t wi = (uint32_t)blk * WB + 2u * c;
 				if (wi * 16u < (h ? R1 : R0))
 				{
 					DFB_BC((unsigned long long)jp.ref_w[h] + wi + 2 <= p.pool_words && ((jp.ref_w[h] + wi) & 1u) == 0, 203);
@@ -524,11 +544,15 @@ __global__ void __launch_bounds__(128, FastOcc<S, MODE>::kMinBlocks) dp_fast_ker
 
 		uint32_t acc = 0x80008000u;
 		uint32_t Y[(MODE == MODE_SPLIT) ? S : 1];    // SPLIT: row maxima inside the current checkpoint block
-		uint32_t info[(MODE == MODE_SPLIT) ? S : 1]; // SPLIT: granules in which the row attains its maximum X, a 16-bit mask per half
+		uint32_t info_r[(MODE == MODE_SPLIT && !INFO_SMEM) ? S : 1]; // SPLIT: granules in which the row attains its maximum X, a 16-bit mask per half
+		auto info = [&](int k) -> uint32_t& {
+			if constexpr (INFO_SMEM) return s_info[warp][k][lane];
+			else return info_r[k];
+		};
 		if (MODE == MODE_SPLIT)
 		{
 #pragma unroll
-			for (int k = 0; k < S; k++) { Y[k] = 0; info[k] = 0; }
+			for (int k = 0; k < S; k++) { Y[k] = 0; info(k) = 0; }
 		}
 		// the sweep, one checkpoint block (CK steps) at a time so that the per-block work (checkpoint,
 		// ring refill, row-maximum bookkeeping) stays out of the per-step instruction stream
@@ -681,7 +705,7 @@ __global__ void __launch_bounds__(128, FastOcc<S, MODE>::kMinBlocks) dp_fast_ker
 					const uint32_t xn = __vmaxs2(X[k], Y[k]);
 					const uint32_t beat = spread_bit15(xn - X[k] + 0x7FFF7FFFu);  // 0xFFFF per half whose block maximum > row maximum
 					const uint32_t below = spread_bit15(xn - Y[k] + 0x7FFF7FFFu); // 0xFFFF per half whose block maximum < row maximum
-					info[k] = (info[k] & ~beat) | (bit2 & ~below);
+					info(k) = (info(k) & ~beat) | (bit2 & ~below);
 					X[k] = xn;
 					Y[k] = 0;
 				}
@@ -762,13 +786,13 @@ __global__ void __launch_bounds__(128, FastOcc<S, MODE>::kMinBlocks) dp_fast_ker
 					{
 						tlo = (0u - (X[k] & 0xFFFFu)) & 0xFFFFu;
 						en_any = true;
-						gr0 |= info[k] & 0xFFFFu;
+						gr0 |= info(k) & 0xFFFFu;
 					}
 					if (b1 > 0 && b2 > 0 && b1 + b2 == best)
 					{
 						thi = (0u - (X[k] >> 16)) & 0xFFFFu;
 						en_any = true;
-						gr1 |= info[k] >> 16;
+						gr1 |= info(k) >> 16;
 					}
 				}
 				ntg[k] = tlo | (thi << 16);
@@ -823,40 +847,42 @@ __global__ void __launch_bounds__(128, FastOcc<S, MODE>::kMinBlocks) dp_fast_ker
 // visits the r-th marked granule of either half -- the two halves of the registers resume from two
 // different checkpoints -- and records every column at which an enabled row reaches its target.
 // ------------------------------------------------------------------------------------------
-template <int S>
+// (four-lane groups: 25-row strips spill 104 bytes at 128 registers, 36 at 168 -- outside the step loop: three CTAs)
+template <int G, int S>
 struct ProbeOcc
 {
 	static constexpr int kEst = 3 * S + 44;
 #ifndef DFB_PROBE_OCC6_EST
 #define DFB_PROBE_OCC6_EST 60 // strips up to this register estimate ask ptxas for six CTAs per SM (build-time knob for A/B runs)
 #endif
-	static constexpr int kMinBlocks = kEst <= DFB_PROBE_OCC6_EST ? 6 : (kEst <= 100 ? 5 : (kEst <= 128 ? 4 : (kEst <= 168 ? 3 : 2)));
+	static constexpr int kMinBlocks =
+	    G == 4 ? 3 : (kEst <= DFB_PROBE_OCC6_EST ? 6 : (kEst <= 100 ? 5 : (kEst <= 128 ? 4 : (kEst <= 168 ? 3 : 2))));
 };
 
 template <int G, int S>
-__global__ void __launch_bounds__(128, ProbeOcc<S>::kMinBlocks) dp_probe_kernel(const __grid_constant__ FastParams p)
+__global__ void __launch_bounds__(128, ProbeOcc<G, S>::kMinBlocks) dp_probe_kernel(const __grid_constant__ FastParams p)
 {
 	constexpr int NG = 32 / G;
-	constexpr int CH = 8 * G;
-	constexpr int CK = 4 * G;
+	constexpr int CK = ckpt_steps(G);
+	constexpr int CH = 2 * CK;
 	constexpr int RING = 2 * CH;
 	// G words in front of every ring: the mirror of its last G-1 columns (ring_decode_block) -- and what puts the rings of a
 	// warp's groups, which read the same index in the same step, into different banks
 	constexpr int RING_STRIDE = RING + G;
-	constexpr int HG = G / 2;
+	constexpr int WB = CH / 16; // pool words of one half in a ring block
 	constexpr int PRE = 32; // ring columns in front of a round's first step (>= G-1, two whole pool words)
-	static_assert(G >= 8 && (G & (G - 1)) == 0 && G <= 32, "group size");
+	static_assert(G >= 4 && (G & (G - 1)) == 0 && G <= 32 && WB <= G, "group size");
 	static_assert(G - 1 <= PRE && PRE + CK <= CH, "a one-block round fits one ring block");
 
 	__shared__ uint32_t s_ring[4][NG][RING_STRIDE];
-	__shared__ __align__(16) uint2 s_raw[4][NG][2][2][HG];
+	__shared__ __align__(16) uint2 s_raw[4][NG][2][2][WB];
 
 	const int lane = threadIdx.x & 31;
 	const int warp = threadIdx.x >> 5;
 	const int q = lane / G;
 	const int g = lane % G;
 	uint32_t* ring = s_ring[warp][q] + G;
-	uint2(*raw)[2][HG] = s_raw[warp][q];
+	uint2(*raw)[2][WB] = s_raw[warp][q];
 
 	const uint32_t B = p.bias;
 	const uint32_t Bp = B | (B << 16);
@@ -934,10 +960,10 @@ __global__ void __launch_bounds__(128, ProbeOcc<S>::kMinBlocks) dp_probe_kernel(
 			// ring index = relative column + PRE; relative column 0 = absolute column b * CK of the half
 			const int c0 = b0 * CK - PRE, c1 = b1 * CK - PRE; // absolute column of ring column 0 (negative in block 0)
 			auto issue_block = [&](int blk) {
-				if (g < HG)
+				if (g < WB)
 				{
-					const int h = g / (G / 4), c = g % (G / 4);
-					const int wi = ((h ? c1 : c0) >> 4) + blk * HG + 2 * c; // (c0, c1 are multiples of 32: arithmetic shift is exact)
+					const int h = g / (WB / 2), c = g % (WB / 2);
+					const int wi = ((h ? c1 : c0) >> 4) + blk * WB + 2 * c; // (c0, c1 are multiples of 32: arithmetic shift is exact)
 					if (wi >= 0 && (uint32_t)wi * 16u < (h ? R1 : R0))
 					{
 						DFB_BC((unsigned long long)jp.ref_w[h] + (unsigned)wi + 2 <= p.pool_words && ((jp.ref_w[h] + (unsigned)wi) & 1u) == 0, 204);
